@@ -3,7 +3,7 @@
 reference's CPU path as baseline.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--config celeba|dsprites|colored] [--batch B_per_gpu]
-                  [--global-batch B] [--impl ours|reference]
+                  [--global-batch B] [--impl ours|reference] [--dump-outputs DIR]
   N > 1:  python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
               --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -297,6 +297,35 @@ def build_step(config, dev, rank, B):
     return step, sampled, host
 
 
+DUMP_SAMPLE = 1 << 20     # elements: a larger tensor is dumped as a seeded sample
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, losses, step):
+    """What the last timed step hands its caller: the losses it returns and the model state it leaves behind (every
+    floating-point parameter and buffer of the step's networks), as out_dir/<name>.npy in float32 (float64 where the
+    state is float64).  A tensor of more than DUMP_SAMPLE elements is written flattened, as the same seeded sample of
+    its elements on every run, so that the dumps of two builds compare element for element."""
+    arrays = {k: v.detach().float().cpu().numpy().reshape(1) for k, v in losses.items()}
+    for mname, m in sorted(vars(step).items()):
+        if not isinstance(m, torch.nn.Module):
+            continue
+        for k, t in m.state_dict().items():
+            if not t.is_floating_point():
+                continue
+            t = t.detach()
+            if t.numel() > DUMP_SAMPLE:
+                idx = np.sort(np.random.RandomState(0).choice(t.numel(), DUMP_SAMPLE, replace=False))
+                t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+            arrays[f"{mname}.{k}"] = t.to(torch.float64 if t.dtype == torch.float64 else torch.float32).cpu().numpy()
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise SystemExit(f"bench.py: --dump-outputs would write {total} bytes (limit {DUMP_MAX_BYTES})")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def _main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -312,7 +341,14 @@ def _main():
     ap.add_argument("--profile-out", default=None, help="write the per-entry-point time table here (json)")
     ap.add_argument("--no-graph", action="store_true", help="launch every kernel from Python instead of replaying "
                     "the captured whole-step CUDA graph")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps, write the losses of the last timed step and the model state it left as "
+                         "DIR/<name>.npy (tensors over 2^20 elements as a seeded sample)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs dumps the CUDA path (--impl ours); the reference arm writes nothing")
     if args.impl == "reference":
         return run_reference(args)
     if args.warmup < 3:
@@ -394,7 +430,7 @@ def _main():
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for i in range(args.steps):
-            step(resident[i % R])
+            last = step(resident[i % R])
         e1.record()
         torch.cuda.synchronize()
         ms_local = e0.elapsed_time(e1)
@@ -404,7 +440,7 @@ def _main():
             flush.fill_(i & 0xff)
             a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             a.record()
-            step(resident[i % R])
+            last = step(resident[i % R])
             b.record()
             evs.append((a, b))
         torch.cuda.synchronize()
@@ -417,6 +453,8 @@ def _main():
     barrier()
     ms = max_over_ranks(ms_local)
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:    # before the e2e replays overwrite the graph's outputs and step the models on
+        dump_outputs(args.dump_outputs, last, eager_step)
 
     # ---- end-to-end: HOST image batch in, losses out, every step -------------------------------------------------
     # graph: while replay i runs, the pinned host batch of step i + 1 is copied on a copy stream (every step's H2D

@@ -1,5 +1,5 @@
 """CPU suite (-m "not gpu"): the oracle against the golden vectors generated from the reference, the
-oracle against the reference itself when /root/reference is present, the host-side mirror (state_dict
+oracle against the reference itself when a checkout of it is present ($EADGAN_REF), the host-side mirror (state_dict
 layout, constructor parity, no-CPU-fallback errors), and the C-ABI library (loads, exports every
 symbol include/eadgan.h declares)."""
 import ctypes
@@ -13,9 +13,12 @@ import pytest
 import torch
 
 from conftest import ROOT
+from oracle import ref_runner
 
 warnings.filterwarnings("ignore")
 GOLDEN = os.path.join(ROOT, "tests", "golden")
+# the upstream EAD-GAN scripts are not part of this repository: point EADGAN_REF at a checkout to run these
+NEEDS_REFERENCE = pytest.mark.skipif(not ref_runner.available(), reason="needs a checkout of the reference ($EADGAN_REF)")
 
 
 def _close(a, b, rtol, atol=1e-9):
@@ -171,7 +174,23 @@ def test_colored_affine_glue_matches_oracle():
     assert (affine.colored_relative_code_torch(c1, c2) - O.colored_affine_color_regularizer(c1, c2)).abs().max() <= 1e-4
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="reference checkout not present (GPU box)")
+def test_celeba_and_dsprites_affine_glue_matches_oracle():
+    """the product's closed-form affine glue (eadgan_b200/affine.py) vs the oracle's matrix form, which the golden
+    fixtures pin to the reference's utils_*.py through the losses and gradients of whole steps (the tests below
+    compare with utils_*.py directly when a checkout of the reference is present)."""
+    from eadgan_b200 import affine
+    from oracle import torch_oracle as O
+    g = torch.Generator().manual_seed(1)
+    c1, c2, c3 = (torch.rand(9, k, generator=g) * 2 - 1 for k in (4, 4, 3))
+    assert (affine.dsprites_matrix23(c1) - O.dsprites_get_matrix(c1)[:, 0:2]).abs().max() <= 1e-6
+    assert (affine.dsprites_align_inverse(c3) - torch.inverse(O.dsprites_align_matrix(c3))[:, 0:2]).abs().max() <= 1e-6
+    assert (affine.dsprites_relative_code_torch(c1, c2) - O.dsprites_affine_regularizer(c1, c2)).abs().max() <= 1e-4
+    c1, c2 = torch.rand(9, 8, generator=g) * 2 - 1, torch.rand(9, 8, generator=g) * 2 - 1
+    assert (affine.celeba_matrix(c1[:, :5]) - O.celeba_get_matrix(c1[:, :5])).abs().max() <= 1e-6
+    assert (affine.celeba_relative_code_torch(c1, c2) - O.celeba_affine_regularizer(c1, c2)).abs().max() <= 1e-4
+
+
+@NEEDS_REFERENCE
 def test_oracle_classes_equal_reference_classes():
     """key-for-key, bit-for-bit equality of the restated modules with the AST-extracted reference classes."""
     from oracle import ref_runner as R, torch_oracle as O
@@ -192,16 +211,16 @@ def test_oracle_classes_equal_reference_classes():
         assert torch.equal(a, b)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="reference checkout not present (GPU box)")
+@NEEDS_REFERENCE
 def test_reference_affine_glue_matches():
     import importlib.util
     import sys
-    from oracle import torch_oracle as O
+    from oracle import ref_runner as R, torch_oracle as O
     from eadgan_b200 import affine
     saved = torch.Tensor.cuda
     torch.Tensor.cuda = lambda self, *a, **k: self
     try:
-        spec = importlib.util.spec_from_file_location("ref_utils_rpqxy", "/root/reference/celebA/utils_rpqxy.py")
+        spec = importlib.util.spec_from_file_location("ref_utils_rpqxy", os.path.join(R.REF_ROOT, "celebA", "utils_rpqxy.py"))
         U = importlib.util.module_from_spec(spec)
         spec.loader.exec_module(U)
         torch.manual_seed(0)
@@ -216,19 +235,19 @@ def test_reference_affine_glue_matches():
         assert (impl_r(c1, c2) - r_ref).abs().max() <= 1e-4
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="reference checkout not present (GPU box)")
+@NEEDS_REFERENCE
 def test_reference_dsprites_affine_glue_matches():
     """dSprites/utils_pxy.py + utils_rp.py executed as is vs the oracle restatement and the device-side
     closed-form glue of the product (eadgan_b200/affine.py)."""
     import importlib.util
-    from oracle import torch_oracle as O
+    from oracle import ref_runner as R, torch_oracle as O
     from eadgan_b200 import affine
     saved = torch.Tensor.cuda
     torch.Tensor.cuda = lambda self, *a, **k: self
     try:
         mods = {}
         for name in ("utils_pxy", "utils_rp"):
-            spec = importlib.util.spec_from_file_location("ref_" + name, f"/root/reference/dSprites/{name}.py")
+            spec = importlib.util.spec_from_file_location("ref_" + name, os.path.join(R.REF_ROOT, "dSprites", name + ".py"))
             mods[name] = importlib.util.module_from_spec(spec)
             mods[name].np = np          # utils_rp.py uses np without importing it (the scripts star-import numpy first)
             spec.loader.exec_module(mods[name])
@@ -509,7 +528,7 @@ def test_approximator_oracle_reproduces_reference_golden():
             _check_fp(t, fp, 1e-5)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="needs the reference checkout (build container only)")
+@NEEDS_REFERENCE
 def test_approximator_oracle_equals_the_executed_script():
     from oracle import ref_runner as R, torch_oracle as O
     ns, log = R.run_approximator(3, seed=1)
