@@ -105,7 +105,6 @@ _PROTOS = {
     "eadgan_affine_grid_bwd": [_P, _I, _I, _I, _P, _P],
     "eadgan_grid_sample_fwd": [_P, _P, _I, _I, _I, _I, _I, _I, _I, _P, _P],
     "eadgan_grid_sample_bwd": [_P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _P, _P, _P],
-    "eadgan_set_reserved_sms": [_I],
     "eadgan_relcode_dims": [_I, _P, _P],
     "eadgan_relcode_fwd": [_I, _P, C.c_longlong, _P, C.c_longlong, _I, _P, _P, _P],
     "eadgan_relcode_bwd": [_I, _P, _P, _I, _P, _P, _P],

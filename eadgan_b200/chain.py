@@ -151,9 +151,6 @@ def prefetch_spectral_norm(seq, count=1):
                 conv.__dict__.setdefault("_eadgan_sn_queue", []).append((entry, ev, tag))
 
 
-pack_prefetch_enabled = os.environ.get("EADGAN_PACK_PREFETCH", "1") != "0"
-
-
 def prefetch_packs(module):
     """Re-pack the bf16 GEMM operands of every conv stack inside ``module`` now, on the side stream.
 
@@ -162,7 +159,7 @@ def prefetch_packs(module):
     permutation kernels per step then overlap the main stream's work instead of preceding the first GEMM that needs
     them.  The layouts are the ones each parameter was consumed in so far (tc._note_use), i.e. nothing happens on the
     first step.  Every pack built here carries an event which its consumer's stream waits on (tc._adopt)."""
-    if precision() != "bf16" or not prefetch_enabled or not pack_prefetch_enabled:
+    if precision() != "bf16" or not prefetch_enabled:
         return
     todo = []
     for seq in module.modules():

@@ -497,8 +497,7 @@ bool nhwc8_ok(const Geo& g, const eadgan_tensor4* const* ts, int nt) {
 }
 Nhwc8 make_nhwc8(const Geo& g) { return Nhwc8{g.n, g.c, g.h, g.w, g.c / 8, g.w * g.c / 8}; }
 int nhwc8_grid(const Geo& g) {
-  static const int per_sm = [] { const char* e = getenv("EADGAN_BN_BLOCKS_PER_SM"); const int v = e ? atoi(e) : 0; return v > 0 ? v : 2; }();
-  const int groups = (g.n * g.h + NHWC8_U - 1) / NHWC8_U, cap = per_sm * eg_sm_count();
+  const int groups = (g.n * g.h + NHWC8_U - 1) / NHWC8_U, cap = 2 * eg_sm_count();   // 2 blocks per SM (profiles/r02ab_*)
   return groups < cap ? groups : cap;
 }
 

@@ -35,7 +35,6 @@ void eg_count_launch();
   } while (0)
 
 int eg_sm_count();
-int eg_tc_units();   // SMs available to the persistent tcgen05 grids (SM count minus those reserved for NCCL)
 
 // ---- device helpers ---------------------------------------------------------
 __device__ __forceinline__ float eg_ld(const void* p, int64_t i, int dtype) {

@@ -43,20 +43,6 @@ extern "C" const char* eadgan_last_error(void) { return g_err; }
 extern "C" int eadgan_version(void) { return EADGAN_VERSION; }
 extern "C" int eadgan_sm_count(void) { return eg_sm_count(); }
 
-// SMs the persistent tcgen05 kernels leave free (eg_tc_units): while gradient all-reduces are in flight on the
-// communication stream the data-parallel layer reserves a few SMs, so that NCCL's CTAs run BESIDE the persistent
-// GEMM grids (which otherwise own every SM's shared memory: the collective then either waits for a kernel
-// boundary, or delays a few late-starting persistent CTAs and with them the whole kernel).
-static std::atomic<int> g_reserved_sms{0};
-extern "C" int eadgan_set_reserved_sms(int n) {
-  g_reserved_sms.store(n < 0 ? 0 : n, std::memory_order_relaxed);
-  return 0;
-}
-int eg_tc_units() {
-  const int sms = eg_sm_count(), r = g_reserved_sms.load(std::memory_order_relaxed);
-  return sms - r >= 2 ? sms - r : 2;
-}
-
 namespace {
 
 int stream_grid(int64_t work_items, int per_block) {

@@ -767,11 +767,11 @@ tc_conv_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
 // pixel the 32 lanes of a warp hold 32 consecutive channels = one 64-byte run of the NHWC tensors, so the fused
 // activation-backward mask is read, and the result written, as full 32-byte sectors.
 // ------------------------------------------------------------------------------------
-template <int EW>
 struct DgTCfg {
   static constexpr int STAGE_BYTES = 3 * A_BYTES;                 // two pixel tiles + one weight tile, 48 KB
   static constexpr int STAGES = 4;
-  static constexpr int CH = EW == 8 ? 32 : 16;                    // pixels per epilogue chunk
+  static constexpr int EW = 16;                                   // epilogue warps
+  static constexpr int CH = 16;                                   // pixels per epilogue chunk
   static constexpr int STG_BYTES = CH * 64;                       // per warp: [CH pixels][32 channels] bf16
   static constexpr int STAT_BYTES = (EW / 4) * 128 * 2 * 4;       // [column group][channel][sum, sum of squares] fp32
   static constexpr int SMEM = STAGES * STAGE_BYTES + 1024 + 256 + EW * STG_BYTES + STAT_BYTES;
@@ -795,11 +795,12 @@ __device__ __forceinline__ void tmem_ld16(uint32_t taddr, float* v) {
 // epilogue is bound by its instruction stream: ncu r02y, 414 instructions per 32x32 chunk of which 160 are the
 // arithmetic and the stores): 0 = generic (every switch read from P), 1 = bias + (Leaky)ReLU (the thin fprop),
 // 2 = fused (Leaky)ReLU-backward mask, 3 = BatchNorm statistics; ReLU is LeakyReLU with slope 0 (set by the launcher).
-// EW = epilogue warps (8 or 16): warp (quad, group) owns channels quad*32.. and 256 / (EW/4) pixel columns.
-template <int SPEC, int EW>
-__global__ void __launch_bounds__(64 + EW * 32, 1)
+// Epilogue warp (quad, group) owns channels quad*32.. and 256 / (EW/4) pixel columns.
+template <int SPEC>
+__global__ void __launch_bounds__(64 + DgTCfg::EW * 32, 1)
 tc_dgradT_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constant__ CUtensorMap map_w, const TcParams P) {
-  using C = DgTCfg<EW>;
+  using C = DgTCfg;
+  constexpr int EW = C::EW;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
   uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem + C::STAGES * C::STAGE_BYTES);
@@ -985,7 +986,7 @@ tc_dgradT_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constan
           if (c0 + CH < cbase + GCOLS) load_mask(c0 + CH);
         }
         float v[CH];
-        if (CH == 32) tmem_ld32(acc + (uint32_t)c0, v); else tmem_ld16(acc + (uint32_t)c0, v);
+        tmem_ld16(acc + (uint32_t)c0, v);
         if (c0 + CH >= cbase + GCOLS) {   // this warp's columns are all in registers: hand the accumulator back
           tc_fence_before();
           __syncwarp();
@@ -1466,22 +1467,21 @@ int opt_in_smem(K kernel, int bytes, std::atomic<uint64_t>& done) {
   return 0;
 }
 
-template <int SPEC, int EW>
+template <int SPEC>
 int launch_channel_major_t(const CUtensorMap& mx, const CUtensorMap& mw, const TcParams& P, cudaStream_t st) {
   static std::atomic<uint64_t> opted{0};
-  if (int e = opt_in_smem(tc_dgradT_kernel<SPEC, EW>, DgTCfg<EW>::SMEM, opted)) return e;
+  if (int e = opt_in_smem(tc_dgradT_kernel<SPEC>, DgTCfg::SMEM, opted)) return e;
   const int total = P.parities * P.m_tiles * P.n_tiles;
-  const int units = eg_tc_units();
+  const int units = eg_sm_count();
   const int waves = (total + units - 1) / units;
   const int grid = (total + waves - 1) / waves;
-  tc_dgradT_kernel<SPEC, EW><<<grid, 64 + EW * 32, DgTCfg<EW>::SMEM, st>>>(mx, mw, P);
+  tc_dgradT_kernel<SPEC><<<grid, 64 + DgTCfg::EW * 32, DgTCfg::SMEM, st>>>(mx, mw, P);
   EG_LAUNCH_CHECK("tc_dgradT_kernel");
   return 0;
 }
 
-int launch_channel_major(const CUtensorMap& mx, const CUtensorMap& mw, const TcParams& P0, cudaStream_t st) {
+int launch_channel_major(const CUtensorMap& mx, const CUtensorMap& mw, TcParams P, cudaStream_t st) {
   // the three epilogue shapes of the training step get a specialised instance (see tc_dgradT_kernel)
-  TcParams P = P0;
   const bool act_lrelu = P.act == EADGAN_ACT_RELU || P.act == EADGAN_ACT_LRELU;
   const bool mask_lrelu = P.mask_mode == EADGAN_ACT_RELU || P.mask_mode == EADGAN_ACT_LRELU;
   int spec = 0;
@@ -1494,13 +1494,12 @@ int launch_channel_major(const CUtensorMap& mx, const CUtensorMap& mw, const TcP
   } else if (!P.mask_mode && P.want_stats == 1 && !P.act) {
     spec = 3;
   }
-  int ew = 16;
-  if (const char* e = getenv("EADGAN_TC_EW")) { if (atoi(e) == 8 || atoi(e) == 16) ew = atoi(e); }
-  if (const char* e = getenv("EADGAN_TC_SPEC")) { if (atoi(e) == 0) { spec = 0; P = P0; } }
-#define EG_CM(S, W) if (spec == S && ew == W) return launch_channel_major_t<S, W>(mx, mw, P, st);
-  EG_CM(0, 8) EG_CM(1, 8) EG_CM(2, 8) EG_CM(3, 8) EG_CM(0, 16) EG_CM(1, 16) EG_CM(2, 16) EG_CM(3, 16)
-#undef EG_CM
-  return EADGAN_ERR_INVALID;
+  switch (spec) {
+    case 1: return launch_channel_major_t<1>(mx, mw, P, st);
+    case 2: return launch_channel_major_t<2>(mx, mw, P, st);
+    case 3: return launch_channel_major_t<3>(mx, mw, P, st);
+  }
+  return launch_channel_major_t<0>(mx, mw, P, st);
 }
 
 bool pow2(int v) { return v > 0 && (v & (v - 1)) == 0; }
@@ -1522,8 +1521,7 @@ int launch_conv(const CUtensorMap& ma, const CUtensorMap& mb, const TcParams& P,
   if (int e = opt_in_smem(tc_conv_kernel<BN, MT, CG>, Cfg<BN, MT, CG>::SMEM, opted)) return e;
   // persistent grid: every CTA (CTA pair) runs the same number of tiles (+-1), at most one CTA per SM
   const int total = P.parities * P.m_tiles * P.n_tiles;
-  int units = eg_tc_units() / CG;
-  if (const char* e = getenv("EADGAN_TC_UNITS")) { if (atoi(e) > 0 && atoi(e) < units) units = atoi(e); }   // experiments
+  const int units = eg_sm_count() / CG;
   const int waves = (total + units - 1) / units;
   const int grid = ((total + waves - 1) / waves) * CG;
   cudaLaunchConfig_t cfg{};
@@ -1532,13 +1530,6 @@ int launch_conv(const CUtensorMap& ma, const CUtensorMap& mb, const TcParams& P,
   attr[0].id = cudaLaunchAttributeClusterDimension;
   attr[0].val.clusterDim.x = CG; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr; cfg.numAttrs = CG == 2 ? 1 : 0;
-  if (CG == 2 && getenv("EADGAN_TC_DEBUG")) {
-    int nc = -1;
-    cudaLaunchConfig_t q = cfg; q.gridDim = dim3(2 * eg_sm_count());
-    cudaError_t er = cudaOccupancyMaxActiveClusters(&nc, tc_conv_kernel<BN, MT, CG>, &q);
-    fprintf(stderr, "[eadgan] tc_conv<%d,%d,%d>: grid %d, total %d tiles, max active clusters %d (%s)\n", BN, MT, CG, grid,
-            total, nc, cudaGetErrorString(er));
-  }
   EG_CUDA(cudaLaunchKernelEx(&cfg, tc_conv_kernel<BN, MT, CG>, ma, mb, P));
   EG_LAUNCH_CHECK("tc_conv_kernel");
   return 0;
@@ -1558,10 +1549,10 @@ TileCfg pick_cfg(int nch, int m_tiles, int parities, bool allow_pair, int force_
   const int sms = eg_sm_count();
   const int64_t tiles = (int64_t)m_tiles * parities * (nch / t.bn);
   t.cg = (allow_pair && t.bn >= 128 && m_tiles >= 2 && tiles >= 2 * sms) ? 2 : 1;
+  // test hook: force CTA pairs on (2) / off (1), so that small, ragged shapes exercise the pair protocol
   if (const char* e = getenv("EADGAN_TC_CG")) { if (allow_pair && t.bn >= 128 && (atoi(e) == 1 || atoi(e) == 2)) t.cg = atoi(e); }
   // two 128-row tiles per CTA tile (sharing every B load) when BLOCK_N <= 128 and there is enough work
   t.mt = (t.bn <= 128 && tiles >= 4 * sms * t.cg) ? 2 : 1;
-  if (const char* e = getenv("EADGAN_TC_MT")) { if (t.bn <= 128 && atoi(e) >= 1 && atoi(e) <= 2) t.mt = atoi(e); }
   return t;
 }
 
@@ -1594,10 +1585,6 @@ int dispatch_conv(const TileCfg& t, const CUtensorMap& ma, const CUtensorMap& mb
 // BLOCK_N: 256 halves the A re-reads and the smem traffic per MAC; keep 128 while the tile count is too
 // small to fill the machine twice
 int pick_bn_tiles(int nch, int m_tiles_x_par) {
-  if (const char* e = getenv("EADGAN_TC_BN")) {  // experiments only (tools/bench_gemm.py)
-    const int bn = atoi(e);
-    if (bn > 0 && nch % bn == 0) return bn;
-  }
   if (nch % 256 == 0 && (int64_t)m_tiles_x_par * (nch / 256) >= 2 * eg_sm_count()) return 256;
   if (nch % 128 == 0) return 128;
   if (nch % 64 == 0) return 64;
@@ -1682,27 +1669,6 @@ extern "C" int eadgan_tc_dgrad(const eadgan_tc_desc* d, const void* dy_pad, cons
   const TileCfg tcfg = pick_cfg(d->c, m_tiles, 4, true);
   const int bn = tcfg.bn;
   EG_REQUIRE(bn > 0, EADGAN_ERR_UNSUPPORTED, "tc_dgrad: c=%d must be a multiple of 32", d->c);
-  // 128-channel outputs with a long pixel dimension: the transposed kernel (see tc_dgradT_kernel)
-  bool transposed = d->c == 128 && d->k % 64 == 0 && !d->out_f32_nchw && (d->c_real <= 0 || d->c_real == d->c);
-  bool enough = (int64_t)m_tiles * 4 >= 8 * eg_sm_count();
-  if (const char* e = getenv("EADGAN_TC_DGRADT")) { if (atoi(e) == 0) transposed = false; else if (atoi(e) == 2) enough = true; }
-  transposed = transposed && enough;
-  if (transposed) {
-    TcParams P{};
-    P.mode = MODE_DGRAD; P.n = d->n; P.p = p; P.q = q;
-    EG_REQUIRE(pick_tile(p, q, 128, &P.Tw, &P.Th, &P.Tb) == 0, EADGAN_ERR_UNSUPPORTED, "tc_dgrad: bad small map");
-    P.tiles_y = p / P.Th; P.N_total = d->c; P.K_ch = d->k; P.qblocks = d->k / 64; P.nkb = 4 * P.qblocks;
-    P.act = d->act; P.slope = d->slope; P.want_stats = d->want_stats; P.mask_mode = d->mask_mode;
-    P.OH = d->h; P.OW = d->w; P.bias = bias; P.out = dx; P.mask = (const __nv_bfloat16*)mask; P.stats = stats;
-    P.sigma = sigma; P.n_store = d->c; P.stat_channels = d->c;
-    P.m_tiles = (m_tiles + 1) / 2; P.n_tiles = d->c / 128; P.parities = 4;
-    EG_REQUIRE(!P.mask_mode || mask, EADGAN_ERR_INVALID, "tc_dgrad: mask_mode without mask");
-    EG_REQUIRE(!P.want_stats || stats, EADGAN_ERR_INVALID, "tc_dgrad: want_stats without stats");
-    CUtensorMap mx, mw;
-    if (int e = map_small(&mx, dy_pad, d->n, d->k, p, q, P.Tw, P.Th, P.Tb)) return e;
-    if (int e = map_matrix(&mw, w_packed, (uint64_t)4 * d->c, (uint64_t)4 * d->k, 128)) return e;
-    return launch_channel_major(mx, mw, P, (cudaStream_t)stream);
-  }
   P.tiles_y = p / P.Th; P.N_total = d->c; P.K_ch = d->k; P.qblocks = (d->k + 63) / 64; P.nkb = 4 * P.qblocks;
   P.act = d->act; P.slope = d->slope; P.out_f32_nchw = d->out_f32_nchw; P.want_stats = d->want_stats;
   P.mask_mode = d->mask_mode; P.OH = d->h; P.OW = d->w; P.bias = bias; P.out = dx;
@@ -1715,6 +1681,18 @@ extern "C" int eadgan_tc_dgrad(const eadgan_tc_desc* d, const void* dy_pad, cons
   EG_REQUIRE(!P.want_stats || stats, EADGAN_ERR_INVALID, "tc_dgrad: want_stats without stats");
   CUtensorMap ma, mb;
   if (int e = map_small(&ma, dy_pad, d->n, d->k, p, q, P.Tw, P.Th, P.Tb)) return e;
+  // 128-channel outputs with a long pixel dimension: the transposed kernel (see tc_dgradT_kernel), 128 channels x 256
+  // pixels per tile.  It shares P: its conditions k % 64 == 0, c_real == c and no out_f32_nchw are what make
+  // qblocks, n_store and out_f32_nchw above right for it too.
+  bool transposed = d->c == 128 && d->k % 64 == 0 && !d->out_f32_nchw && (d->c_real <= 0 || d->c_real == d->c);
+  bool enough = (int64_t)m_tiles * 4 >= 8 * eg_sm_count();
+  // test hook: 0 / 2 = never / always use the transposed kernel where it applies
+  if (const char* e = getenv("EADGAN_TC_DGRADT")) { if (atoi(e) == 0) transposed = false; else if (atoi(e) == 2) enough = true; }
+  if (transposed && enough) {
+    P.m_tiles = (m_tiles + 1) / 2; P.n_tiles = d->c / 128; P.parities = 4;
+    if (int e = map_matrix(&mb, w_packed, (uint64_t)4 * d->c, (uint64_t)4 * d->k, 128)) return e;
+    return launch_channel_major(ma, mb, P, (cudaStream_t)stream);
+  }
   if (int e = map_matrix(&mb, w_packed, (uint64_t)4 * d->c, (uint64_t)4 * d->k, bn / tcfg.cg)) return e;
   return dispatch_conv(tcfg, ma, mb, P, m_tiles, d->c, 4, (cudaStream_t)stream);
 }
@@ -1735,12 +1713,13 @@ int wgrad_plan(const eadgan_tc_desc* d, WgParams* P, int* bn, int* splits, int* 
   *bn = (P->Ktot % 256 == 0) ? 256 : (P->Ktot % 128 == 0 ? 128 : 64);
   // CTA pairs (256 ko rows per tile, see WgCfg) when there are whole 256-row tiles and a long reduction
   *cg = (*bn == 256 && d->k % 256 == 0 && P->steps_total >= 256) ? 2 : 1;
+  // test hook: force CTA pairs on (2) / off (1), as in pick_cfg
   if (const char* e = getenv("EADGAN_TC_CG")) { if (*bn == 256 && d->k % 256 == 0 && (atoi(e) == 1 || atoi(e) == 2)) *cg = atoi(e); }
   const int tiles = (P->Ktot / *bn) * ((d->k + 127) / 128) / *cg;
   // split of the pixel reduction: one CTA per (tile, split) and one CTA per SM at a time, so the kernel runs in
   // waves of sm_count CTAs.  Pick the split count minimising  waves * steps_per_split  (tensor time, a 64-pixel
   // step of a 128 x bn tile is bn*2 clocks) plus the fp32 partial-sum traffic (written once, read once).
-  const int sms = eg_tc_units() / *cg;   // concurrently running CTAs (CTA pairs)
+  const int sms = eg_sm_count() / *cg;   // concurrently running CTAs (CTA pairs)
   const int max_s = (P->steps_total + 7) / 8;
   const int k_pad = ((d->k + 127) / 128) * 128;
   double best = 1e300;
@@ -1768,7 +1747,7 @@ int launch_wgrad(const CUtensorMap& mdy, const CUtensorMap& mx, const WgParams& 
   WgParams Q = P;
   Q.kk_tiles = (int)grid.x; Q.ko_tiles = (int)grid.y; Q.splits = (int)grid.z;
   const int total = Q.kk_tiles * Q.ko_tiles * Q.splits;
-  const int units = eg_tc_units() / CG;
+  const int units = eg_sm_count() / CG;
   const int waves = (total + units - 1) / units;
   const int ctas = ((total + waves - 1) / waves) * CG;
   cudaLaunchConfig_t cfg{};
@@ -2270,7 +2249,7 @@ extern "C" int eadgan_tc_thin_fprop(const eadgan_tc_desc* d, const void* r_buf, 
   const TileCfg tcfg = pick_cfg(d->k, m_tiles, 1, false, bn);
   P.tiles_y = p / P.Th; P.N_total = d->k; P.K_ch = 4; P.qblocks = 1; P.nkb = 1;
   bool channel_major = d->k % 128 == 0 && !d->out_f32_nchw && (int64_t)m_tiles * (d->k / 128) >= 8 * eg_sm_count();
-  if (const char* e = getenv("EADGAN_TC_DGRADT")) {
+  if (const char* e = getenv("EADGAN_TC_DGRADT")) {   // test hook: 0 / 2 = never / always channel-major where it applies
     if (atoi(e) == 0) channel_major = false;
     else if (atoi(e) == 2) channel_major = d->k % 128 == 0 && !d->out_f32_nchw;
   }

@@ -40,17 +40,6 @@ class DataParallel:
         self._plans = {}      # id(optimizer) -> plan
         self._armed = None
         self._hooks_installed = set()
-        # SMs the persistent tcgen05 grids leave to NCCL while bucket all-reduces are in flight (see csrc/elementwise.cu)
-        # Measured on 2 x B200 (profiles/r02l_dp_reserve_sms.txt): no gain from 4 / 8 / 16 reserved SMs, with or without
-        # NCCL_MAX_CTAS -- the exposed communication is not the bucket all-reduces competing for SMs -- so the default is 0.
-        self.reserve_sms = int(os.environ.get("EADGAN_DP_RESERVE_SMS", "0")) if device.type == "cuda" else 0
-        self._reserved = False
-
-    def _reserve(self, on):
-        if self.reserve_sms > 0 and on != self._reserved:
-            from ._lib import call
-            call("eadgan_set_reserved_sms", self.reserve_sms if on else 0)
-            self._reserved = on
 
     # ---- SyncBN -----------------------------------------------------------------------
     def allreduce_sum_(self, t):
@@ -121,7 +110,6 @@ class DataParallel:
             self._launch(b)
 
     def _launch(self, b):
-        self._reserve(True)     # from here to reduce(): the rest of this backward runs beside the collective
         if self.comm_stream is not None:
             self.comm_stream.wait_stream(torch.cuda.current_stream())
             with torch.cuda.stream(self.comm_stream):
@@ -148,7 +136,6 @@ class DataParallel:
                 b["work"] = None
                 b["dirty"] = False
                 self._launch(b)
-        self._reserve(False)
         for b in plan["buckets"]:
             b["work"].wait()
             if self.comm_stream is not None:

@@ -9,7 +9,6 @@ is the reference's and every forward/backward runs on the sm_100a kernels.
 from __future__ import annotations
 
 import itertools
-import os
 
 import torch
 
@@ -70,8 +69,7 @@ class CelebAStep:
         self.opt_info = Adam(itertools.chain(self.G.parameters(), self.D.parameters()), lr=0.0002, betas=betas)
         self.bce, self.mse, self.ce = nn.BCELoss(), nn.MSELoss(), nn.CrossEntropyLoss()
         self.device = torch.device(device)
-        e = os.environ.get("EADGAN_DEFER_D")       # experiments: force the placement of opt_D.step() (see __call__)
-        self._defer_D = None if e is None else e != "0"
+        self._defer_D = None    # None: defer opt_D.step() under data parallelism only; True / False force it (see __call__)
 
     def optimizers(self):
         return [self.opt_G, self.opt_D, self.opt_info]

@@ -74,9 +74,6 @@ const char* eadgan_last_error(void);
 int eadgan_version(void);
 /* number of SMs of the current device (grid sizing on the host side) */
 int eadgan_sm_count(void);
-/* SMs the persistent tcgen05 grids leave free from now on (0 = none): set by the data-parallel layer while gradient
- * all-reduces are in flight so that the collective's CTAs run beside the GEMM grids (eadgan_b200/parallel.py) */
-int eadgan_set_reserved_sms(int n);
 /* total number of kernels this library has launched in this process (bench.py's gpu_launches) */
 int64_t eadgan_kernel_launches(void);
 
