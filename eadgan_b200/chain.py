@@ -14,9 +14,9 @@ groups (every G / D / Encoder trunk of the reference: celebA/EAD-GAN_celebA.py:7
     are accumulated in the ConvTranspose epilogue (fp64 atomics) and the normalise + ReLU pass
     is one streaming kernel; the LeakyReLU/ReLU backward of layer L is fused into the epilogue
     of layer L+1's input-gradient kernel (mask = saved output of layer L);
-  * layers the tensor-core path does not cover (Cin = 3 first layer, Cout = 3 / 19 last layers,
-    the 1x1-input ConvTranspose) run on the generic SIMT kernels directly on the same buffers
-    (strided bf16 views) -- there is no torch / cuDNN fallback anywhere.
+  * layers the tensor-core path does not cover run on the generic SIMT kernels directly on the
+    same buffers (strided bf16 views) -- there is no torch / cuDNN fallback anywhere.
+    ``_plan_kernels`` picks the kernel family of every stage and direction, in one place.
 
 Forward pre-hooks of the wrapped modules (legacy spectral_norm) are honoured: they run before
 the chain and the chain consumes ``module.weight`` (= weight_orig / sigma, an autograd tensor).
@@ -107,6 +107,16 @@ prefetch_enabled = True     # False: prefetch_spectral_norm is a no-op and every
                             # (state snapshots taken BETWEEN phases then hold u / v exactly as far as the forwards got)
 
 
+def _side_stream(dev):
+    """the per-device side stream of the prefetches, ordered after everything queued on the current stream so far
+    (the last optimiser step, every earlier u / v update and every earlier consumer of the old packs)"""
+    side = _sn_streams.get(dev)
+    if side is None:
+        side = _sn_streams[dev] = torch.cuda.Stream(device=dev)
+    side.wait_stream(torch.cuda.current_stream())
+    return side
+
+
 def prefetch_spectral_norm(seq, count=1):
     """Run the spectral-norm power iterations of the NEXT ``count`` forwards of ``seq`` now, on a side stream.
 
@@ -127,11 +137,7 @@ def prefetch_spectral_norm(seq, count=1):
     w0 = getattr(convs[0], "weight_orig", None)
     if w0 is None or not w0.is_cuda:
         return
-    cur = torch.cuda.current_stream()
-    side = _sn_streams.get(w0.device)
-    if side is None:
-        side = _sn_streams[w0.device] = torch.cuda.Stream(device=w0.device)
-    side.wait_stream(cur)          # the weights (last optimiser step) and every earlier u / v update are visible
+    side = _side_stream(w0.device)
     with torch.cuda.stream(side):
         for _ in range(count):
             done = []
@@ -176,13 +182,7 @@ def prefetch_packs(module):
                 todo.append(p)
     if not todo:
         return
-    dev = todo[0].device
-    cur = torch.cuda.current_stream()
-    side = _sn_streams.get(dev)
-    if side is None:
-        side = _sn_streams[dev] = torch.cuda.Stream(device=dev)
-    side.wait_stream(cur)          # the optimiser step (and every earlier consumer of the old packs) comes first
-    with torch.cuda.stream(side):
+    with torch.cuda.stream(_side_stream(todo[0].device)):
         for p in todo:
             tc.prefetch_packs(p)
 
@@ -333,7 +333,7 @@ def _thin_ok(d, direction):
 
 
 def _impl(st, d, last):
-    """which kernel family runs the forward of this stage."""
+    """which kernel family runs the forward of this stage (called by _plan_kernels)."""
     unit = d.r == 4 and d.stride == 1 and d.pad == 0 and d.h == 4 and d.w == 4 and d.p == 1 and d.q == 1
     plain = st.bn is None and st.act[0] == ACT_NONE
     if unit and plain and d.c % 128 == 0:
@@ -349,6 +349,62 @@ def _impl(st, d, last):
             return "simt"  # zero-padded OUTPUT channels are only supported for an fp32 NCHW result
         return "tc"
     return "simt"
+
+
+class _StagePlan:
+    """How one stage runs: its geometry ``d``, the kernel family of its forward (``fwd``), weight gradient
+    (``wgrad``) and input gradient (``dx``), and the layout of the buffers around it.
+
+    Families: "tc" (tcgen05 implicit GEMM, csrc/tc_conv.cu), "thin" (the same kernels with the 1..4-channel image as
+    big map, row-expanded to K = 64), "dense_T" / "dense_C" / "dense" (the 1x1 <-> 4x4 layers as batch GEMMs) and
+    "simt" (the any-geometry SIMT kernels, csrc/simt_conv.cu)."""
+    __slots__ = ("d", "ca", "fwd", "wgrad", "dx", "fuse", "in_fmt", "out_fmt", "in_shape", "out_shape")
+
+
+def _plan_kernels(stages, in_shape):
+    """-> one _StagePlan per stage of a compiled chain (``_plan(seq)``) run on an NCHW input of ``in_shape``.
+
+    This is the only place that picks kernels.  The executor asks autograd only WHETHER a planned kernel runs (a
+    frozen weight, an input that needs no gradient), never which one."""
+    plans = []
+    for si, st in enumerate(stages):
+        last, conv = si == len(stages) - 1, st.kind == "conv"
+        prev = stages[si - 1] if si > 0 else None
+        p = _StagePlan()
+        d = p.d = _geom(st, in_shape)
+        p.in_shape = tuple(in_shape)
+        p.out_shape = (d.n, d.k, d.p, d.q) if conv else (d.n, d.c, d.h, d.w)
+        p.fwd = _impl(st, d, last)
+        p.ca = _calloc(d) if p.fwd == "tc" else d.c
+        if p.fwd in ("dense_T", "dense_C"):
+            p.wgrad = "dense"
+            p.dx = "dense" if p.fwd == "dense_C" and si > 0 else "simt"
+        elif p.fwd == "thin":
+            if conv and last:
+                raise RuntimeError("eadgan_b200.chain: a thin conv cannot be the last stage")
+            p.wgrad = "thin" if _thin_ok(d, "wgrad") else "simt"
+            if conv:    # the image gradient of the chain's input: GEMM + col2im epilogue
+                p.dx = "thin" if si == 0 and _thin_ok(d, "dgrad") else "simt"
+            else:       # a small-map gradient from the row-expanded image gradient
+                p.dx = "thin" if si > 0 else "simt"
+        elif p.fwd == "tc":
+            p.wgrad = "tc" if _tc_ok(d, "wgrad") else "simt"
+            # zero-padded result channels need the fp32 NCHW epilogue: a conv's input gradient onto fewer than 32
+            # channels runs on the tensor cores only for the chain's input
+            tc_dx = _tc_ok(d, "dgrad" if conv else "fprop") and not (conv and si > 0 and p.ca != d.c)
+            p.dx = "tc" if tc_dx else "simt"
+        else:
+            p.wgrad = p.dx = "simt"
+        # the first stage reads the caller's fp32 NCHW tensor where its kernel can, every other buffer is padded
+        # NHWC bf16; only the chain's result is fp32 NCHW again
+        p.in_fmt = "ext" if si == 0 and (p.fwd in ("dense_T", "simt") or (p.fwd == "thin" and conv)) else "pad"
+        p.out_fmt = "ext" if last else "pad"
+        # the previous stage's LeakyReLU / ReLU backward runs in the epilogue of this stage's input-gradient kernel
+        # (mask = this stage's saved input, a padded buffer)
+        p.fuse = prev is not None and prev.bn is None and prev.act[0] != ACT_NONE
+        plans.append(p)
+        in_shape = p.out_shape
+    return plans
 
 
 def _chan_sums(buf, c):
@@ -382,107 +438,91 @@ class _Arena:
         return out
 
 
+class _Saved:
+    """what the forward of one stage leaves for its backward, and the stage's weight in every form a kernel reads"""
+    __slots__ = ("w", "src", "lazy", "pi", "has_b", "inp", "y", "R", "a", "pre", "mean", "invstd", "gamma", "beta",
+                 "count", "n_local", "sum_x")
+
+    def __init__(self, w, src, pi, has_b):
+        self.w, self.src, self.pi, self.has_b = w, src, pi, has_b
+        self.lazy = src is not None and len(src) > 2 and bool(src[2])
+        self.R = self.a = self.pre = None
+
+    def values(self):
+        """the weight VALUES (W / sigma for spectral-normalised layers), materialised on first use"""
+        if self.lazy:
+            Fn.spectral_norm_materialize(self.src[0], self.src[1], self.w)
+            self.lazy = False
+        return self.w.contiguous()
+
+    def packed(self, direction, ca):
+        """(bf16 GEMM operand of the weight for `direction`, sigma or None)"""
+        if self.src is not None:
+            return tc.pack_w_cached(self.src[0], direction, ca), self.src[1]
+        return tc.pack_w(self.values(), None, direction, ca), None
+
+    def packed_thin(self, direction):
+        if self.src is not None:
+            return tc.thin_pack_w_cached(self.src[0], direction), self.src[1]
+        return tc.thin_pack_w(self.values(), direction), None
+
+
 class _ChainFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, stages, srcs, *params):
         st_ = stream()
         dev = x.device
+        plans = _plan_kernels(stages, tuple(x.shape))
         cur = _Buf(x.contiguous(), "ext")
         saved = []
         pi = 0
         # ONE zero fill for all per-channel fp64 statistics vectors of this forward (a fill kernel per BatchNorm layer
         # was ~40 launches of a few microseconds per step)
-        arena = _Arena(sum(2 * (s_.conv.weight.shape[0] if s_.kind == "conv" else s_.conv.weight.shape[1])
-                           for s_ in stages if s_.bn is not None), dev)
-        for si, st in enumerate(stages):
-            w, b = params[pi], params[pi + 1]
-            pi += 2
-            gamma = beta = None
-            if st.bn is not None:
-                gamma, beta = params[pi], params[pi + 1]
-                pi += 2
-            last = si == len(stages) - 1
-            d = _geom(st, cur.nchw)
-            direction = "fprop" if st.kind == "conv" else "dgrad"
-            out_shape = (d.n, d.k, d.p, d.q) if st.kind == "conv" else (d.n, d.c, d.h, d.w)
+        arena = _Arena(sum(2 * p.out_shape[1] for st, p in zip(stages, plans) if st.bn is not None), dev)
+        for si, (st, p) in enumerate(zip(stages, plans)):
+            sv = _Saved(params[pi], srcs[si], pi, params[pi + 1] is not None)
+            b = params[pi + 1]
+            pi += 4 if st.bn is not None else 2
+            d, conv, last = p.d, st.kind == "conv", si == len(stages) - 1
+            out_shape = p.out_shape
             cout = out_shape[1]
             epi_act = st.act if st.bn is None else (ACT_NONE, 0.0)
             stats = arena.take(2 * cout) if st.bn is not None else None
-            wc = w.contiguous()
-            impl = _impl(st, d, last)
-            rec = {"d": d, "w": wc, "has_b": b is not None, "impl": impl, "pi": pi - (4 if st.bn is not None else 2)}
-            src = srcs[si]
-            lazy = [src is not None and len(src) > 2 and bool(src[2])]
-
-            def wvals(_src=src, _wc=wc, _w=w, _lazy=lazy):
-                """the weight VALUES (W / sigma for spectral-normalised layers), materialised on first use"""
-                if _lazy[0]:
-                    Fn.spectral_norm_materialize(_src[0], _src[1], _w)
-                    _lazy[0] = False
-                return _wc if _wc.data_ptr() == _w.data_ptr() else _w.contiguous()
-            rec["wvals"] = wvals
-
-            def packed(direction, ca, _src=src):
-                """(bf16 GEMM operand, sigma) of this stage's weight for `direction`"""
-                if _src is not None and tuple(_src[0].shape[2:]) == (4, 4):
-                    return tc.pack_w_cached(_src[0], direction, ca), _src[1]
-                return tc.pack_w(wvals(), None, direction, ca), None
-            rec["packed"] = packed
-
-            def packed_thin(direction, _src=src):
-                if _src is not None:
-                    return tc.thin_pack_w_cached(_src[0], direction), _src[1]
-                return tc.thin_pack_w(wvals(), direction), None
-            rec["packed_thin"] = packed_thin
-            if impl == "thin" and st.kind == "conv":
-                inp = cur
-                r = tc.thin_expand(cur.view())
-                rec["R"] = r
-                wpk, sg = packed_thin("fprop")
-                if last:
-                    raise RuntimeError("eadgan_b200.chain: a thin conv cannot be the last stage")
-                out = _Buf(tc.thin_fprop(r, wpk, b, d.c, cout, epi_act[0], epi_act[1], stats=stats, sigma=sg), "pad")
-            elif impl == "thin":       # ConvTranspose onto the image: GEMM over input pixels + col2im epilogue
-                inp = _Buf(cur.padded(), "pad")
-                wpk, sg = packed_thin("dgrad")
-                out = _Buf(tc.thin_dgrad(inp.t, wpk, b, d.c, epi_act[0], epi_act[1], sigma=sg), "ext")
-            elif impl == "dense_T":      # 1x1 -> 4x4 ConvTranspose: batch GEMM, scatter epilogue
-                a = tc.pad_rows(cur.t.reshape(d.n, d.k), _r64(d.k))
-                out = _Buf(tc.dense_scatter(a, tc.dense_pack(wvals(), _r64(d.k), False), b, d.c), "pad")
-                inp = cur
-                rec["a"] = a
-            elif impl == "dense_C":    # 4x4 -> 1x1 Conv head: batch GEMM, gather prologue
-                inp = _Buf(cur.padded(), "pad")
-                o = tc.dense_gather(inp.t, tc.dense_pack(wvals(), 32, True), b, d.k)
-                out = _Buf(o.view(d.n, d.k, 1, 1), "ext")
-            elif impl == "tc":
-                ca = _calloc(d)
-                if st.kind == "conv":
-                    inp = _Buf(cur.t if cur.fmt == "pad" else tc.to_padded(cur.t, ca), "pad")
-                    wpk, sg = packed("fprop", ca)
-                    out_t = tc.fprop(inp.t, wpk, b, cout, epi_act[0], epi_act[1], out_f32_nchw=last, stats=stats,
-                                     sigma=sg)
-                else:
-                    inp = _Buf(cur.padded(), "pad")
-                    wpk, sg = packed("dgrad", ca)
-                    out_t = tc.dgrad(inp.t, wpk, b, ca, epi_act[0], epi_act[1], out_f32_nchw=last, stats=stats,
-                                     c_real=d.c if ca != d.c else 0, sigma=sg)
-                out = _Buf(out_t, "ext" if last else "pad")
+            # a conv reads its big map zero-padded to p.ca channels
+            inp = cur if cur.fmt == p.in_fmt else _Buf(tc.to_padded(cur.t, p.ca if conv else None), "pad")
+            if p.fwd == "thin" and conv:
+                sv.R = tc.thin_expand(inp.view())
+                wpk, sg = sv.packed_thin("fprop")
+                out_t = tc.thin_fprop(sv.R, wpk, b, d.c, cout, *epi_act, stats=stats, sigma=sg)
+            elif p.fwd == "thin":      # ConvTranspose onto the image: GEMM over input pixels + col2im epilogue
+                wpk, sg = sv.packed_thin("dgrad")
+                out_t = tc.thin_dgrad(inp.t, wpk, b, d.c, *epi_act, sigma=sg)
+            elif p.fwd == "dense_T":
+                sv.a = tc.pad_rows(inp.t.reshape(d.n, d.k), _r64(d.k))
+                out_t = tc.dense_scatter(sv.a, tc.dense_pack(sv.values(), _r64(d.k), False), b, d.c)
+            elif p.fwd == "dense_C":
+                out_t = tc.dense_gather(inp.t, tc.dense_pack(sv.values(), 32, True), b, d.k).view(out_shape)
+            elif p.fwd == "tc" and conv:
+                wpk, sg = sv.packed("fprop", p.ca)
+                out_t = tc.fprop(inp.t, wpk, b, cout, *epi_act, out_f32_nchw=last, stats=stats, sigma=sg)
+            elif p.fwd == "tc":
+                wpk, sg = sv.packed("dgrad", p.ca)
+                out_t = tc.dgrad(inp.t, wpk, b, p.ca, *epi_act, out_f32_nchw=last, stats=stats,
+                                 c_real=d.c if p.ca != d.c else 0, sigma=sg)
             else:
-                inp = cur
-                if last:
-                    out = _Buf(torch.empty(out_shape, device=dev, dtype=torch.float32), "ext")
-                else:
-                    out = _Buf(tc.alloc_padded(out_shape[0], out_shape[2], out_shape[3], cout, dev), "pad")
-                ind, outd = t4(inp.view()), t4(out.view())
-                call("eadgan_conv_fprop" if st.kind == "conv" else "eadgan_conv_dgrad", C.byref(d), C.byref(ind),
-                     ptr(wvals()), ptr(b), epi_act[0], float(epi_act[1]), C.byref(outd), None, ACT_NONE, 0.0, st_)
+                out_t = (torch.empty(out_shape, device=dev, dtype=torch.float32) if last
+                         else tc.alloc_padded(out_shape[0], out_shape[2], out_shape[3], cout, dev))
+                ind, outd = t4(inp.view()), t4(out_t if last else tc.interior(out_t))
+                call("eadgan_conv_fprop" if conv else "eadgan_conv_dgrad", C.byref(d), C.byref(ind),
+                     ptr(sv.values()), ptr(b), epi_act[0], float(epi_act[1]), C.byref(outd), None, ACT_NONE, 0.0, st_)
                 if stats is not None:
                     call("eadgan_bn_stats", C.byref(outd), out_shape[0], cout, out_shape[2], out_shape[3],
                          ptr(stats), st_)
-            rec["inp"] = inp
+            out = _Buf(out_t, p.out_fmt)
+            sv.inp = inp
             if st.bn is not None:
                 bn = st.bn
+                gamma, beta = params[pi - 2], params[pi - 1]
                 n_local = float(out_shape[0] * out_shape[2] * out_shape[3])
                 count = n_local
                 sum_x = stats                      # this rank's S(x) (first C entries), kept for backward
@@ -498,67 +538,67 @@ class _ChainFn(torch.autograd.Function):
                 xd, yd = t4(out.view()), t4(y.view())
                 call("eadgan_bn_apply", C.byref(xd), out_shape[0], cout, out_shape[2], out_shape[3], ptr(mean),
                      ptr(invstd), ptr(gamma), ptr(beta), st.act[0], float(st.act[1]), C.byref(yd), st_)
-                rec.update(pre=out, mean=mean, invstd=invstd, gamma=gamma, beta=beta, count=count, n_local=n_local,
-                           sum_x=sum_x)
+                sv.pre, sv.mean, sv.invstd, sv.gamma, sv.beta = out, mean, invstd, gamma, beta
+                sv.count, sv.n_local, sv.sum_x = count, n_local, sum_x
                 out = y
-            rec["y"] = out
+            sv.y = out
             if gate_log is not None and st.act[0] in (L.ACT_RELU, L.ACT_LRELU):
                 gate_log[-1][1].append(out.view() > 0)
-            saved.append(rec)
+            saved.append(sv)
             cur = out
         # the returned tensor is saved through autograd (no ctx <-> output reference cycle)
-        saved[-1]["y"] = None
+        saved[-1].y = None
         ctx.save_for_backward(cur.t)
-        ctx.stages, ctx.saved = stages, saved
+        ctx.stages, ctx.plans, ctx.saved = stages, plans, saved
         return cur.t
 
     @staticmethod
     def backward(ctx, gout):
-        stages, saved = ctx.stages, ctx.saved
-        saved[-1]["y"] = _Buf(ctx.saved_tensors[0], "ext")
+        stages, plans, saved = ctx.stages, ctx.plans, ctx.saved
+        saved[-1].y = _Buf(ctx.saved_tensors[0], "ext")
         st_ = stream()
         dev = gout.device
         g = _Buf(gout.contiguous(), "ext")
         g_masked = False
         db_sums = None   # fp64 per-channel sums of g, accumulated by the epilogue of the kernel that produced g
         grads = []
-        arena = _Arena(sum(3 * max(sv_["d"].k, sv_["d"].c) for sv_ in saved), dev)   # every fp64 sum vector of this backward
+        arena = _Arena(sum(3 * max(p.d.k, p.d.c) for p in plans), dev)   # every fp64 sum vector of this backward
         for si in range(len(stages) - 1, -1, -1):
-            st, sv = stages[si], saved[si]
-            d, impl = sv["d"], sv["impl"]
-            cout = d.k if st.kind == "conv" else d.c
-            n, _, oh, ow = sv["y"].nchw
+            st, p, sv = stages[si], plans[si], saved[si]
+            d, conv = p.d, st.kind == "conv"
+            n, cout, oh, ow = p.out_shape
             dgamma = dbeta = None
             # which parameter gradients autograd actually wants (inputs: x, stages, srcs, then w, b[, gamma, beta] per
             # stage).  A step driver freezes the networks a phase's optimiser does not own (phase G: D), so their
             # weight-gradient GEMMs, bias sums and spectral-norm backward are never launched (SURVEY.md section 7.3-8)
-            need_dw = ctx.needs_input_grad[3 + sv["pi"]]
-            need_db = sv["has_b"] and ctx.needs_input_grad[3 + sv["pi"] + 1]
+            need_dw = ctx.needs_input_grad[3 + sv.pi]
+            need_db = sv.has_b and ctx.needs_input_grad[3 + sv.pi + 1]
+            need_dx = si > 0 or ctx.needs_input_grad[0]
             # ---- 1. gradient w.r.t. the conv output (pre-BN / pre-activation) ----------------
             if st.bn is not None:
                 sums = arena.take(2 * cout)
-                gd, xd, yd = t4(g.view()), t4(sv["pre"].view()), t4(sv["y"].view())
-                call("eadgan_bn_bwd_reduce", C.byref(gd), C.byref(xd), C.byref(yd), n, cout, oh, ow, ptr(sv["mean"]),
-                     ptr(sv["invstd"]), ptr(sv["gamma"]), ptr(sv["beta"]), st.act[0], float(st.act[1]), ptr(sums), st_)
+                gd, xd, yd = t4(g.view()), t4(sv.pre.view()), t4(sv.y.view())
+                call("eadgan_bn_bwd_reduce", C.byref(gd), C.byref(xd), C.byref(yd), n, cout, oh, ow, ptr(sv.mean),
+                     ptr(sv.invstd), ptr(sv.gamma), ptr(sv.beta), st.act[0], float(st.act[1]), ptr(sums), st_)
                 local = sums
                 if Fn._allreduce_sum is not None:
                     local = sums.clone()
                     Fn._allreduce_sum(sums)
-                call("eadgan_bn_bwd_apply", C.byref(gd), C.byref(xd), C.byref(yd), n, cout, oh, ow, ptr(sv["mean"]),
-                     ptr(sv["invstd"]), ptr(sv["gamma"]), ptr(sv["beta"]), st.act[0], float(st.act[1]), ptr(sums),
-                     float(sv["count"]), C.byref(gd), st_)  # in place: dz overwrites g
+                call("eadgan_bn_bwd_apply", C.byref(gd), C.byref(xd), C.byref(yd), n, cout, oh, ow, ptr(sv.mean),
+                     ptr(sv.invstd), ptr(sv.gamma), ptr(sv.beta), st.act[0], float(st.act[1]), ptr(sums),
+                     float(sv.count), C.byref(gd), st_)  # in place: dz overwrites g
                 # dgamma / dbeta, and the conv-bias gradient (= sum of dx, zero up to rounding) in closed
                 # form from the fp64 sums: no extra pass over dz
                 small = torch.empty(3 * cout, device=dev, dtype=torch.float32)
                 dgamma, dbeta, db_bn = small[:cout], small[cout:2 * cout], small[2 * cout:]
-                call("eadgan_bn_bwd_finalize", ptr(local), ptr(sums), ptr(sv["sum_x"]), float(sv["n_local"]),
-                     float(sv["count"]), ptr(sv["mean"]), ptr(sv["invstd"]), ptr(sv["gamma"]), cout, ptr(dgamma),
-                     ptr(dbeta), ptr(db_bn) if sv["has_b"] else None, st_)
+                call("eadgan_bn_bwd_finalize", ptr(local), ptr(sums), ptr(sv.sum_x), float(sv.n_local),
+                     float(sv.count), ptr(sv.mean), ptr(sv.invstd), ptr(sv.gamma), cout, ptr(dgamma),
+                     ptr(dbeta), ptr(db_bn) if sv.has_b else None, st_)
                 dz = g
             elif st.act[0] != ACT_NONE and not g_masked:
-                if g.fmt != "ext" or sv["y"].fmt != "ext":
+                if g.fmt != "ext" or sv.y.fmt != "ext":
                     raise RuntimeError("eadgan_b200.chain: unfused activation backward on a private buffer")
-                dz = _Buf(Fn.act_bwd(g.t, sv["y"].t, st.act[0], st.act[1]), "ext")
+                dz = _Buf(Fn.act_bwd(g.t, sv.y.t, st.act[0], st.act[1]), "ext")
             else:
                 dz = g
             if not need_db:
@@ -571,112 +611,73 @@ class _ChainFn(torch.autograd.Function):
             else:
                 db = _chan_sums(dz, cout)
             db_sums = None
-            prev = stages[si - 1] if si > 0 else None
-            need_dx = si > 0 or ctx.needs_input_grad[0]
-            fuse = need_dx and prev is not None and prev.bn is None and prev.act[0] != ACT_NONE
-            mask_act, mask_slope = (prev.act if fuse else (ACT_NONE, 0.0))
-            in_shape = (d.n, d.c, d.h, d.w) if st.kind == "conv" else (d.n, d.k, d.p, d.q)
-            dx = None
-            # the dx computed here IS the previous stage's pre-activation gradient when that stage has no BN and
-            # its activation backward is fused (or absent): let the producing epilogue also sum it per channel
-            # (= that stage's bias gradient), instead of a separate pass over dx
-            want_sums = (need_dx and prev is not None and prev.bn is None and saved[si - 1]["has_b"]
-                         and ctx.needs_input_grad[3 + saved[si - 1]["pi"] + 1]
-                         and (fuse or prev.act[0] == ACT_NONE) and in_shape[1] <= 1024)
-            sums_buf = arena.take(in_shape[1]) if want_sums else None
-            sums_used = False
-            # ---- 2./3. weight gradient and input gradient -----------------------------------------
-            if impl == "thin":
-                dw = None
-                if st.kind == "conv":      # big map = stage input (image), small map = dz
-                    r = sv["R"]
-                    if not need_dw:
-                        pass
-                    elif _thin_ok(d, "wgrad"):
-                        dw = tc.thin_wgrad(r, dz.padded(), d.c)
-                    else:
-                        dw = torch.empty_like(sv["w"])
-                        Fn.conv_wgrad(d, t4(sv["inp"].view()), t4(dz.view()), dw)
-                    if need_dx and si == 0 and _thin_ok(d, "dgrad"):
-                        wpk, sg = sv["packed_thin"]("dgrad")
-                        dx = _Buf(tc.thin_dgrad(dz.padded(), wpk, None, d.c, sigma=sg), "ext")
-                else:                      # big map = dz (image gradient), small map = stage input
-                    r = tc.thin_expand(dz.view()) if (need_dw or (need_dx and si > 0)) else None
-                    if not need_dw:
-                        pass
-                    elif _thin_ok(d, "wgrad"):
-                        dw = tc.thin_wgrad(r, sv["inp"].t, d.c)
-                    else:
-                        dw = torch.empty_like(sv["w"])
-                        Fn.conv_wgrad(d, t4(dz.view()), t4(sv["inp"].view()), dw)
-                    if need_dx and si > 0:
-                        wpk, sg = sv["packed_thin"]("fprop")
-                        dx = _Buf(tc.thin_fprop(r, wpk, None, d.c, in_shape[1], mask=sv["inp"].t if fuse else None,
-                                                mask_mode=mask_act, slope=mask_slope, stats=sums_buf, stats_mode=2,
-                                                sigma=sg), "pad")
-                        sums_used = want_sums
-            elif impl == "dense_T":
-                dw = tc.dense_wgrad(sv["a"], dz.padded(), d.k) if need_dw else None
-            elif impl == "dense_C":
+            # the dx computed here IS the previous stage's pre-activation gradient when that stage has no BN (its
+            # activation backward, if any, is fused): let the producing epilogue also sum it per channel (= that
+            # stage's bias gradient), instead of a separate pass over dx
+            want_sums = (si > 0 and stages[si - 1].bn is None and saved[si - 1].has_b
+                         and ctx.needs_input_grad[3 + saved[si - 1].pi + 1] and p.in_shape[1] <= 1024)
+            sums_buf = arena.take(p.in_shape[1]) if want_sums else None
+            # ---- 2. weight gradient ------------------------------------------------------------------
+            x_big, dy_small = (sv.inp, dz) if conv else (dz, sv.inp)
+            r, a = sv.R, sv.a       # row-expanded image (thin) / small map as GEMM rows (dense) of the forward
+            if p.fwd == "thin" and not conv and (need_dw or (need_dx and p.dx == "thin")):
+                r = tc.thin_expand(dz.view())          # the image gradient is this stage's big map
+            if p.fwd == "dense_C":
                 a = tc.pad_rows(dz.t.reshape(d.n, d.k), 64)
-                dw = tc.dense_wgrad(a, sv["inp"].t, d.k) if need_dw else None
-                if need_dx and (si > 0) and (not fuse or sv["inp"].fmt == "pad"):
-                    dx = _Buf(tc.dense_scatter(a, tc.dense_pack(sv["wvals"](), 64, False), None, d.c,
-                                               mask=sv["inp"].t if fuse else None, mask_act=mask_act,
-                                               slope=mask_slope, chan_sums=sums_buf), "pad")
-                    sums_used = want_sums
+            dw = None
+            if not need_dw:
+                pass
+            elif p.wgrad == "thin":
+                dw = tc.thin_wgrad(r, dy_small.padded(), d.c)
+            elif p.wgrad == "dense":
+                dw = tc.dense_wgrad(a, x_big.padded(), d.k)
+            elif p.wgrad == "tc":
+                xb = x_big.t if x_big.fmt == "pad" else tc.to_padded(x_big.t, p.ca)
+                if not conv and p.ca != d.c:
+                    dz = _Buf(xb, "pad")  # reuse the channel-padded copy for the input gradient below
+                dw = tc.wgrad(xb, dy_small.padded(), c_real=d.c if p.ca != d.c else 0)
             else:
-                ca = _calloc(d) if impl == "tc" else d.c
-                x_big, dy_small = (sv["inp"], dz) if st.kind == "conv" else (dz, sv["inp"])
-                if not need_dw:
-                    dw = None
-                elif impl == "tc" and _tc_ok(d, "wgrad"):
-                    xb = x_big.t if x_big.fmt == "pad" else tc.to_padded(x_big.t, ca)
-                    if st.kind == "convT" and ca != d.c:
-                        dz = _Buf(xb, "pad")  # reuse the channel-padded copy for the input gradient below
-                        x_big = dz
-                    dw = tc.wgrad(xb, dy_small.padded(), c_real=d.c if ca != d.c else 0)
-                else:
-                    dw = torch.empty_like(sv["w"])
-                    Fn.conv_wgrad(d, t4(x_big.view()), t4(dy_small.view()), dw)
-                if need_dx:
-                    direction = "dgrad" if st.kind == "conv" else "fprop"
-                    tc_dx = impl == "tc" and _tc_ok(d, direction) and (not fuse or sv["inp"].fmt == "pad")
-                    if tc_dx and ca != d.c and st.kind == "conv" and si > 0:
-                        tc_dx = False  # zero-padded result channels need the fp32 NCHW epilogue (si == 0)
-                    if tc_dx:
-                        wpk, sg = sv["packed"](direction, ca)
-                        if st.kind == "conv":
-                            dx_t = tc.dgrad(dz.padded(), wpk, None, ca, mask=sv["inp"].t if fuse else None,
-                                            mask_mode=mask_act, slope=mask_slope, out_f32_nchw=(si == 0),
-                                            c_real=d.c if ca != d.c else 0, stats=sums_buf, stats_mode=2, sigma=sg)
-                        else:
-                            dzp = dz.t if dz.fmt == "pad" else tc.to_padded(dz.t, ca)
-                            dx_t = tc.fprop(dzp, wpk, None, in_shape[1], mask=sv["inp"].t if fuse else None,
-                                            mask_mode=mask_act, slope=mask_slope, out_f32_nchw=(si == 0),
-                                            stats=sums_buf, stats_mode=2, sigma=sg)
-                        dx = _Buf(dx_t, "ext" if si == 0 else "pad")
-                        sums_used = want_sums
-            if need_dx and dx is None:   # generic SIMT input gradient on the same buffers
-                if si > 0:
-                    dx = _Buf(tc.alloc_padded(in_shape[0], in_shape[2], in_shape[3], in_shape[1], dev), "pad")
-                else:
-                    dx = _Buf(torch.empty(in_shape, device=dev, dtype=torch.float32), "ext")
-                dzv = dz.view()
-                if dzv.shape[1] != cout:
-                    dzv = dzv[:, :cout]
-                dzd, dxd = t4(dzv), t4(dx.view())
-                md = t4(sv["inp"].view()) if fuse else None
-                call("eadgan_conv_dgrad" if st.kind == "conv" else "eadgan_conv_fprop", C.byref(d), C.byref(dzd),
-                     ptr(sv["wvals"]()), None, ACT_NONE, 0.0, C.byref(dxd), C.byref(md) if fuse else None, mask_act,
-                     float(mask_slope), st_)
+                dw = torch.empty_like(sv.w, memory_format=torch.contiguous_format)
+                Fn.conv_wgrad(d, t4(x_big.view()), t4(dy_small.view()), dw)
+            # ---- 3. input gradient -------------------------------------------------------------------
             if need_dx:
-                g, g_masked = dx, fuse
-                db_sums = sums_buf if sums_used else None
+                mask = sv.inp.t if p.fuse else None
+                mask_act, mask_slope = stages[si - 1].act if p.fuse else (ACT_NONE, 0.0)
+                if p.dx == "thin" and conv:
+                    wpk, sg = sv.packed_thin("dgrad")
+                    dx_t = tc.thin_dgrad(dz.padded(), wpk, None, d.c, sigma=sg)
+                elif p.dx == "thin":
+                    wpk, sg = sv.packed_thin("fprop")
+                    dx_t = tc.thin_fprop(r, wpk, None, d.c, d.k, mask=mask, mask_mode=mask_act, slope=mask_slope,
+                                         stats=sums_buf, stats_mode=2, sigma=sg)
+                elif p.dx == "dense":
+                    dx_t = tc.dense_scatter(a, tc.dense_pack(sv.values(), 64, False), None, d.c, mask=mask,
+                                            mask_act=mask_act, slope=mask_slope, chan_sums=sums_buf)
+                elif p.dx == "tc" and conv:
+                    wpk, sg = sv.packed("dgrad", p.ca)
+                    dx_t = tc.dgrad(dz.padded(), wpk, None, p.ca, mask=mask, mask_mode=mask_act, slope=mask_slope,
+                                    out_f32_nchw=si == 0, c_real=d.c if p.ca != d.c else 0, stats=sums_buf,
+                                    stats_mode=2, sigma=sg)
+                elif p.dx == "tc":
+                    wpk, sg = sv.packed("fprop", p.ca)
+                    dzp = dz.t if dz.fmt == "pad" else tc.to_padded(dz.t, p.ca)
+                    dx_t = tc.fprop(dzp, wpk, None, d.k, mask=mask, mask_mode=mask_act, slope=mask_slope,
+                                    out_f32_nchw=si == 0, stats=sums_buf, stats_mode=2, sigma=sg)
+                else:
+                    ic, ih, iw = p.in_shape[1:]
+                    dx_t = (tc.alloc_padded(d.n, ih, iw, ic, dev) if si > 0
+                            else torch.empty(p.in_shape, device=dev, dtype=torch.float32))
+                    dzd, dxd = t4(dz.view()), t4(dx_t if si == 0 else tc.interior(dx_t))
+                    md = t4(sv.inp.view()) if p.fuse else None
+                    call("eadgan_conv_dgrad" if conv else "eadgan_conv_fprop", C.byref(d), C.byref(dzd),
+                         ptr(sv.values()), None, ACT_NONE, 0.0, C.byref(dxd), C.byref(md) if p.fuse else None,
+                         mask_act, float(mask_slope), st_)
+                g, g_masked = _Buf(dx_t, "ext" if si == 0 else "pad"), p.fuse
+                db_sums = sums_buf if p.dx != "simt" else None
             stage_grads = [dw, db]
             if st.bn is not None:
                 stage_grads += [dgamma, dbeta]
             grads = stage_grads + grads
         dx0 = g.t if ctx.needs_input_grad[0] else None
-        ctx.saved = None
+        ctx.saved = ctx.plans = None
         return (dx0, None, None, *grads)

@@ -15,6 +15,7 @@ import ctypes as C
 import torch
 
 from . import _lib as L
+from . import tc
 from ._lib import ACT_NONE, ACT_LRELU, ACT_RELU, ACT_SIGMOID, ACT_TANH, call, ptr, stream, t4
 
 # ----------------------------------------------------------------------------------
@@ -70,20 +71,11 @@ def channel_sum(t):
 # ----------------------------------------------------------------------------------
 # convolution family (fp32 SIMT path)
 # ----------------------------------------------------------------------------------
-_ws_cache = {}
-
-
 def conv_wgrad(d, x_t4, dy_t4, dw):
-    """dw (overwritten) = SIMT weight gradient; split partials go through a per-(device, stream) workspace owned
-    here (the library allocates nothing) and are summed in a fixed order: deterministic."""
+    """dw (overwritten) = SIMT weight gradient; split partials go through the per-(device, stream) workspace of
+    eadgan_b200.tc (the library allocates nothing) and are summed in a fixed order: deterministic."""
     need = L.lib().eadgan_conv_wgrad_workspace(C.byref(d))
-    ws = None
-    if need:
-        key = (dw.device, torch.cuda.current_stream().cuda_stream)
-        ws = _ws_cache.get(key)
-        if ws is None or ws.numel() < need:
-            ws = torch.empty(need, device=dw.device, dtype=torch.uint8)
-            _ws_cache[key] = ws
+    ws = tc._workspace(need, dw.device) if need else None
     call("eadgan_conv_wgrad", C.byref(d), C.byref(x_t4), C.byref(dy_t4), ptr(dw), ptr(ws),
          C.c_size_t(need), stream())
 

@@ -64,9 +64,7 @@ class GraphedStep:
         # graph: tc.clear_pool(), or a larger workspace replacing a cache entry, can then no longer free memory under
         # the graph.  (The warm-up steps filled the pool, so capture creates almost no buffer: a buffer first created
         # INSIDE a capture has its zero fill recorded and re-executed by every replay.)
-        from . import functional as Fn
-        self._keepalive = ([b for free in tc._pool.values() for b in free] + births + list(tc._ws_cache.values())
-                           + list(Fn._ws_cache.values()))
+        self._keepalive = [b for free in tc._pool.values() for b in free] + births + list(tc._ws_cache.values())
         tc.invalidate_caches()
         self.kernels_per_replay = int(_lib.lib().eadgan_kernel_launches() - k0)
         self._first = True

@@ -61,8 +61,6 @@ def clear_pool():
     _pool_gen += 1
     _pool.clear()
     _ws_cache.clear()
-    from . import functional as Fn
-    Fn._ws_cache.clear()
 
 
 def interior(xp):
@@ -114,18 +112,25 @@ _pack_cache = {}
 
 def pack_w_cached(param, direction="fprop", c_alloc=None):
     """pack_w of a PARAMETER object (a G weight, or the weight_orig of a spectral-normalised layer), cached until
-    the parameter changes: torch's version counter catches in-place torch ops (load_state_dict, stock
-    optimisers), the ``_eadgan_stepped`` serial our fused Adam leaves on every parameter it updates (through raw
-    pointers) catches that one, _lib.weights_epoch everything wholesale (load_state_dict, graph replays).  Entries are
-    tied to the parameter OBJECT (weak reference), never to an address that a later tensor could reuse.  Code
-    that rewrites a parameter through ``.data`` must call eadgan_b200.invalidate_caches()."""
-    key = (id(param), direction, c_alloc)
+    the parameter changes (``_cached_pack``)."""
+    return _cached_pack(param, "wide", direction, c_alloc)
+
+
+def _cached_pack(param, kind, direction, c_alloc):
+    """pack_w ("wide") or thin_pack_w ("thin") of a parameter, cached until the parameter changes: torch's version
+    counter catches in-place torch ops (load_state_dict, stock optimisers), the ``_eadgan_stepped`` serial our fused
+    Adam leaves on every parameter it updates (through raw pointers) catches that one, _lib.weights_epoch everything
+    wholesale (load_state_dict, graph replays).  Entries are tied to the parameter OBJECT (weak reference), never to
+    an address that a later tensor could reuse.  Code that rewrites a parameter through ``.data`` must call
+    eadgan_b200.invalidate_caches()."""
+    key = (id(param), direction if kind == "wide" else "thin_" + direction, c_alloc)
     token = (param._version, param.data_ptr(), L.weights_epoch, getattr(param, "_eadgan_stepped", 0))
-    _note_use(param, "wide", direction, c_alloc)
+    _note_use(param, kind, direction, c_alloc)
     hit = _pack_cache.get(key)
     if hit is not None and hit[0]() is param and hit[1] == token:
         return _adopt(hit)
-    out = pack_w(param.detach(), None, direction, c_alloc)
+    w = param.detach()
+    out = thin_pack_w(w, direction) if kind == "thin" else pack_w(w, None, direction, c_alloc)
     if hit is None or hit[0]() is not param:
         weakref.finalize(param, _pack_cache.pop, key, None)
     _pack_cache[key] = (weakref.ref(param), token, out) + _built_on()
@@ -173,10 +178,7 @@ def prefetch_packs(param):
     _ahead = True
     try:
         for kind, direction, c_alloc in tuple(getattr(param, "_eadgan_pack_uses", ())):
-            if kind == "thin":
-                thin_pack_w_cached(param, direction)
-            else:
-                pack_w_cached(param, direction, c_alloc)
+            _cached_pack(param, kind, direction, c_alloc)
     finally:
         _ahead = False
 
@@ -222,6 +224,8 @@ _ws_cache = {}
 
 
 def _workspace(need, device):
+    """scratch of at least ``need`` bytes for the kernels that split a reduction over CTAs (every wgrad, the dense
+    gather): one per (device, stream), reused by every such launch on that stream, grown when a launch needs more"""
     key = (device, torch.cuda.current_stream().cuda_stream)
     ws = _ws_cache.get(key)
     if ws is None or ws.numel() < need:
@@ -302,17 +306,8 @@ def thin_pack_w(w, direction):
 
 
 def thin_pack_w_cached(param, direction):
-    key = (id(param), "thin_" + direction, None)
-    token = (param._version, param.data_ptr(), L.weights_epoch, getattr(param, "_eadgan_stepped", 0))
-    _note_use(param, "thin", direction, None)
-    hit = _pack_cache.get(key)
-    if hit is not None and hit[0]() is param and hit[1] == token:
-        return _adopt(hit)
-    out = thin_pack_w(param.detach(), direction)
-    if hit is None or hit[0]() is not param:
-        weakref.finalize(param, _pack_cache.pop, key, None)
-    _pack_cache[key] = (weakref.ref(param), token, out) + _built_on()
-    return out
+    """thin_pack_w of a parameter, cached until it changes (``_cached_pack``)."""
+    return _cached_pack(param, "thin", direction, None)
 
 
 def thin_fprop(r, wpk, bias, c, k, act=ACT_NONE, slope=0.0, mask=None, mask_mode=0, stats=None, stats_mode=1, sigma=None,

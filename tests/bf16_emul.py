@@ -48,6 +48,7 @@ def emulate(ours_seq, ref_seq, x, update_running=False):
     ref_seq: torch.nn.Sequential with the same layout holding the parameters to differentiate."""
     stages = chain._compile(ours_seq)
     assert stages is not None, "not a chain-able Sequential"
+    plans = chain._plan_kernels(stages, tuple(x.shape))
     idx = {id(m): i for i, m in enumerate(ours_seq._modules.values())}
     ref_mods = list(ref_seq._modules.values())
     h = x
@@ -56,8 +57,7 @@ def emulate(ours_seq, ref_seq, x, update_running=False):
         conv = ref_mods[idx[id(st.conv)]]
         for hook in conv._forward_pre_hooks.values():  # spectral norm on the torch side
             hook(conv, (h,))
-        d = chain._geom(st, tuple(h.shape))
-        tensor_core = chain._impl(st, d, last) != "simt"
+        tensor_core = plans[si].fwd != "simt"
         w = conv.weight
         hin = rb(h) if (tensor_core or si > 0) else h   # private buffers / tensor-core operands are bf16
         if tensor_core:

@@ -344,38 +344,78 @@ def test_sass_is_blackwell_native():
         assert mnemonic in sass, mnemonic
 
 
-def test_chain_plans_route_every_celeba_and_dsprites_layer_to_a_tensor_core_kernel():
-    """host logic of the bf16 chain executor (no kernels run): which kernel family each layer of the reference
-    networks is planned on.  Guards the geometry rules (_tc_ok / _thin_ok / dense) against regressions that would
-    silently push a hot layer back to the SIMT kernels."""
+def _kernel_plan(seq, in_shape):
+    """the bf16 chain executor's plan of a conv stack, one line per stage:
+    "forward / weight-gradient / input-gradient family, big-map channels:allocated, small-map channels,
+    input > output buffer format[, fuse]" -- and the stack's output shape"""
     from eadgan_b200 import chain
-    from eadgan_b200.steps import celeba, dsprites
+    stages = chain._plan(seq)
+    assert stages is not None
+    plans = chain._plan_kernels(stages, in_shape)
+    return ([f"{p.fwd}/{p.wgrad}/{p.dx} c{p.d.c}:{p.ca} k{p.d.k} {p.in_fmt}>{p.out_fmt}" + (" fuse" if p.fuse else "")
+             for p in plans], plans[-1].out_shape)
 
-    def impls(seq, in_shape):
-        stages = chain._plan(seq)
-        assert stages is not None
-        out, shape = [], in_shape
-        for i, st in enumerate(stages):
-            d = chain._geom(st, shape)
-            out.append(chain._impl(st, d, i == len(stages) - 1))
-            shape = (d.n, d.k, d.p, d.q) if st.kind == "conv" else (d.n, d.c, d.h, d.w)
-        return out, shape
+
+def test_chain_plans_route_every_celeba_and_dsprites_layer_to_a_tensor_core_kernel():
+    """host logic of the bf16 chain executor (no kernels run): which kernel family runs the forward, the weight
+    gradient and the input gradient of each layer of the reference networks.  Guards the geometry rules (_tc_ok /
+    _thin_ok / dense) against regressions that would silently push a hot layer back to the SIMT kernels."""
+    from eadgan_b200.steps import celeba, dsprites, mnist
 
     torch.manual_seed(0)
-    got, shape = impls(celeba.Generator().conv_blocks, (8, 218, 1, 1))
-    assert got == ["dense_T", "tc", "tc", "tc", "thin"] and shape == (8, 3, 64, 64)
-    got, shape = impls(celeba.Discriminator().main, (8, 3, 64, 64))
-    assert got == ["thin", "tc", "tc", "tc", "dense_C"] and shape == (8, 19, 1, 1)
+    got, shape = _kernel_plan(celeba.Generator().conv_blocks, (8, 218, 1, 1))
+    assert got == ["dense_T/dense/simt c1024:1024 k218 ext>pad",
+                   "tc/tc/tc c512:512 k1024 pad>pad",
+                   "tc/tc/tc c256:256 k512 pad>pad",
+                   "tc/tc/tc c128:128 k256 pad>pad",
+                   "thin/thin/thin c3:3 k128 pad>ext"] and shape == (8, 3, 64, 64), got
+    got, shape = _kernel_plan(celeba.Discriminator().main, (8, 3, 64, 64))
+    assert got == ["thin/thin/thin c3:3 k128 ext>pad",
+                   "tc/tc/tc c128:128 k256 pad>pad fuse",
+                   "tc/tc/tc c256:256 k512 pad>pad fuse",
+                   "tc/tc/tc c512:512 k1024 pad>pad fuse",
+                   "dense_C/dense/dense c1024:1024 k19 pad>ext fuse"] and shape == (8, 19, 1, 1), got
     for ch in (1, 3):
-        got, shape = impls(dsprites.Generator(ch, 4 if ch == 1 else 7).conv_block, (8, 64, 4, 4))
-        assert got == ["tc", "tc", "tc", "thin"] and shape == (8, ch, 64, 64)
-        got, shape = impls(dsprites.Discriminator(ch).conv_block, (8, ch, 64, 64))
-        assert got == ["thin", "tc", "tc", "tc"] and shape == (8, 64, 4, 4)
-    # backward directions of the 32-channel dSprites layers (k = 32: zero-filled 64-wide TMA boxes)
-    d32 = chain._geom(chain._plan(dsprites.Discriminator(1).conv_block)[1], (8, 32, 32, 32))
-    assert chain._tc_ok(d32, "dgrad") and chain._tc_ok(d32, "wgrad")
-    d0 = chain._geom(chain._plan(dsprites.Discriminator(1).conv_block)[0], (8, 1, 64, 64))
-    assert chain._thin_ok(d0, "dgrad") and chain._thin_ok(d0, "wgrad")
+        got, shape = _kernel_plan(dsprites.Generator(ch, 4 if ch == 1 else 7).conv_block, (8, 64, 4, 4))
+        assert got == ["tc/tc/tc c64:64 k64 pad>pad"] * 3 + [f"thin/thin/thin c{ch}:{ch} k64 pad>ext"], got
+        assert shape == (8, ch, 64, 64)
+        # k = 32 layers: zero-filled 64-wide TMA boxes in both backward directions
+        trunk = [f"thin/thin/thin c{ch}:{ch} k32 ext>pad", "tc/tc/tc c32:32 k32 pad>pad fuse",
+                 "tc/tc/tc c32:32 k64 pad>pad fuse", "tc/tc/tc c64:64 k64 pad>ext fuse"]
+        for net in (dsprites.Discriminator(ch), dsprites.Encoder(ch), dsprites.Encoder_pxy(ch)):
+            got, shape = _kernel_plan(net.conv_block, (8, ch, 64, 64))
+            assert got == trunk and shape == (8, 64, 4, 4), (type(net).__name__, got)
+    # 3x3 stride-2 convs: no tensor-core kernel covers them
+    got, shape = _kernel_plan(mnist.Discriminator().conv_blocks, (8, 1, 32, 32))
+    assert got == ["simt/simt/simt c1:1 k16 ext>pad", "simt/simt/simt c16:16 k32 pad>pad fuse",
+                   "simt/simt/simt c32:32 k64 pad>pad fuse", "simt/simt/simt c64:64 k128 pad>ext fuse"], got
+    assert shape == (8, 128, 2, 2)
+
+
+def test_chain_plans_of_small_and_channel_padded_stacks():
+    """the plan of the stacks tests/test_chain_gpu.py runs, and of layers whose big map has 5..31 channels (zero-padded
+    to 32 on the tensor-core path), which no reference network has"""
+    import eadgan_b200.nn as enn
+    from test_chain_gpu import SMALL, _build
+
+    plans = {name: _kernel_plan(_build(enn, spec), shape) for name, spec, shape in SMALL}
+    assert plans["dsprites_trunk"] == (["tc/tc/tc c32:32 k32 pad>pad", "tc/tc/tc c32:32 k64 pad>pad fuse",
+                                        "tc/tc/tc c64:64 k64 pad>ext fuse"], (6, 64, 4, 4))
+    # a 16-wide image is not the 32-wide one of the thin input-gradient kernel: the tensor-core path pads 1 -> 32
+    assert plans["dsprites_G"] == (["tc/tc/tc c64:64 k64 pad>pad"] * 2 + ["tc/tc/tc c1:32 k64 pad>ext"], (6, 1, 32, 32))
+    # first stage: the input gradient has zero-padded channels too, written by the fp32 NCHW epilogue
+    seq = enn.Sequential(enn.Conv2d(16, 64, 4, 2, 1), enn.LeakyReLU(0.2), enn.Conv2d(64, 64, 4, 2, 1))
+    assert _kernel_plan(seq, (8, 16, 32, 32)) == (["tc/tc/tc c16:32 k64 pad>pad", "tc/tc/tc c64:64 k64 pad>ext fuse"],
+                                                  (8, 64, 8, 8))
+    # last stage: the forward writes fp32 NCHW; the weight gradient's channel-padded copy of dz feeds the input gradient
+    seq = enn.Sequential(enn.ConvTranspose2d(64, 64, 4, 2, 1), enn.ReLU(), enn.ConvTranspose2d(64, 16, 4, 2, 1))
+    assert _kernel_plan(seq, (8, 64, 8, 8)) == (["tc/tc/tc c64:64 k64 pad>pad", "tc/tc/tc c16:32 k64 pad>ext fuse"],
+                                                (8, 16, 32, 32))
+    # not last: a ConvTranspose onto 16 channels runs on SIMT, and so does a later conv's input gradient.  (Only the
+    # rules are pinned here: that conv's tensor-core forward gets an unpadded 16-channel buffer, which tc_fprop rejects)
+    seq = enn.Sequential(enn.ConvTranspose2d(64, 16, 4, 2, 1), enn.LeakyReLU(0.2), enn.Conv2d(16, 64, 4, 2, 1))
+    assert _kernel_plan(seq, (8, 64, 8, 8)) == (["simt/simt/simt c16:16 k64 ext>pad", "tc/tc/simt c16:32 k64 pad>ext fuse"],
+                                                (8, 64, 8, 8))
 
 
 def test_header_is_plain_c():
