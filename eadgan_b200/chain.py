@@ -332,8 +332,16 @@ def _thin_ok(d, direction):
     return d.k % 32 == 0 and d.q <= 64  # wgrad
 
 
+# the tensor-core epilogues stage a fused bias and accumulate fused BatchNorm statistics for at most this many output
+# channels (STAT_MAX_CH in csrc/tc_conv.cu)
+FUSE_MAX_CH = 1024
+
+
 def _impl(st, d, last):
     """which kernel family runs the forward of this stage (called by _plan_kernels)."""
+    out_ch = d.k if st.kind == "conv" else d.c
+    if out_ch > FUSE_MAX_CH and (st.conv.bias is not None or st.bn is not None):
+        return "simt"      # bias / statistics too wide for the fused epilogues: the SIMT kernels have no such limit
     unit = d.r == 4 and d.stride == 1 and d.pad == 0 and d.h == 4 and d.w == 4 and d.p == 1 and d.q == 1
     plain = st.bn is None and st.act[0] == ACT_NONE
     if unit and plain and d.c % 128 == 0:
@@ -488,8 +496,13 @@ class _ChainFn(torch.autograd.Function):
             cout = out_shape[1]
             epi_act = st.act if st.bn is None else (ACT_NONE, 0.0)
             stats = arena.take(2 * cout) if st.bn is not None else None
-            # a conv reads its big map zero-padded to p.ca channels
-            inp = cur if cur.fmt == p.in_fmt else _Buf(tc.to_padded(cur.t, p.ca if conv else None), "pad")
+            # a conv reads its big map zero-padded to p.ca channels: a padded buffer of fewer channels (the output of a
+            # SIMT stage onto 5..31 channels) is copied into a channel-padded one
+            in_c = p.ca if conv else p.in_shape[1]
+            if cur.fmt == p.in_fmt and (cur.fmt == "ext" or cur.t.shape[3] == in_c):
+                inp = cur
+            else:
+                inp = _Buf(tc.to_padded(cur.view(), in_c), "pad")
             if p.fwd == "thin" and conv:
                 sv.R = tc.thin_expand(inp.view())
                 wpk, sg = sv.packed_thin("fprop")

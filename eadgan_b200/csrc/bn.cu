@@ -81,7 +81,7 @@ __device__ void reduce_kind0(const Geo g, double* sums, F f) {
 template <class F>
 __device__ void reduce_kind1(const Geo g, double* sums, F f) {
   __shared__ double sh0[256], sh1[256];
-  const int cb = g.c < 256 ? g.c : 256;      // channels per pass (c is a multiple of cb or < 256)
+  const int cb = g.c < 256 ? g.c : 256;      // channels per pass; the last pass of c > 256 may be partial
   const int lanes = 256 / cb;                // pixel lanes per block (>=1)
   const int tch = threadIdx.x % cb, tl = threadIdx.x / cb;
   const int64_t pixels = (int64_t)g.rows * g.w;
@@ -551,10 +551,10 @@ int make_geo(Geo* g, int n, int c, int h, int w, const eadgan_tensor4* const* ts
     kind = k;
   }
   g->kind = kind; g->n = n; g->c = c; g->h = h; g->w = w;
+  // kind 1 takes any channel count: reduce_kind1 masks the channels past c of a partial last 256-channel pass, and
+  // foreach_elem derives the channel of every element as i % c
   if (kind == 0) { g->rows = n * c; g->inner = h * w; }
   else { g->rows = n * h; g->inner = w * c; }
-  if (kind == 1)
-    EG_REQUIRE(c <= 256 || c % 256 == 0, EADGAN_ERR_UNSUPPORTED, "%s: NHWC needs c<=256 or c%%256==0", who);
   return 0;
 }
 

@@ -411,11 +411,68 @@ def test_chain_plans_of_small_and_channel_padded_stacks():
     seq = enn.Sequential(enn.ConvTranspose2d(64, 64, 4, 2, 1), enn.ReLU(), enn.ConvTranspose2d(64, 16, 4, 2, 1))
     assert _kernel_plan(seq, (8, 64, 8, 8)) == (["tc/tc/tc c64:64 k64 pad>pad", "tc/tc/tc c16:32 k64 pad>ext fuse"],
                                                 (8, 16, 32, 32))
-    # not last: a ConvTranspose onto 16 channels runs on SIMT, and so does a later conv's input gradient.  (Only the
-    # rules are pinned here: that conv's tensor-core forward gets an unpadded 16-channel buffer, which tc_fprop rejects)
+    # not last: a ConvTranspose onto 16 channels runs on SIMT into a 16-channel buffer; the tensor-core conv after it
+    # reads that map channel-padded to 32 (the executor copies it), and its input gradient runs on SIMT
     seq = enn.Sequential(enn.ConvTranspose2d(64, 16, 4, 2, 1), enn.LeakyReLU(0.2), enn.Conv2d(16, 64, 4, 2, 1))
     assert _kernel_plan(seq, (8, 64, 8, 8)) == (["simt/simt/simt c16:16 k64 ext>pad", "tc/tc/simt c16:32 k64 pad>ext fuse"],
                                                 (8, 64, 8, 8))
+    # a bias or BatchNorm statistics on more than 1024 output channels do not fit the fused epilogues: SIMT
+    seq = enn.Sequential(enn.Conv2d(64, 2048, 4, 2, 1), enn.LeakyReLU(0.2), enn.Conv2d(2048, 64, 4, 2, 1))
+    assert _kernel_plan(seq, (8, 64, 8, 8)) == (["simt/simt/simt c64:64 k2048 ext>pad",
+                                                 "tc/tc/tc c2048:2048 k64 pad>ext fuse"], (8, 64, 2, 2))
+    seq = enn.Sequential(enn.Conv2d(64, 2048, 4, 2, 1, bias=False), enn.LeakyReLU(0.2), enn.Conv2d(2048, 64, 4, 2, 1))
+    assert _kernel_plan(seq, (8, 64, 8, 8))[0][0] == "tc/tc/tc c64:64 k2048 pad>pad"
+
+
+# Every (forward, weight gradient, input gradient, input format, output format, fused mask, channel-padded) row and every
+# (BatchNorm, activation) pair that tests/test_chain_stages_gpu.py runs against its fp64 referee.  A planner rule that
+# adds a row makes this test fail until a catalogue entry reaches it.
+CATALOGUE_ROWS = {
+    ("dense_C", "dense", "dense", "pad", "ext", True, False),
+    ("dense_T", "dense", "simt", "ext", "pad", False, False),
+    ("simt", "simt", "simt", "ext", "pad", False, False),
+    ("simt", "simt", "simt", "pad", "ext", True, False),
+    ("simt", "simt", "simt", "pad", "pad", True, False),
+    ("tc", "simt", "tc", "pad", "pad", False, False),
+    ("tc", "tc", "simt", "pad", "ext", False, True),
+    ("tc", "tc", "simt", "pad", "pad", True, False),
+    ("tc", "tc", "simt", "pad", "pad", True, True),
+    ("tc", "tc", "tc", "pad", "ext", False, False),
+    ("tc", "tc", "tc", "pad", "ext", False, True),
+    ("tc", "tc", "tc", "pad", "ext", True, False),
+    ("tc", "tc", "tc", "pad", "ext", True, True),
+    ("tc", "tc", "tc", "pad", "pad", False, False),
+    ("tc", "tc", "tc", "pad", "pad", False, True),
+    ("tc", "tc", "tc", "pad", "pad", True, False),
+    ("thin", "thin", "simt", "ext", "pad", False, False),
+    ("thin", "thin", "simt", "pad", "pad", True, False),
+    ("thin", "thin", "thin", "ext", "pad", False, False),
+    ("thin", "thin", "thin", "pad", "ext", False, False),
+    ("thin", "thin", "thin", "pad", "ext", True, False),
+}
+
+
+def test_stage_catalogue_covers_every_plan_row():
+    from eadgan_b200 import chain
+    from eadgan_b200._lib import ACT_LRELU, ACT_NONE, ACT_RELU, ACT_SIGMOID, ACT_TANH
+    import eadgan_b200.nn as enn
+    from test_chain_stages_gpu import STAGES, build
+
+    rows, pairs, fused_masks = set(), set(), set()
+    for name, spec, shape in STAGES:
+        stages = chain._plan(build(enn, spec))
+        assert stages is not None, name
+        plans = chain._plan_kernels(stages, shape)
+        for si, (st, p) in enumerate(zip(stages, plans)):
+            rows.add((p.fwd, p.wgrad, p.dx, p.in_fmt, p.out_fmt, p.fuse, p.ca != p.d.c))
+            pairs.add((st.bn is not None, st.act[0]))
+            if p.fuse:
+                fused_masks.add((p.dx, stages[si - 1].act[0]))
+    assert rows == CATALOGUE_ROWS, (rows - CATALOGUE_ROWS, CATALOGUE_ROWS - rows)
+    acts = {ACT_NONE, ACT_RELU, ACT_LRELU, ACT_TANH, ACT_SIGMOID}
+    assert pairs == {(bn, a) for bn in (False, True) for a in acts}, pairs
+    # every activation's backward fused into a tensor-core input gradient
+    assert {a for dx, a in fused_masks if dx == "tc"} == acts - {ACT_NONE}, fused_masks
 
 
 def test_header_is_plain_c():

@@ -32,33 +32,105 @@ def test_gemm(cuda, mnk):
 GEOS = [(4, 128, 32, 256), (4, 256, 16, 512), (16, 512, 8, 1024), (3, 128, 32, 256), (8, 32, 32, 64),
         (5, 64, 8, 64), (2, 128, 64, 128), (8, 32, 64, 32), (6, 32, 32, 32), (3, 64, 16, 96)]
 
+# ---- epilogue variants, on two ragged geometries (128 channels: the channel-major dgrad applies; 64 channels: it does
+# not).  Forward epilogue activations, and the fused activation backward of an input gradient (mask = the producer's
+# saved output) with or without the per-channel sums of the final value (stats_mode 2, include/eadgan.h).
+EPI_GEOS = [(3, 128, 32, 256), (5, 64, 8, 64)]
+MASKS = ("relu", "lrelu", "tanh", "sigmoid")
+MASK_SLOPE = 0.2
 
-@pytest.mark.parametrize("geo", GEOS)
-def test_fprop(cuda, geo):
-    """Conv2d(c,k,4,2,1) forward + bias + LeakyReLU, padded NHWC bf16 in and out."""
+
+def _act_id(name):
+    from eadgan_b200 import _lib
+    return {"none": _lib.ACT_NONE, "relu": _lib.ACT_RELU, "lrelu": _lib.ACT_LRELU, "tanh": _lib.ACT_TANH,
+            "sigmoid": _lib.ACT_SIGMOID}[name]
+
+
+def _act_ref(v, name, slope):
+    if name == "relu":
+        return torch.relu(v)
+    if name == "lrelu":
+        return TF.leaky_relu(v, slope)
+    if name == "tanh":
+        return torch.tanh(v)
+    if name == "sigmoid":
+        return torch.sigmoid(v)
+    return v
+
+
+def _saved_output(name, shape, dev):
+    """a bf16 post-activation tensor as a producer of activation ``name`` saves it (exact zeros included for ReLU)"""
+    return _bf(_act_ref(torch.randn(shape, device=dev), name, MASK_SLOPE))
+
+
+def _act_grad_ref(y, name):
+    """the activation derivative through its saved output y (fp64)"""
+    y = y.double()
+    if name == "relu":
+        return (y > 0).double()
+    if name == "lrelu":
+        return torch.where(y > 0, 1.0, MASK_SLOPE).double()
+    if name == "tanh":
+        return 1 - y * y
+    return y * (1 - y)
+
+
+def _check_sums(sums, ref):
+    """per-channel sums against fp64, relative to the largest per-channel sum of |value|"""
+    want = ref.double().sum((0, 2, 3))
+    assert float((sums - want).abs().max() / ref.double().abs().sum((0, 2, 3)).max()) <= 2e-3
+
+
+def _mask_cases(geos, extra=((None, ""),)):
+    return [pytest.param(g, m, s, e, id=f"mask_{m}-stats{s}{tag}-g{j}")
+            for j, g in enumerate(geos) for m in MASKS for s in (0, 2) for e, tag in extra]
+
+
+@pytest.mark.parametrize("geo,act,mask", [pytest.param(g, "lrelu", None, id=f"geo{i}") for i, g in enumerate(GEOS)] +
+                         [pytest.param(g, a, None, id=f"act_{a}-g{j}") for j, g in enumerate(EPI_GEOS)
+                          for a in ("relu", "tanh", "sigmoid")] +
+                         [pytest.param(g, "none", (m, s), id=f"mask_{m}-stats{s}-g{j}") for j, g in enumerate(EPI_GEOS)
+                          for m in MASKS for s in (0, 2)])
+def test_fprop(cuda, geo, act, mask):
+    """Conv2d(c,k,4,2,1) forward + bias + activation, padded NHWC bf16 in and out; and the same kernel as a
+    ConvTranspose input gradient with the producer's activation backward fused (mask) and the per-channel sums."""
     from eadgan_b200 import tc
-    from eadgan_b200._lib import ACT_LRELU
     n, c, h, k = geo
     torch.manual_seed(1)
     x = _bf(torch.randn(n, c, h, h, device=cuda))
     w = _bf(torch.randn(k, c, 4, 4, device=cuda) * 0.05)
     b = torch.randn(k, device=cuda)
-    ref = TF.leaky_relu(TF.conv2d(x, w, b, stride=2, padding=1), 0.1)
     xp = tc.to_padded(x)
     assert torch.equal(tc.from_padded(xp), x)
     wpk = tc.pack_w(w, None, "fprop")
-    out32 = tc.fprop(xp, wpk, b, k, ACT_LRELU, 0.1, out_f32_nchw=True)
+    if mask is not None:
+        mname, stats_mode = mask
+        y = _saved_output(mname, (n, k, h // 2, h // 2), cuda)
+        ref = TF.conv2d(x.double(), w.double(), None, stride=2, padding=1) * _act_grad_ref(y, mname)
+        sums = torch.zeros(k, device=cuda, dtype=torch.float64) if stats_mode else None
+        out = tc.fprop(xp, wpk, None, k, mask=tc.to_padded(y), mask_mode=_act_id(mname), slope=MASK_SLOPE, stats=sums,
+                       stats_mode=2)
+        assert rel_err(tc.from_padded(out), ref) <= 1e-2
+        if stats_mode:
+            _check_sums(sums, ref)
+        return
+    slope = 0.1 if act == "lrelu" else 0.0
+    ref = _act_ref(TF.conv2d(x, w, b, stride=2, padding=1), act, slope)
+    out32 = tc.fprop(xp, wpk, b, k, _act_id(act), slope, out_f32_nchw=True)
     assert rel_err(out32, ref) <= 2e-3
-    outp = tc.fprop(xp, wpk, b, k, ACT_LRELU, 0.1)
+    outp = tc.fprop(xp, wpk, b, k, _act_id(act), slope)
     assert rel_err(tc.from_padded(outp), ref) <= 1e-2
     # halo must still be zero
     assert float(outp[:, 0].abs().max()) == 0 and float(outp[:, :, 0].abs().max()) == 0
     assert float(outp[:, -1].abs().max()) == 0 and float(outp[:, :, -1].abs().max()) == 0
 
 
-@pytest.mark.parametrize("geo", GEOS)
-def test_dgrad(cuda, geo):
-    """ConvTranspose2d(k,c,4,2,1) forward (= conv dgrad) + bias, with fused BN statistics."""
+@pytest.mark.parametrize("geo,act", [pytest.param(g, "none", id=f"geo{i}") for i, g in enumerate(GEOS)] +
+                         [pytest.param(g, a, id=f"act_{a}-g{j}") for j, g in enumerate(EPI_GEOS)
+                          for a in ("relu", "tanh", "sigmoid")])
+def test_dgrad(cuda, geo, act):
+    """ConvTranspose2d(k,c,4,2,1) forward (= conv dgrad) + bias [+ activation], with fused BN statistics of the
+    pre-activation value."""
     from eadgan_b200 import tc
     n, c, h, k = geo
     if k % 64 and k != 32:
@@ -67,34 +139,49 @@ def test_dgrad(cuda, geo):
     y = _bf(torch.randn(n, k, h // 2, h // 2, device=cuda))
     w = _bf(torch.randn(k, c, 4, 4, device=cuda) * 0.05)
     b = torch.randn(c, device=cuda)
-    ref = TF.conv_transpose2d(y, w, b, stride=2, padding=1)
+    pre = TF.conv_transpose2d(y, w, b, stride=2, padding=1)
+    ref = _act_ref(pre, act, 0.0)
     yp = tc.to_padded(y)
     wpk = tc.pack_w(w, None, "dgrad")
     stats = torch.zeros(2 * c, device=cuda, dtype=torch.float64)
-    out32 = tc.dgrad(yp, wpk, b, c, out_f32_nchw=True, stats=stats)
+    out32 = tc.dgrad(yp, wpk, b, c, _act_id(act), out_f32_nchw=True, stats=stats)
     assert rel_err(out32, ref) <= 2e-3
-    assert rel_err(stats[:c], ref.double().sum((0, 2, 3))) <= 2e-3
-    assert rel_err(stats[c:], (ref.double() ** 2).sum((0, 2, 3))) <= 2e-3
-    outp = tc.dgrad(yp, wpk, b, c)
+    assert rel_err(stats[:c], pre.double().sum((0, 2, 3))) <= 2e-3
+    assert rel_err(stats[c:], (pre.double() ** 2).sum((0, 2, 3))) <= 2e-3
+    outp = tc.dgrad(yp, wpk, b, c, _act_id(act))
     assert rel_err(tc.from_padded(outp), ref) <= 1e-2
 
 
-@pytest.mark.parametrize("geo", GEOS)
-def test_dgrad_mask(cuda, geo):
-    """conv backward-data with the LeakyReLU backward of the producer layer fused (mask)."""
+@pytest.mark.parametrize("geo,mask,stats_mode,dgradt",
+                         [pytest.param(g, "lrelu", 0, None, id=f"geo{i}") for i, g in enumerate(GEOS)] +
+                         _mask_cases(EPI_GEOS[:1], ((0, "-pixel_major"), (2, "-channel_major"))) +
+                         _mask_cases(EPI_GEOS[1:], ((0, "-pixel_major"),)))
+def test_dgrad_mask(cuda, monkeypatch, geo, mask, stats_mode, dgradt):
+    """conv backward-data with the activation backward of the producer layer fused (mask), optionally with the
+    per-channel sums of the result (the producer's bias gradient), on the pixel-major and channel-major kernels."""
     from eadgan_b200 import tc
-    from eadgan_b200._lib import ACT_LRELU
     n, c, h, k = geo
     if k % 64 and k != 32:
         pytest.skip("tc dgrad needs k = 32 or k % 64 == 0")
+    if dgradt is not None:
+        monkeypatch.setenv("EADGAN_TC_DGRADT", str(dgradt))
     torch.manual_seed(3)
     dy = _bf(torch.randn(n, k, h // 2, h // 2, device=cuda))
     w = _bf(torch.randn(k, c, 4, 4, device=cuda) * 0.05)
-    act_out = _bf(torch.randn(n, c, h, h, device=cuda))  # saved post-activation tensor of the producer
-    ref = TF.conv_transpose2d(dy, w, None, stride=2, padding=1) * torch.where(act_out > 0, 1.0, 0.1)
+    if dgradt is None:
+        act_out = _bf(torch.randn(n, c, h, h, device=cuda))  # saved post-activation tensor of the producer
+        ref = TF.conv_transpose2d(dy, w, None, stride=2, padding=1) * torch.where(act_out > 0, 1.0, 0.1)
+        slope = 0.1
+    else:
+        act_out = _saved_output(mask, (n, c, h, h), cuda)
+        ref = TF.conv_transpose2d(dy.double(), w.double(), None, stride=2, padding=1) * _act_grad_ref(act_out, mask)
+        slope = MASK_SLOPE
+    sums = torch.zeros(c, device=cuda, dtype=torch.float64) if stats_mode else None
     outp = tc.dgrad(tc.to_padded(dy), tc.pack_w(w, None, "dgrad"), None, c, mask=tc.to_padded(act_out),
-                    mask_mode=ACT_LRELU, slope=0.1)
+                    mask_mode=_act_id(mask), slope=slope, stats=sums, stats_mode=2)
     assert rel_err(tc.from_padded(outp), ref) <= 1e-2
+    if stats_mode:
+        _check_sums(sums, ref)
 
 
 @pytest.mark.parametrize("geo", GEOS)
@@ -151,9 +238,11 @@ def test_channel_padded_image_layers(cuda):
     assert rel_err(outt, reft) <= 2e-3
 
 
-@pytest.mark.parametrize("n", [8, 130, 200])
-def test_dense_layers(cuda, n):
-    """ConvTranspose2d(218,1024,4,1,0) on 1x1 and Conv2d(1024,19,4,1,0) on 4x4 as batch GEMMs."""
+@pytest.mark.parametrize("n,mask,stats_mode", [pytest.param(n, "lrelu", 0, id=str(n)) for n in (8, 130, 200)] +
+                         [pytest.param(130, m, s, id=f"130-mask_{m}-stats{s}") for m in MASKS for s in (0, 2)])
+def test_dense_layers(cuda, n, mask, stats_mode):
+    """ConvTranspose2d(218,1024,4,1,0) on 1x1 and Conv2d(1024,19,4,1,0) on 4x4 as batch GEMMs; the head's input
+    gradient with the producer's activation backward fused, optionally with the per-channel sums of the result."""
     from eadgan_b200 import tc
     from eadgan_b200._lib import ACT_LRELU
     torch.manual_seed(7)
@@ -186,8 +275,20 @@ def test_dense_layers(cuda, n):
     gy = torch.autograd.grad(TF.conv2d(yr, wh, None).view(n, 19), yr, gh)[0]
     ah = tc.pad_rows(gh, 64)
     assert rel_err(tc.dense_wgrad(ah, yp, 19), gwh) <= 2e-3
-    dxp = tc.dense_scatter(ah, tc.dense_pack(wh, 64, False), None, C, mask=yp, mask_act=ACT_LRELU, slope=0.1)
-    assert rel_err(tc.from_padded(dxp), gy * torch.where(y > 0, 1.0, 0.1)) <= 1e-2
+    if stats_mode == 0 and mask == "lrelu":
+        dxp = tc.dense_scatter(ah, tc.dense_pack(wh, 64, False), None, C, mask=yp, mask_act=ACT_LRELU, slope=0.1)
+        assert rel_err(tc.from_padded(dxp), gy * torch.where(y > 0, 1.0, 0.1)) <= 1e-2
+    if n == 130 and mask is not None:
+        # the masked input gradient against fp64 on the same bf16 operands
+        ym = _saved_output(mask, (n, C, 4, 4), cuda)
+        gyd = TF.conv_transpose2d(gh.double().view(n, 19, 1, 1), wh.double())
+        ref = gyd * _act_grad_ref(ym, mask)
+        sums = torch.zeros(C, device=cuda, dtype=torch.float64) if stats_mode else None
+        dxp = tc.dense_scatter(ah, tc.dense_pack(wh, 64, False), None, C, mask=tc.to_padded(ym), mask_act=_act_id(mask),
+                               slope=MASK_SLOPE, chan_sums=sums)
+        assert rel_err(tc.from_padded(dxp), ref) <= 1e-2
+        if stats_mode:
+            _check_sums(sums, ref)
 
 
 # ---- cta_group::2 (CTA pairs): forced on through EADGAN_TC_CG so that small, ragged cases exercise the pair protocol

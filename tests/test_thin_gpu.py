@@ -39,9 +39,14 @@ def test_expand_layout(cuda, geo):
     assert torch.equal(r2[:, :, 1:-1, 1, :c], want[:, :, 0::2, :].permute(0, 2, 3, 1))
 
 
-@pytest.mark.parametrize("geo", GEOS)
-def test_thin_fprop(cuda, geo):
-    """Conv2d(c<=4, k, 4, 2, 1) forward + bias + LeakyReLU (+ 1/sigma), padded NHWC bf16 out."""
+@pytest.mark.parametrize("geo,mask", [pytest.param(g, None, id=f"geo{i}") for i, g in enumerate(GEOS)] +
+                         [pytest.param(g, (m, s, dt), id=f"mask_{m}-stats{s}-dgradt{dt}-g{j}")
+                          for j, g in enumerate([(4, 3, 64, 128), (3, 1, 64, 32)]) for m in ("relu", "lrelu", "tanh", "sigmoid")
+                          for s in (0, 2) for dt in ((0, 2) if g[3] == 128 else (0,))])
+def test_thin_fprop(cuda, monkeypatch, geo, mask):
+    """Conv2d(c<=4, k, 4, 2, 1) forward + bias + LeakyReLU (+ 1/sigma), padded NHWC bf16 out; and the same kernel as the
+    input gradient of a ConvTranspose onto the image, with the producer's activation backward fused (mask) and the
+    per-channel sums of the result, on the pixel-major and (128 channels) channel-major kernels."""
     from eadgan_b200 import tc
     from eadgan_b200._lib import ACT_LRELU
     n, c, h, k = geo
@@ -50,6 +55,19 @@ def test_thin_fprop(cuda, geo):
     w = _bf(torch.randn(k, c, 4, 4, device=cuda) * 0.1)
     b = torch.randn(k, device=cuda)
     sigma = torch.tensor([1.7], device=cuda)
+    if mask is not None:
+        from test_tc_gpu import MASK_SLOPE, _act_grad_ref, _act_id, _check_sums, _saved_output
+        mname, stats_mode, dgradt = mask
+        monkeypatch.setenv("EADGAN_TC_DGRADT", str(dgradt))
+        y = _saved_output(mname, (n, k, h // 2, h // 2), cuda)
+        ref = TF.conv2d(x.double(), w.double(), None, stride=2, padding=1) / 1.7 * _act_grad_ref(y, mname)
+        sums = torch.zeros(k, device=cuda, dtype=torch.float64) if stats_mode else None
+        out = tc.thin_fprop(tc.thin_expand(x), tc.thin_pack_w(w, "fprop"), None, c, k, mask=tc.to_padded(y),
+                            mask_mode=_act_id(mname), slope=MASK_SLOPE, stats=sums, stats_mode=2, sigma=sigma)
+        assert rel_err(tc.from_padded(out), ref) <= 1e-2
+        if stats_mode:
+            _check_sums(sums, ref)
+        return
     ref = TF.leaky_relu(TF.conv2d(x, w / 1.7, b, stride=2, padding=1), 0.1)
     outp = tc.thin_fprop(tc.thin_expand(x), tc.thin_pack_w(w, "fprop"), b, c, k, ACT_LRELU, 0.1, sigma=sigma)
     assert rel_err(tc.from_padded(outp), ref) <= 1e-2
