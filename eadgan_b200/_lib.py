@@ -77,6 +77,7 @@ _PROTOS = {
     "eadgan_bn_bwd_apply": [_T4, _T4, _T4, _I, _I, _I, _I, _P, _P, _P, _P, _I, _F, _P, _D, _T4, _P],
     "eadgan_bn_bwd_finalize": [_P, _P, _P, _D, _D, _P, _P, _P, _I, _P, _P, _P, _P],
     "eadgan_bn_eval": [_T4, _I, _I, _I, _I, _P, _P, _F, _P, _P, _I, _F, _T4, _P],
+    "eadgan_bn_eval_bwd": [_T4, _T4, _T4, _I, _I, _I, _I, _P, _P, _F, _P, _P, _I, _F, _P, _T4, _P, _P, _P, _P],
     "eadgan_act_fwd": [_P, _P, _L, _I, _F, _P],
     "eadgan_act_bwd": [_P, _P, _P, _L, _I, _F, _P],
     "eadgan_softmax_fwd": [_P, _P, _I, _I, _P],

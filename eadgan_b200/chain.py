@@ -14,6 +14,11 @@ groups (every G / D / Encoder trunk of the reference: celebA/EAD-GAN_celebA.py:7
     are accumulated in the ConvTranspose epilogue (fp64 atomics) and the normalise + ReLU pass
     is one streaming kernel; the LeakyReLU/ReLU backward of layer L is fused into the epilogue
     of layer L+1's input-gradient kernel (mask = saved output of layer L);
+  * a BatchNorm in eval mode (``.eval()``, torch semantics) normalises with its running statistics:
+    no fused statistics, no cross-rank all-reduce, no running-statistics update; its backward is
+    one pass (dx in place, plus the fp64 sums that give dgamma, dbeta and the conv-bias gradient).
+    The conv output before BatchNorm is kept exactly as in training mode, and the kernel families
+    are the training-mode ones; the stage's BatchNorm mode is recorded in its plan by the forward;
   * layers the tensor-core path does not cover run on the generic SIMT kernels directly on the
     same buffers (strided bf16 views) -- there is no torch / cuDNN fallback anywhere.
     ``_plan_kernels`` picks the kernel family of every stage and direction, in one place.
@@ -208,8 +213,6 @@ def try_run(seq, x):
     stages = _plan(seq)
     if stages is None:
         return None
-    if any(st.bn is not None and not st.bn.training for st in stages):
-        return None  # eval-mode BN: per-op path
     params, srcs = [], []
     for st in stages:
         queue = st.conv.__dict__.get("_eadgan_sn_queue")
@@ -253,7 +256,8 @@ def try_run(seq, x):
             srcs.append(None)
         params += [w, st.conv.bias]
         if st.bn is not None:
-            st.bn.num_batches_tracked.add_(1)
+            if st.bn.training:
+                st.bn.num_batches_tracked.add_(1)
             params += [st.bn.weight, st.bn.bias]
     if gate_log is not None:
         gate_log.append((seq, []))
@@ -361,12 +365,16 @@ def _impl(st, d, last):
 
 class _StagePlan:
     """How one stage runs: its geometry ``d``, the kernel family of its forward (``fwd``), weight gradient
-    (``wgrad``) and input gradient (``dx``), and the layout of the buffers around it.
+    (``wgrad``) and input gradient (``dx``), the mode of its BatchNorm (``bn``: None, "train" or "eval"), and the
+    layout of the buffers around it.
 
     Families: "tc" (tcgen05 implicit GEMM, csrc/tc_conv.cu), "thin" (the same kernels with the 1..4-channel image as
     big map, row-expanded to K = 64), "dense_T" / "dense_C" / "dense" (the 1x1 <-> 4x4 layers as batch GEMMs) and
-    "simt" (the any-geometry SIMT kernels, csrc/simt_conv.cu)."""
-    __slots__ = ("d", "ca", "fwd", "wgrad", "dx", "fuse", "in_fmt", "out_fmt", "in_shape", "out_shape")
+    "simt" (the any-geometry SIMT kernels, csrc/simt_conv.cu).
+
+    The BatchNorm mode is read from ``bn.training`` when the forward builds the plan; the backward follows the plan,
+    so switching the module between ``.train()`` and ``.eval()`` after a forward does not change its backward."""
+    __slots__ = ("d", "ca", "fwd", "wgrad", "dx", "bn", "fuse", "in_fmt", "out_fmt", "in_shape", "out_shape")
 
 
 def _plan_kernels(stages, in_shape):
@@ -382,6 +390,7 @@ def _plan_kernels(stages, in_shape):
         d = p.d = _geom(st, in_shape)
         p.in_shape = tuple(in_shape)
         p.out_shape = (d.n, d.k, d.p, d.q) if conv else (d.n, d.c, d.h, d.w)
+        p.bn = None if st.bn is None else ("train" if st.bn.training else "eval")
         p.fwd = _impl(st, d, last)
         p.ca = _calloc(d) if p.fwd == "tc" else d.c
         if p.fwd in ("dense_T", "dense_C"):
@@ -448,8 +457,10 @@ class _Arena:
 
 class _Saved:
     """what the forward of one stage leaves for its backward, and the stage's weight in every form a kernel reads"""
-    __slots__ = ("w", "src", "lazy", "pi", "has_b", "inp", "y", "R", "a", "pre", "mean", "invstd", "gamma", "beta",
-                 "count", "n_local", "sum_x")
+    # a BatchNorm stage keeps its conv output ``pre`` and the normalisation it applied: ``mean`` / ``invstd`` of the
+    # batch in training mode; in eval mode ``mean`` / ``invstd`` are running_mean / running_var, with ``eps``
+    __slots__ = ("w", "src", "lazy", "pi", "has_b", "inp", "y", "R", "a", "pre", "mean", "invstd", "eps", "gamma",
+                 "beta", "count", "n_local", "sum_x")
 
     def __init__(self, w, src, pi, has_b):
         self.w, self.src, self.pi, self.has_b = w, src, pi, has_b
@@ -486,7 +497,7 @@ class _ChainFn(torch.autograd.Function):
         pi = 0
         # ONE zero fill for all per-channel fp64 statistics vectors of this forward (a fill kernel per BatchNorm layer
         # was ~40 launches of a few microseconds per step)
-        arena = _Arena(sum(2 * p.out_shape[1] for st, p in zip(stages, plans) if st.bn is not None), dev)
+        arena = _Arena(sum(2 * p.out_shape[1] for p in plans if p.bn == "train"), dev)
         for si, (st, p) in enumerate(zip(stages, plans)):
             sv = _Saved(params[pi], srcs[si], pi, params[pi + 1] is not None)
             b = params[pi + 1]
@@ -495,7 +506,7 @@ class _ChainFn(torch.autograd.Function):
             out_shape = p.out_shape
             cout = out_shape[1]
             epi_act = st.act if st.bn is None else (ACT_NONE, 0.0)
-            stats = arena.take(2 * cout) if st.bn is not None else None
+            stats = arena.take(2 * cout) if p.bn == "train" else None   # eval: running statistics, nothing to fuse
             # a conv reads its big map zero-padded to p.ca channels: a padded buffer of fewer channels (the output of a
             # SIMT stage onto 5..31 channels) is copied into a channel-padded one
             in_c = p.ca if conv else p.in_shape[1]
@@ -533,7 +544,19 @@ class _ChainFn(torch.autograd.Function):
                          ptr(stats), st_)
             out = _Buf(out_t, p.out_fmt)
             sv.inp = inp
-            if st.bn is not None:
+            if p.bn == "eval":
+                # running statistics: no statistics pass, no finalize, no cross-rank communication, no update
+                bn = st.bn
+                gamma, beta = params[pi - 2], params[pi - 1]
+                y = _Buf(tc.alloc_padded(out_shape[0], out_shape[2], out_shape[3], cout, dev), "pad")
+                xd, yd = t4(out.view()), t4(y.view())
+                call("eadgan_bn_eval", C.byref(xd), out_shape[0], cout, out_shape[2], out_shape[3],
+                     ptr(bn.running_mean), ptr(bn.running_var), float(bn.eps), ptr(gamma), ptr(beta), st.act[0],
+                     float(st.act[1]), C.byref(yd), st_)
+                sv.pre, sv.gamma, sv.beta = out, gamma, beta
+                sv.mean, sv.invstd, sv.eps = bn.running_mean, bn.running_var, float(bn.eps)
+                out = y
+            elif p.bn == "train":
                 bn = st.bn
                 gamma, beta = params[pi - 2], params[pi - 1]
                 n_local = float(out_shape[0] * out_shape[2] * out_shape[3])
@@ -588,7 +611,18 @@ class _ChainFn(torch.autograd.Function):
             need_db = sv.has_b and ctx.needs_input_grad[3 + sv.pi + 1]
             need_dx = si > 0 or ctx.needs_input_grad[0]
             # ---- 1. gradient w.r.t. the conv output (pre-BN / pre-activation) ----------------
-            if st.bn is not None:
+            if p.bn == "eval":
+                # one pass, in place on g; dgamma, dbeta and the conv-bias gradient from its fp64 sums (no all-reduce:
+                # they are ordinary local gradients, reduced with the others by the optimiser's bucket all-reduce)
+                sums = arena.take(2 * cout)
+                gd, xd, yd = t4(g.view()), t4(sv.pre.view()), t4(sv.y.view())
+                small = torch.empty(3 * cout, device=dev, dtype=torch.float32)
+                dgamma, dbeta, db_bn = small[:cout], small[cout:2 * cout], small[2 * cout:]
+                call("eadgan_bn_eval_bwd", C.byref(gd), C.byref(xd), C.byref(yd), n, cout, oh, ow, ptr(sv.mean),
+                     ptr(sv.invstd), sv.eps, ptr(sv.gamma), ptr(sv.beta), st.act[0], float(st.act[1]), ptr(sums),
+                     C.byref(gd), ptr(dgamma), ptr(dbeta), ptr(db_bn) if sv.has_b else None, st_)
+                dz = g
+            elif p.bn == "train":
                 sums = arena.take(2 * cout)
                 gd, xd, yd = t4(g.view()), t4(sv.pre.view()), t4(sv.y.view())
                 call("eadgan_bn_bwd_reduce", C.byref(gd), C.byref(xd), C.byref(yd), n, cout, oh, ow, ptr(sv.mean),

@@ -11,7 +11,9 @@
 //   kind 1  NHWC rows    : a "row" is one (n,y) line of w*c contiguous elements
 //                          (halo-padded private buffers: sc==1, sw==c, any sh/sn)
 // Algorithmic bytes / element: stats 4 (fp32) or 2 (bf16) read; apply read+write;
-// bwd_reduce 2 reads; bwd_apply 2 reads + 1 write.
+// bwd_reduce 2 reads; bwd_apply 2 reads + 1 write.  Eval mode (running statistics) has no
+// batch-wide dependency: its backward is ONE pass (eval_bwd, 2 reads + 1 write) plus a
+// per-channel finalize of dgamma / dbeta / conv-bias gradient.
 #include <cstdlib>
 #include "common.cuh"
 
@@ -145,6 +147,27 @@ __global__ void __launch_bounds__(256) bn_bwd_reduce_kernel(BwdArgs a, Geo g, do
     const float xv = eg_ld(a.x.ptr, row_base(a.x, g, row) + i, a.x.dtype);
     v0 = dz;
     v1 = dz * (xv - a.mean[ch]) * a.invstd[ch];
+  };
+  if (g.kind == 0) reduce_kind0(g, sums, f); else reduce_kind1(g, sums, f);
+}
+
+// eval-mode backward, one pass: nothing depends on the batch's statistics, so the per-element gradient is written
+// while the per-channel sums are accumulated.  dz = dy * act'(y), dx = dz * gamma * rsqrt(rv + eps),
+// sums = [S dz | S dz * xhat] with xhat = (x - rm) * rsqrt(rv + eps).  Every element is read and written by the same
+// thread, so dx may alias dy.  (a.mean = running_mean, a.invstd = running_var here.)
+__global__ void __launch_bounds__(256) bn_eval_bwd_kernel(BwdArgs a, Geo g, float eps, double* sums) {
+  auto f = [&](int row, int i, int ch, float& v0, float& v1) {
+    float dz = eg_ld(a.dy.ptr, row_base(a.dy, g, row) + i, a.dy.dtype);
+    if (a.act != EADGAN_ACT_NONE) {
+      const float yv = eg_ld(a.y.ptr, row_base(a.y, g, row) + i, a.y.dtype);
+      dz *= eg_act_grad(yv, a.act, a.slope);
+    }
+    const float is = rsqrtf(a.invstd[ch] + eps);
+    const float ga = a.gamma ? a.gamma[ch] : 1.f;
+    const float xv = eg_ld(a.x.ptr, row_base(a.x, g, row) + i, a.x.dtype);
+    eg_st(a.dx.ptr, row_base(a.dx, g, row) + i, a.dx.dtype, dz * ga * is);
+    v0 = dz;
+    v1 = dz * (xv - a.mean[ch]) * is;
   };
   if (g.kind == 0) reduce_kind0(g, sums, f); else reduce_kind1(g, sums, f);
 }
@@ -485,6 +508,83 @@ __global__ void __launch_bounds__(256) bn_bwd_apply_nhwc8_kernel(BwdArgs a, Nhwc
   }
 }
 
+// eval-mode backward on the padded bf16 buffers: bn_bwd_reduce_nhwc8 and the dx store in one pass (dx = dz * sc).
+// The parameters are the running statistics, converted exactly as bn_apply_nhwc8_kernel converts them, so the
+// recomputed ReLU / LeakyReLU gate equals the stored output's gate bit for bit.  dx may alias dy: every 16-byte
+// vector is loaded before the same thread stores it.  Bytes per element: 4R+2W (6R+2W with the gate read from y).
+template <bool GATE_FROM_X>
+__global__ void __launch_bounds__(256) bn_eval_bwd_nhwc8_kernel(BwdArgs a, Nhwc8 g, float eps, double* sums) {
+  __shared__ double sh[2 * 1024];
+  for (int i = threadIdx.x; i < 2 * g.c; i += 256) sh[i] = 0.0;
+  __syncthreads();
+  ChanParams p;
+  const int ch0 = (threadIdx.x % g.cv) * 8;
+  load_params(p, ch0, a.mean, a.invstd, a.gamma, a.beta);
+#pragma unroll
+  for (int j = 0; j < 8; ++j) p.is[j] = rsqrtf(p.is[j] + eps);
+  derive_params(p);
+  const float slope_neg = a.act == EADGAN_ACT_RELU ? 0.f : a.slope;
+  float s0[8], s1[8];
+#pragma unroll
+  for (int j = 0; j < 8; ++j) s0[j] = s1[j] = 0.f;
+  const int rows = g.n * g.h;
+  for (int row0 = blockIdx.x * NHWC8_U; row0 < rows; row0 += gridDim.x * NHWC8_U) {
+    const uint4 *dyr[NHWC8_U], *xr[NHWC8_U], *yr[NHWC8_U];
+    uint4* dxr[NHWC8_U];
+#pragma unroll
+    for (int u = 0; u < NHWC8_U; ++u) {
+      const int row = min(row0 + u, rows - 1);
+      const int b = row / g.h, y = row - b * g.h;
+      dyr[u] = row_ptr(a.dy, b, y);
+      xr[u] = row_ptr(a.x, b, y);
+      yr[u] = GATE_FROM_X ? nullptr : row_ptr(a.y, b, y);
+      dxr[u] = const_cast<uint4*>(row_ptr(a.dx, b, y));
+    }
+    for (int v = threadIdx.x; v < g.row_vecs; v += 256) {
+      uint4 rdz[NHWC8_U], rx[NHWC8_U], ry[NHWC8_U];
+#pragma unroll
+      for (int u = 0; u < NHWC8_U; ++u) {
+        rdz[u] = dyr[u][v];     // plain loads: dy may be the buffer this kernel writes
+        rx[u] = __ldg(xr[u] + v);
+        if (!GATE_FROM_X) ry[u] = __ldg(yr[u] + v);
+      }
+#pragma unroll
+      for (int u = 0; u < NHWC8_U; ++u) {
+        if (row0 + u < rows) {
+          float dz[8], xv[8];
+          bf8_to_f32(rdz[u], dz);
+          bf8_to_f32(rx[u], xv);
+          if (GATE_FROM_X) {
+            if (a.act != EADGAN_ACT_NONE) {
+#pragma unroll
+              for (int j = 0; j < 8; ++j) dz[j] *= bn_gate(xv[j], p, j, slope_neg);
+            }
+          } else {
+            float yv[8];
+            bf8_to_f32(ry[u], yv);
+#pragma unroll
+            for (int j = 0; j < 8; ++j) dz[j] *= eg_act_grad(yv[j], a.act, a.slope);
+          }
+#pragma unroll
+          for (int j = 0; j < 8; ++j) {
+            s0[j] += dz[j];
+            s1[j] = fmaf(dz[j], fmaf(xv[j], p.is[j], p.nm[j]), s1[j]);
+            dz[j] *= p.sc[j];
+          }
+          dxr[u][v] = f32_to_bf8(dz);
+        }
+      }
+    }
+  }
+#pragma unroll
+  for (int j = 0; j < 8; ++j) {
+    atomicAdd(&sh[ch0 + j], (double)s0[j]);
+    atomicAdd(&sh[g.c + ch0 + j], (double)s1[j]);
+  }
+  __syncthreads();
+  for (int i = threadIdx.x; i < 2 * g.c; i += 256) atomicAdd(&sums[i], sh[i]);
+}
+
 // all tensors channel-fastest bf16 rows with 16-byte aligned runs, and c/8 divides 256
 bool nhwc8_ok(const Geo& g, const eadgan_tensor4* const* ts, int nt) {
   if (g.kind != 1 || g.c % 8 != 0 || g.c > 1024 || 256 % (g.c / 8) != 0) return false;
@@ -534,6 +634,20 @@ __global__ void bn_bwd_finalize_kernel(const double* loc, const double* glob, co
     const double sxhat = fwd_loc ? (fwd_loc[ch] - n_loc * (double)mean[ch]) * is : 0.0;
     const double ga = gamma ? (double)gamma[ch] : 1.0;
     dbias[ch] = (float)(ga * is * (loc[ch] - n_loc * glob[ch] / count - sxhat * glob[c + ch] / count));
+  }
+}
+
+// eval mode: dbeta = S dz, dgamma = S dz*xhat, and the gradient of a conv bias feeding the BatchNorm, sum of dx =
+// gamma * rsqrt(rv + eps) * S dz (not zero in eval mode: the normalisation does not depend on the batch)
+__global__ void bn_eval_bwd_finalize_kernel(const double* sums, const float* rvar, float eps, const float* gamma,
+                                            int c, float* dgamma, float* dbeta, float* dbias) {
+  const int ch = blockIdx.x * blockDim.x + threadIdx.x;
+  if (ch >= c) return;
+  if (dbeta) dbeta[ch] = (float)sums[ch];
+  if (dgamma) dgamma[ch] = (float)sums[c + ch];
+  if (dbias) {
+    const double ga = gamma ? (double)gamma[ch] : 1.0;
+    dbias[ch] = (float)(ga * (double)rsqrtf(rvar[ch] + eps) * sums[ch]);
   }
 }
 
@@ -627,8 +741,46 @@ extern "C" int eadgan_bn_eval(const eadgan_tensor4* x, int n, int c, int h, int 
   EG_REQUIRE(x && y && running_mean && running_var, EADGAN_ERR_INVALID, "bn_eval: NULL argument");
   if (int e = make_geo(&g, n, c, h, w, ts, 2, "bn_eval")) return e;
   ApplyArgs a{*x, *y, running_mean, running_var, gamma, beta, act, slope, eps, 1};
+  if (nhwc8_ok(g, ts, 2)) {
+    bn_apply_nhwc8_kernel<<<nhwc8_grid(g), 256, 0, (cudaStream_t)stream>>>(a, make_nhwc8(g));
+    EG_LAUNCH_CHECK("bn_apply_nhwc8_kernel(eval)");
+    return 0;
+  }
   bn_apply_kernel<<<elem_grid(g), 256, 0, (cudaStream_t)stream>>>(a, g);
   EG_LAUNCH_CHECK("bn_apply_kernel(eval)");
+  return 0;
+}
+
+extern "C" int eadgan_bn_eval_bwd(const eadgan_tensor4* dy, const eadgan_tensor4* x, const eadgan_tensor4* y,
+                                  int n, int c, int h, int w, const float* running_mean, const float* running_var,
+                                  float eps, const float* gamma, const float* beta, int act, float slope,
+                                  double* sums, const eadgan_tensor4* dx, float* dgamma, float* dbeta, float* dbias,
+                                  void* stream) {
+  Geo g;
+  EG_REQUIRE(dy && x && dx && running_mean && running_var && sums, EADGAN_ERR_INVALID,
+             "bn_eval_bwd: NULL argument");
+  EG_REQUIRE(act == EADGAN_ACT_NONE || y, EADGAN_ERR_INVALID, "bn_eval_bwd: fused activation needs y");
+  const eadgan_tensor4* ts[] = {dy, x, dx, act != EADGAN_ACT_NONE ? y : nullptr};
+  if (int e = make_geo(&g, n, c, h, w, ts, 4, "bn_eval_bwd")) return e;
+  BwdArgs a{};
+  a.dy = *dy; a.x = *x; if (y) a.y = *y; a.dx = *dx;
+  a.mean = running_mean; a.invstd = running_var; a.gamma = gamma; a.beta = beta; a.act = act; a.slope = slope;
+  cudaStream_t s = (cudaStream_t)stream;
+  const bool gate_x = act == EADGAN_ACT_NONE || act == EADGAN_ACT_RELU || act == EADGAN_ACT_LRELU;
+  const eadgan_tensor4* fs[] = {dy, x, dx, gate_x ? nullptr : y};
+  if (nhwc8_ok(g, fs, 4)) {
+    if (gate_x) bn_eval_bwd_nhwc8_kernel<true><<<nhwc8_grid(g), 256, 0, s>>>(a, make_nhwc8(g), eps, sums);
+    else bn_eval_bwd_nhwc8_kernel<false><<<nhwc8_grid(g), 256, 0, s>>>(a, make_nhwc8(g), eps, sums);
+    EG_LAUNCH_CHECK("bn_eval_bwd_nhwc8_kernel");
+  } else {
+    bn_eval_bwd_kernel<<<reduce_grid(g), 256, 0, s>>>(a, g, eps, sums);
+    EG_LAUNCH_CHECK("bn_eval_bwd_kernel");
+  }
+  if (dgamma || dbeta || dbias) {
+    bn_eval_bwd_finalize_kernel<<<(c + 127) / 128, 128, 0, s>>>(sums, running_var, eps, gamma, c, dgamma, dbeta,
+                                                                dbias);
+    EG_LAUNCH_CHECK("bn_eval_bwd_finalize_kernel");
+  }
   return 0;
 }
 

@@ -205,7 +205,7 @@ class _BatchNormFn(torch.autograd.Function):
             call("eadgan_bn_eval", C.byref(xd), n, c, h, w, ptr(rmean), ptr(rvar), float(eps), ptr(gamma),
                  ptr(beta), act, float(slope), C.byref(yd), st)
             ctx.training = False
-            ctx.save_for_backward(x, gamma, rvar, y)
+            ctx.save_for_backward(x, gamma, beta, rmean, rvar, y if act != ACT_NONE else None)
             ctx.cfg = (eps, act, slope)
             return y
         sums = torch.zeros(2 * c, device=x.device, dtype=torch.float64)
@@ -230,9 +230,21 @@ class _BatchNormFn(torch.autograd.Function):
         dy = dy.contiguous()
         st = stream()
         if not ctx.training:
-            x, gamma, rvar, y = ctx.saved_tensors
-            raise RuntimeError("batch_norm: backward through eval-mode BatchNorm2d is not on the "
-                               "reference's hot path and is not implemented")
+            # running statistics: no batch-wide term, one pass for dx and the per-channel sums (no all-reduce: the
+            # normalisation does not depend on other ranks' data)
+            x, gamma, beta, rmean, rvar, y = ctx.saved_tensors
+            eps, act, slope = ctx.cfg
+            n, c, h, w = x.shape
+            sums = torch.zeros(2 * c, device=x.device, dtype=torch.float64)
+            small = torch.empty(2 * c, device=x.device, dtype=torch.float32)
+            dgamma, dbeta = small[:c], small[c:]
+            dx = torch.empty_like(x)
+            dyd, xd, dxd = t4(dy), t4(x), t4(dx)
+            yd = t4(y) if y is not None else None
+            call("eadgan_bn_eval_bwd", C.byref(dyd), C.byref(xd), C.byref(yd) if yd is not None else None, n, c, h, w,
+                 ptr(rmean), ptr(rvar), float(eps), ptr(gamma), ptr(beta), act, float(slope), ptr(sums),
+                 C.byref(dxd), ptr(dgamma), ptr(dbeta), None, st)
+            return dx, dgamma, dbeta, None, None, None, None, None, None, None
         x, gamma, beta, mean, invstd, y = ctx.saved_tensors
         count, act, slope = ctx.cfg
         n, c, h, w = x.shape

@@ -257,6 +257,17 @@ int eadgan_bn_bwd_finalize(const double* local_sums, const double* global_sums,
 int eadgan_bn_eval(const eadgan_tensor4* x, int n, int c, int h, int w, const float* running_mean,
                    const float* running_var, float eps, const float* gamma, const float* beta,
                    int act, float slope, const eadgan_tensor4* y, void* stream);
+/* eval-mode backward (torch NativeBatchNormBackward0 with training=False, plus the fused activation's
+ * backward), one pass: dz = dy * act'(.), dx = dz * gamma * rsqrt(running_var + eps), and
+ * sums[0:C] = sum dz, sums[C:2C] = sum dz * xhat with xhat = (x - running_mean) * rsqrt(running_var + eps)
+ * (fp64, sums must be zeroed).  dx may alias dy.  The ReLU / LeakyReLU gate is recomputed from x on
+ * bf16 NHWC buffers whose c / 8 divides 256, else read from y (y is the saved post-activation output).
+ * Then, for each of dgamma / dbeta / dbias that is not NULL: dgamma = sum dz*xhat, dbeta = sum dz, and the
+ * gradient of a conv bias feeding this BatchNorm, dbias = gamma * rsqrt(running_var + eps) * sum dz. */
+int eadgan_bn_eval_bwd(const eadgan_tensor4* dy, const eadgan_tensor4* x, const eadgan_tensor4* y,
+                       int n, int c, int h, int w, const float* running_mean, const float* running_var,
+                       float eps, const float* gamma, const float* beta, int act, float slope, double* sums,
+                       const eadgan_tensor4* dx, float* dgamma, float* dbeta, float* dbias, void* stream);
 
 /* ------------------------------------------------------------------------- */
 /* pointwise activations and row softmax (nn.LeakyReLU/ReLU/Tanh, F.sigmoid,   */
