@@ -460,7 +460,7 @@ class _Saved:
     # a BatchNorm stage keeps its conv output ``pre`` and the normalisation it applied: ``mean`` / ``invstd`` of the
     # batch in training mode; in eval mode ``mean`` / ``invstd`` are running_mean / running_var, with ``eps``
     __slots__ = ("w", "src", "lazy", "pi", "has_b", "inp", "y", "R", "a", "pre", "mean", "invstd", "eps", "gamma",
-                 "beta", "count", "n_local", "sum_x")
+                 "beta", "count", "sum_x")
 
     def __init__(self, w, src, pi, has_b):
         self.w, self.src, self.pi, self.has_b = w, src, pi, has_b
@@ -544,38 +544,22 @@ class _ChainFn(torch.autograd.Function):
                          ptr(stats), st_)
             out = _Buf(out_t, p.out_fmt)
             sv.inp = inp
-            if p.bn == "eval":
-                # running statistics: no statistics pass, no finalize, no cross-rank communication, no update
+            if p.bn is not None:
                 bn = st.bn
                 gamma, beta = params[pi - 2], params[pi - 1]
                 y = _Buf(tc.alloc_padded(out_shape[0], out_shape[2], out_shape[3], cout, dev), "pad")
-                xd, yd = t4(out.view()), t4(y.view())
-                call("eadgan_bn_eval", C.byref(xd), out_shape[0], cout, out_shape[2], out_shape[3],
-                     ptr(bn.running_mean), ptr(bn.running_var), float(bn.eps), ptr(gamma), ptr(beta), st.act[0],
-                     float(st.act[1]), C.byref(yd), st_)
+                if p.bn == "eval":
+                    # running statistics: no statistics pass, no finalize, no cross-rank communication, no update
+                    xd, yd = t4(out.view()), t4(y.view())
+                    call("eadgan_bn_eval", C.byref(xd), out_shape[0], cout, out_shape[2], out_shape[3],
+                         ptr(bn.running_mean), ptr(bn.running_var), float(bn.eps), ptr(gamma), ptr(beta), st.act[0],
+                         float(st.act[1]), C.byref(yd), st_)
+                    sv.mean, sv.invstd, sv.eps = bn.running_mean, bn.running_var, float(bn.eps)
+                else:
+                    sv.mean, sv.invstd, sv.count, sv.sum_x = Fn.bn_train_forward(
+                        out.view(), stats, gamma, beta, bn.running_mean, bn.running_var, bn.momentum, bn.eps, *st.act,
+                        y.view(), keep_sum_x=True)
                 sv.pre, sv.gamma, sv.beta = out, gamma, beta
-                sv.mean, sv.invstd, sv.eps = bn.running_mean, bn.running_var, float(bn.eps)
-                out = y
-            elif p.bn == "train":
-                bn = st.bn
-                gamma, beta = params[pi - 2], params[pi - 1]
-                n_local = float(out_shape[0] * out_shape[2] * out_shape[3])
-                count = n_local
-                sum_x = stats                      # this rank's S(x) (first C entries), kept for backward
-                if Fn._allreduce_sum is not None:
-                    sum_x = stats[:cout].clone()
-                    Fn._allreduce_sum(stats)
-                    count *= Fn._world_size
-                mean = torch.empty(cout, device=dev, dtype=torch.float32)
-                invstd = torch.empty(cout, device=dev, dtype=torch.float32)
-                call("eadgan_bn_finalize", ptr(stats), count, cout, float(bn.eps), float(bn.momentum), ptr(mean),
-                     ptr(invstd), ptr(bn.running_mean), ptr(bn.running_var), st_)
-                y = _Buf(tc.alloc_padded(out_shape[0], out_shape[2], out_shape[3], cout, dev), "pad")
-                xd, yd = t4(out.view()), t4(y.view())
-                call("eadgan_bn_apply", C.byref(xd), out_shape[0], cout, out_shape[2], out_shape[3], ptr(mean),
-                     ptr(invstd), ptr(gamma), ptr(beta), st.act[0], float(st.act[1]), C.byref(yd), st_)
-                sv.pre, sv.mean, sv.invstd, sv.gamma, sv.beta = out, mean, invstd, gamma, beta
-                sv.count, sv.n_local, sv.sum_x = count, n_local, sum_x
                 out = y
             sv.y = out
             if gate_log is not None and st.act[0] in (L.ACT_RELU, L.ACT_LRELU):
@@ -602,7 +586,7 @@ class _ChainFn(torch.autograd.Function):
         for si in range(len(stages) - 1, -1, -1):
             st, p, sv = stages[si], plans[si], saved[si]
             d, conv = p.d, st.kind == "conv"
-            n, cout, oh, ow = p.out_shape
+            cout = p.out_shape[1]
             dgamma = dbeta = None
             # which parameter gradients autograd actually wants (inputs: x, stages, srcs, then w, b[, gamma, beta] per
             # stage).  A step driver freezes the networks a phase's optimiser does not own (phase G: D), so their
@@ -611,36 +595,17 @@ class _ChainFn(torch.autograd.Function):
             need_db = sv.has_b and ctx.needs_input_grad[3 + sv.pi + 1]
             need_dx = si > 0 or ctx.needs_input_grad[0]
             # ---- 1. gradient w.r.t. the conv output (pre-BN / pre-activation) ----------------
-            if p.bn == "eval":
-                # one pass, in place on g; dgamma, dbeta and the conv-bias gradient from its fp64 sums (no all-reduce:
-                # they are ordinary local gradients, reduced with the others by the optimiser's bucket all-reduce)
-                sums = arena.take(2 * cout)
-                gd, xd, yd = t4(g.view()), t4(sv.pre.view()), t4(sv.y.view())
-                small = torch.empty(3 * cout, device=dev, dtype=torch.float32)
-                dgamma, dbeta, db_bn = small[:cout], small[cout:2 * cout], small[2 * cout:]
-                call("eadgan_bn_eval_bwd", C.byref(gd), C.byref(xd), C.byref(yd), n, cout, oh, ow, ptr(sv.mean),
-                     ptr(sv.invstd), sv.eps, ptr(sv.gamma), ptr(sv.beta), st.act[0], float(st.act[1]), ptr(sums),
-                     C.byref(gd), ptr(dgamma), ptr(dbeta), ptr(db_bn) if sv.has_b else None, st_)
-                dz = g
-            elif p.bn == "train":
-                sums = arena.take(2 * cout)
-                gd, xd, yd = t4(g.view()), t4(sv.pre.view()), t4(sv.y.view())
-                call("eadgan_bn_bwd_reduce", C.byref(gd), C.byref(xd), C.byref(yd), n, cout, oh, ow, ptr(sv.mean),
-                     ptr(sv.invstd), ptr(sv.gamma), ptr(sv.beta), st.act[0], float(st.act[1]), ptr(sums), st_)
-                local = sums
-                if Fn._allreduce_sum is not None:
-                    local = sums.clone()
-                    Fn._allreduce_sum(sums)
-                call("eadgan_bn_bwd_apply", C.byref(gd), C.byref(xd), C.byref(yd), n, cout, oh, ow, ptr(sv.mean),
-                     ptr(sv.invstd), ptr(sv.gamma), ptr(sv.beta), st.act[0], float(st.act[1]), ptr(sums),
-                     float(sv.count), C.byref(gd), st_)  # in place: dz overwrites g
-                # dgamma / dbeta, and the conv-bias gradient (= sum of dx, zero up to rounding) in closed
-                # form from the fp64 sums: no extra pass over dz
-                small = torch.empty(3 * cout, device=dev, dtype=torch.float32)
-                dgamma, dbeta, db_bn = small[:cout], small[cout:2 * cout], small[2 * cout:]
-                call("eadgan_bn_bwd_finalize", ptr(local), ptr(sums), ptr(sv.sum_x), float(sv.n_local),
-                     float(sv.count), ptr(sv.mean), ptr(sv.invstd), ptr(sv.gamma), cout, ptr(dgamma),
-                     ptr(dbeta), ptr(db_bn) if sv.has_b else None, st_)
+            if p.bn is not None:
+                # in place: dz overwrites g.  dgamma, dbeta and the conv-bias gradient come from the pass's fp64 sums
+                sums, gv = arena.take(2 * cout), g.view()
+                if p.bn == "eval":
+                    dgamma, dbeta, db_bn = Fn.bn_eval_backward(gv, sv.pre.view(), sv.y.view(), sv.mean, sv.invstd,
+                                                               sv.eps, sv.gamma, sv.beta, *st.act, sums, gv,
+                                                               want_dbias=sv.has_b)
+                else:
+                    dgamma, dbeta, db_bn = Fn.bn_train_backward(gv, sv.pre.view(), sv.y.view(), sv.mean, sv.invstd,
+                                                                sv.gamma, sv.beta, *st.act, sv.count, sums, gv,
+                                                                sum_x=sv.sum_x if sv.has_b else None)
                 dz = g
             elif st.act[0] != ACT_NONE and not g_masked:
                 if g.fmt != "ext" or sv.y.fmt != "ext":

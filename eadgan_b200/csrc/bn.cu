@@ -127,49 +127,46 @@ __global__ void __launch_bounds__(256) bn_stats_kernel(eadgan_tensor4 x, Geo g, 
   if (g.kind == 0) reduce_kind0(g, sums, f); else reduce_kind1(g, sums, f);
 }
 
+// The three backward passes.  BWD_REDUCE (training, first half): sums = [S dz | S dz*xhat] for the cross-rank
+// all-reduce.  BWD_APPLY (training, second half): dx from the all-reduced sums.  BWD_EVAL (running statistics): nothing
+// depends on the batch, so dx = dz * gamma * rsqrt(rv + eps) is written while the sums are accumulated, in one pass;
+// there mean / invstd are running_mean / running_var, with eps.  dz = dy * act'(y), xhat = (x - mean) * invstd.
+enum BwdMode { BWD_REDUCE, BWD_APPLY, BWD_EVAL };
+
 struct BwdArgs {
   eadgan_tensor4 dy, x, y, dx;
   const float *mean, *invstd, *gamma, *beta;
-  const double* sums;
+  double* sums;   // written by BWD_REDUCE / BWD_EVAL, read by BWD_APPLY
   double count;
   int act;
   float slope;
+  float eps;
 };
 
-// dz = dy * act'(y);  xhat = (x - mean) * invstd
-__global__ void __launch_bounds__(256) bn_bwd_reduce_kernel(BwdArgs a, Geo g, double* sums) {
-  auto f = [&](int row, int i, int ch, float& v0, float& v1) {
-    float dz = eg_ld(a.dy.ptr, row_base(a.dy, g, row) + i, a.dy.dtype);
-    if (a.act != EADGAN_ACT_NONE) {
-      const float yv = eg_ld(a.y.ptr, row_base(a.y, g, row) + i, a.y.dtype);
-      dz *= eg_act_grad(yv, a.act, a.slope);
-    }
-    const float xv = eg_ld(a.x.ptr, row_base(a.x, g, row) + i, a.x.dtype);
-    v0 = dz;
-    v1 = dz * (xv - a.mean[ch]) * a.invstd[ch];
-  };
-  if (g.kind == 0) reduce_kind0(g, sums, f); else reduce_kind1(g, sums, f);
+__device__ __forceinline__ float bn_dz(const BwdArgs& a, const Geo& g, int row, int i) {
+  float dz = eg_ld(a.dy.ptr, row_base(a.dy, g, row) + i, a.dy.dtype);
+  if (a.act != EADGAN_ACT_NONE) {
+    const float yv = eg_ld(a.y.ptr, row_base(a.y, g, row) + i, a.y.dtype);
+    dz *= eg_act_grad(yv, a.act, a.slope);
+  }
+  return dz;
 }
 
-// eval-mode backward, one pass: nothing depends on the batch's statistics, so the per-element gradient is written
-// while the per-channel sums are accumulated.  dz = dy * act'(y), dx = dz * gamma * rsqrt(rv + eps),
-// sums = [S dz | S dz * xhat] with xhat = (x - rm) * rsqrt(rv + eps).  Every element is read and written by the same
-// thread, so dx may alias dy.  (a.mean = running_mean, a.invstd = running_var here.)
-__global__ void __launch_bounds__(256) bn_eval_bwd_kernel(BwdArgs a, Geo g, float eps, double* sums) {
+// BWD_REDUCE or BWD_EVAL.  In eval mode every element is read and written by the same thread, so dx may alias dy.
+template <int MODE>
+__global__ void __launch_bounds__(256) bn_bwd_reduce_kernel(BwdArgs a, Geo g) {
   auto f = [&](int row, int i, int ch, float& v0, float& v1) {
-    float dz = eg_ld(a.dy.ptr, row_base(a.dy, g, row) + i, a.dy.dtype);
-    if (a.act != EADGAN_ACT_NONE) {
-      const float yv = eg_ld(a.y.ptr, row_base(a.y, g, row) + i, a.y.dtype);
-      dz *= eg_act_grad(yv, a.act, a.slope);
-    }
-    const float is = rsqrtf(a.invstd[ch] + eps);
-    const float ga = a.gamma ? a.gamma[ch] : 1.f;
+    const float dz = bn_dz(a, g, row, i);
+    const float is = MODE == BWD_EVAL ? rsqrtf(a.invstd[ch] + a.eps) : a.invstd[ch];
     const float xv = eg_ld(a.x.ptr, row_base(a.x, g, row) + i, a.x.dtype);
-    eg_st(a.dx.ptr, row_base(a.dx, g, row) + i, a.dx.dtype, dz * ga * is);
+    if (MODE == BWD_EVAL) {
+      const float ga = a.gamma ? a.gamma[ch] : 1.f;
+      eg_st(a.dx.ptr, row_base(a.dx, g, row) + i, a.dx.dtype, dz * ga * is);
+    }
     v0 = dz;
     v1 = dz * (xv - a.mean[ch]) * is;
   };
-  if (g.kind == 0) reduce_kind0(g, sums, f); else reduce_kind1(g, sums, f);
+  if (g.kind == 0) reduce_kind0(g, a.sums, f); else reduce_kind1(g, a.sums, f);
 }
 
 // ---------------- elementwise passes -----------------------------------------------------
@@ -211,11 +208,7 @@ __global__ void __launch_bounds__(256) bn_apply_kernel(ApplyArgs a, Geo g) {
 __global__ void __launch_bounds__(256) bn_bwd_apply_kernel(BwdArgs a, Geo g) {
   const double inv_count = 1.0 / a.count;
   foreach_elem(g, [&](int row, int i, int ch) {
-    float dz = eg_ld(a.dy.ptr, row_base(a.dy, g, row) + i, a.dy.dtype);
-    if (a.act != EADGAN_ACT_NONE) {
-      const float yv = eg_ld(a.y.ptr, row_base(a.y, g, row) + i, a.y.dtype);
-      dz *= eg_act_grad(yv, a.act, a.slope);
-    }
+    const float dz = bn_dz(a, g, row, i);
     const float xv = eg_ld(a.x.ptr, row_base(a.x, g, row) + i, a.x.dtype);
     const float is = a.invstd[ch];
     const float xhat = (xv - a.mean[ch]) * is;
@@ -232,8 +225,8 @@ __global__ void __launch_bounds__(256) bn_bwd_apply_kernel(BwdArgs a, Geo g) {
 // A row (n, y) of the interior is one contiguous run of w*c bf16 = w*c/8 16-byte vectors.  256 threads per
 // block, grid-stride over rows; vector v of a row holds channels 8*(v % (c/8)).., and because c/8 divides
 // 256 every thread keeps ONE channel group for the whole kernel, so the per-channel parameters live in
-// registers.  Bytes per element: apply 2R+2W, bwd_reduce 4R (dy, x; the ReLU/LeakyReLU gate is recomputed
-// from x with the forward's own expression instead of reading y), bwd_apply 4R+2W.
+// registers.  Bytes per element: apply 2R+2W, bwd reduce 4R (dy, x; the ReLU/LeakyReLU gate is recomputed
+// from x with the forward's own expression instead of reading y), bwd apply and eval bwd 4R+2W.
 struct Nhwc8 {
   int n, c, h, w;
   int cv;         // c / 8
@@ -262,15 +255,72 @@ __device__ __forceinline__ const uint4* row_ptr(const eadgan_tensor4& t, int b, 
 }
 
 constexpr int NHWC8_U = 4;   // rows processed together by a block (independent loads in flight per thread)
+
+// The row walk of every nhwc8 kernel.  A block takes NHWC8_U rows at a time (the pointers of a partial last group are
+// clamped to the last row) and, for each of its 16-byte vectors v, issues the loads of the NIN tensors `in` for all
+// NHWC8_U rows before it calls body(raw, dst) for each row that exists: raw[k] is vector v of in[k], dst points at
+// vector v of `out` (nullptr without OUT).  NHWC8_U independent loads per thread are in flight: one load per thread
+// left the kernels latency-bound at ~3 TB/s (2048 threads x 16 B per SM per memory round trip).  in[0] is read with a
+// plain load when PLAIN0 (it may be the buffer `out` aliases), every other input through __ldg.
+template <int NIN, bool PLAIN0, bool OUT, class Body>
+__device__ __forceinline__ void nhwc8_rows(const Nhwc8& g, const eadgan_tensor4* in, const eadgan_tensor4& out,
+                                           Body body) {
+  const int rows = g.n * g.h;
+  for (int row0 = blockIdx.x * NHWC8_U; row0 < rows; row0 += gridDim.x * NHWC8_U) {
+    const uint4* r[NHWC8_U][NIN];
+    uint4* o[NHWC8_U];
+#pragma unroll
+    for (int u = 0; u < NHWC8_U; ++u) {
+      const int row = min(row0 + u, rows - 1);
+      const int b = row / g.h, y = row - b * g.h;
+#pragma unroll
+      for (int k = 0; k < NIN; ++k) r[u][k] = row_ptr(in[k], b, y);
+      o[u] = OUT ? const_cast<uint4*>(row_ptr(out, b, y)) : nullptr;
+    }
+    for (int v = threadIdx.x; v < g.row_vecs; v += 256) {
+      uint4 raw[NHWC8_U][NIN];
+#pragma unroll
+      for (int u = 0; u < NHWC8_U; ++u) {
+#pragma unroll
+        for (int k = 0; k < NIN; ++k) raw[u][k] = PLAIN0 && k == 0 ? r[u][k][v] : __ldg(r[u][k] + v);
+      }
+#pragma unroll
+      for (int u = 0; u < NHWC8_U; ++u) {
+        if (row0 + u < rows) body(raw[u], OUT ? o[u] + v : nullptr);
+      }
+    }
+  }
+}
+
+// the per-channel sums [S s0 | S s1] of the block: 8 channels per thread into shared memory, then one global fp64
+// atomic per block and entry
+__device__ __forceinline__ void block_sums(int c, int ch0, const float* s0, const float* s1, double* sums) {
+  __shared__ double sh[2 * 1024];
+  for (int i = threadIdx.x; i < 2 * c; i += 256) sh[i] = 0.0;
+  __syncthreads();
+#pragma unroll
+  for (int j = 0; j < 8; ++j) {
+    atomicAdd(&sh[ch0 + j], (double)s0[j]);
+    atomicAdd(&sh[c + ch0 + j], (double)s1[j]);
+  }
+  __syncthreads();
+  for (int i = threadIdx.x; i < 2 * c; i += 256) atomicAdd(&sums[i], sh[i]);
+}
+
 struct ChanParams { float mean[8], is[8], ga[8], be[8], sc[8], sh[8], nm[8]; };   // sc = is*ga, sh = be - mean*sc, nm = -mean*is
+// eval: mean / invstd are running_mean / running_var, converted to the inverse standard deviation here
 __device__ __forceinline__ void load_params(ChanParams& p, int ch0, const float* mean, const float* invstd,
-                                            const float* gamma, const float* beta) {
+                                            const float* gamma, const float* beta, bool eval, float eps) {
 #pragma unroll
   for (int j = 0; j < 8; ++j) {
     p.mean[j] = mean[ch0 + j];
     p.is[j] = invstd[ch0 + j];
     p.ga[j] = gamma ? gamma[ch0 + j] : 1.f;
     p.be[j] = beta ? beta[ch0 + j] : 0.f;
+  }
+  if (eval) {
+#pragma unroll
+    for (int j = 0; j < 8; ++j) p.is[j] = rsqrtf(p.is[j] + eps);
   }
 }
 // one FMA per element instead of sub/mul/mul/add: y = x*sc + sh, xhat = x*is + nm (bf16 buffers: the fp32
@@ -287,46 +337,36 @@ __device__ __forceinline__ void derive_params(ChanParams& p) {
 __global__ void __launch_bounds__(256) bn_apply_nhwc8_kernel(ApplyArgs a, Nhwc8 g) {
   ChanParams p;
   const int ch0 = (threadIdx.x % g.cv) * 8;
-  load_params(p, ch0, a.mean, a.invstd, a.gamma, a.beta);
-  if (a.eval) {
-#pragma unroll
-    for (int j = 0; j < 8; ++j) p.is[j] = rsqrtf(p.is[j] + a.eps);
-  }
+  load_params(p, ch0, a.mean, a.invstd, a.gamma, a.beta, a.eval, a.eps);
   derive_params(p);
   const bool leaky = a.act == EADGAN_ACT_RELU || a.act == EADGAN_ACT_LRELU;
   const float neg = a.act == EADGAN_ACT_RELU ? 0.f : a.slope;
-  // NHWC8_U rows per block iteration: every thread keeps NHWC8_U independent 16-byte loads in flight (one load
-  // per thread left the kernel latency-bound at ~3 TB/s: 2048 threads x 16 B per SM per memory round trip)
-  const int rows = g.n * g.h;
-  for (int row0 = blockIdx.x * NHWC8_U; row0 < rows; row0 += gridDim.x * NHWC8_U) {
-    const uint4* xr[NHWC8_U];
-    uint4* yr[NHWC8_U];
+  nhwc8_rows<1, false, true>(g, &a.x, a.y, [&](const uint4* raw, uint4* dst) {
+    float f[8];
+    bf8_to_f32(raw[0], f);
 #pragma unroll
-    for (int u = 0; u < NHWC8_U; ++u) {
-      const int row = min(row0 + u, rows - 1);
-      const int b = row / g.h, y = row - b * g.h;
-      xr[u] = row_ptr(a.x, b, y);
-      yr[u] = const_cast<uint4*>(row_ptr(a.y, b, y));
+    for (int j = 0; j < 8; ++j) {
+      const float t = fmaf(f[j], p.sc[j], p.sh[j]);
+      f[j] = leaky ? (t > 0.f ? t : t * neg) : eg_act(t, a.act, a.slope);
     }
-    for (int v = threadIdx.x; v < g.row_vecs; v += 256) {
-      uint4 raw[NHWC8_U];
+    *dst = f32_to_bf8(f);
+  });
+}
+
+// forward statistics (sum x, sum x^2) of a bf16 NHWC buffer whose producer could not fuse them (dense 1x1 -> 4x4
+// layers): same access pattern as the kernels around it instead of one 2-byte load per thread and iteration
+__global__ void __launch_bounds__(256) bn_stats_nhwc8_kernel(eadgan_tensor4 x, Nhwc8 g, double* sums) {
+  const int ch0 = (threadIdx.x % g.cv) * 8;
+  float s0[8], s1[8];
 #pragma unroll
-      for (int u = 0; u < NHWC8_U; ++u) raw[u] = __ldg(xr[u] + v);
+  for (int j = 0; j < 8; ++j) s0[j] = s1[j] = 0.f;
+  nhwc8_rows<1, false, false>(g, &x, x, [&](const uint4* raw, uint4*) {
+    float f[8];
+    bf8_to_f32(raw[0], f);
 #pragma unroll
-      for (int u = 0; u < NHWC8_U; ++u) {
-        if (row0 + u < rows) {
-          float f[8];
-          bf8_to_f32(raw[u], f);
-#pragma unroll
-          for (int j = 0; j < 8; ++j) {
-            const float t = fmaf(f[j], p.sc[j], p.sh[j]);
-            f[j] = leaky ? (t > 0.f ? t : t * neg) : eg_act(t, a.act, a.slope);
-          }
-          yr[u][v] = f32_to_bf8(f);
-        }
-      }
-    }
-  }
+    for (int j = 0; j < 8; ++j) { s0[j] += f[j]; s1[j] = fmaf(f[j], f[j], s1[j]); }
+  });
+  block_sums(g.c, ch0, s0, s1, sums);
 }
 
 // gate of a ReLU / LeakyReLU that follows the affine transform, recomputed from x exactly as apply did
@@ -334,255 +374,59 @@ __device__ __forceinline__ float bn_gate(float x, const ChanParams& p, int j, fl
   return fmaf(x, p.sc[j], p.sh[j]) > 0.f ? 1.f : slope_neg;
 }
 
-template <bool GATE_FROM_X>
-__global__ void __launch_bounds__(256) bn_bwd_reduce_nhwc8_kernel(BwdArgs a, Nhwc8 g, double* sums) {
-  __shared__ double sh[2 * 1024];
-  for (int i = threadIdx.x; i < 2 * g.c; i += 256) sh[i] = 0.0;
-  __syncthreads();
+// The three backward passes (see BwdMode) on the padded bf16 buffers.  GATE_FROM_X: the activation is none, ReLU or
+// LeakyReLU, and its gate is recomputed from x (bn_gate) instead of reading y.  In eval mode the parameters are the
+// running statistics, converted exactly as bn_apply_nhwc8_kernel converts them, so the recomputed gate equals the
+// stored output's gate bit for bit; and dx may alias dy: dy is read with plain loads, and every 16-byte vector is
+// loaded before the same thread stores it.
+template <int MODE, bool GATE_FROM_X>
+__global__ void __launch_bounds__(256) bn_bwd_nhwc8_kernel(BwdArgs a, Nhwc8 g) {
   ChanParams p;
   const int ch0 = (threadIdx.x % g.cv) * 8;
-  load_params(p, ch0, a.mean, a.invstd, a.gamma, a.beta);
+  load_params(p, ch0, a.mean, a.invstd, a.gamma, a.beta, MODE == BWD_EVAL, a.eps);
   derive_params(p);
   const float slope_neg = a.act == EADGAN_ACT_RELU ? 0.f : a.slope;
-  float s0[8], s1[8];
-#pragma unroll
-  for (int j = 0; j < 8; ++j) s0[j] = s1[j] = 0.f;
-  const int rows = g.n * g.h;
-  for (int row0 = blockIdx.x * NHWC8_U; row0 < rows; row0 += gridDim.x * NHWC8_U) {
-    const uint4 *dyr[NHWC8_U], *xr[NHWC8_U], *yr[NHWC8_U];
-#pragma unroll
-    for (int u = 0; u < NHWC8_U; ++u) {
-      const int row = min(row0 + u, rows - 1);
-      const int b = row / g.h, y = row - b * g.h;
-      dyr[u] = row_ptr(a.dy, b, y);
-      xr[u] = row_ptr(a.x, b, y);
-      yr[u] = GATE_FROM_X ? nullptr : row_ptr(a.y, b, y);
-    }
-    for (int v = threadIdx.x; v < g.row_vecs; v += 256) {
-      uint4 rdz[NHWC8_U], rx[NHWC8_U], ry[NHWC8_U];
-#pragma unroll
-      for (int u = 0; u < NHWC8_U; ++u) {
-        rdz[u] = __ldg(dyr[u] + v);
-        rx[u] = __ldg(xr[u] + v);
-        if (!GATE_FROM_X) ry[u] = __ldg(yr[u] + v);
-      }
-#pragma unroll
-      for (int u = 0; u < NHWC8_U; ++u) {
-        if (row0 + u < rows) {
-          float dz[8], xv[8];
-          bf8_to_f32(rdz[u], dz);
-          bf8_to_f32(rx[u], xv);
-          if (GATE_FROM_X) {
-            if (a.act != EADGAN_ACT_NONE) {
-#pragma unroll
-              for (int j = 0; j < 8; ++j) dz[j] *= bn_gate(xv[j], p, j, slope_neg);
-            }
-          } else {
-            float yv[8];
-            bf8_to_f32(ry[u], yv);
-#pragma unroll
-            for (int j = 0; j < 8; ++j) dz[j] *= eg_act_grad(yv[j], a.act, a.slope);
-          }
-#pragma unroll
-          for (int j = 0; j < 8; ++j) {
-            s0[j] += dz[j];
-            s1[j] = fmaf(dz[j], fmaf(xv[j], p.is[j], p.nm[j]), s1[j]);
-          }
-        }
-      }
-    }
-  }
+  const double inv_count = MODE == BWD_APPLY ? 1.0 / a.count : 0.0;
+  float s0[8], s1[8];   // BWD_REDUCE / BWD_EVAL: the sums; BWD_APPLY: dx = sc*dz - s0 - xhat*s1
 #pragma unroll
   for (int j = 0; j < 8; ++j) {
-    atomicAdd(&sh[ch0 + j], (double)s0[j]);
-    atomicAdd(&sh[g.c + ch0 + j], (double)s1[j]);
-  }
-  __syncthreads();
-  for (int i = threadIdx.x; i < 2 * g.c; i += 256) atomicAdd(&sums[i], sh[i]);
-}
-
-// forward statistics (sum x, sum x^2) of a bf16 NHWC buffer whose producer could not fuse them (dense 1x1 -> 4x4
-// layers): same access pattern as the kernels above instead of one 2-byte load per thread and iteration
-__global__ void __launch_bounds__(256) bn_stats_nhwc8_kernel(eadgan_tensor4 x, Nhwc8 g, double* sums) {
-  __shared__ double sh[2 * 1024];
-  for (int i = threadIdx.x; i < 2 * g.c; i += 256) sh[i] = 0.0;
-  __syncthreads();
-  const int ch0 = (threadIdx.x % g.cv) * 8;
-  float s0[8], s1[8];
-#pragma unroll
-  for (int j = 0; j < 8; ++j) s0[j] = s1[j] = 0.f;
-  const int rows = g.n * g.h;
-  for (int row0 = blockIdx.x * NHWC8_U; row0 < rows; row0 += gridDim.x * NHWC8_U) {
-    const uint4* xr[NHWC8_U];
-#pragma unroll
-    for (int u = 0; u < NHWC8_U; ++u) {
-      const int row = min(row0 + u, rows - 1);
-      const int b = row / g.h, y = row - b * g.h;
-      xr[u] = row_ptr(x, b, y);
+    if (MODE == BWD_APPLY) {
+      s0[j] = p.sc[j] * (float)(a.sums[ch0 + j] * inv_count);
+      s1[j] = p.sc[j] * (float)(a.sums[g.c + ch0 + j] * inv_count);
+    } else {
+      s0[j] = s1[j] = 0.f;
     }
-    for (int v = threadIdx.x; v < g.row_vecs; v += 256) {
-      uint4 raw[NHWC8_U];
+  }
+  const eadgan_tensor4 in[3] = {a.dy, a.x, a.y};
+  nhwc8_rows<GATE_FROM_X ? 2 : 3, MODE == BWD_EVAL, MODE != BWD_REDUCE>(g, in, a.dx, [&](const uint4* raw, uint4* dst) {
+    float dz[8], xv[8];
+    bf8_to_f32(raw[0], dz);
+    bf8_to_f32(raw[1], xv);
+    if constexpr (GATE_FROM_X) {
+      if (a.act != EADGAN_ACT_NONE) {
 #pragma unroll
-      for (int u = 0; u < NHWC8_U; ++u) raw[u] = __ldg(xr[u] + v);
+        for (int j = 0; j < 8; ++j) dz[j] *= bn_gate(xv[j], p, j, slope_neg);
+      }
+    } else {
+      float yv[8];
+      bf8_to_f32(raw[2], yv);
 #pragma unroll
-      for (int u = 0; u < NHWC8_U; ++u) {
-        if (row0 + u < rows) {
-          float f[8];
-          bf8_to_f32(raw[u], f);
+      for (int j = 0; j < 8; ++j) dz[j] *= eg_act_grad(yv[j], a.act, a.slope);
+    }
 #pragma unroll
-          for (int j = 0; j < 8; ++j) { s0[j] += f[j]; s1[j] = fmaf(f[j], f[j], s1[j]); }
-        }
+    for (int j = 0; j < 8; ++j) {
+      if (MODE == BWD_APPLY) {
+        const float xhat = fmaf(xv[j], p.is[j], p.nm[j]);
+        dz[j] = fmaf(-xhat, s1[j], fmaf(dz[j], p.sc[j], -s0[j]));
+      } else {
+        s0[j] += dz[j];
+        s1[j] = fmaf(dz[j], fmaf(xv[j], p.is[j], p.nm[j]), s1[j]);
+        if (MODE == BWD_EVAL) dz[j] *= p.sc[j];
       }
     }
-  }
-#pragma unroll
-  for (int j = 0; j < 8; ++j) {
-    atomicAdd(&sh[ch0 + j], (double)s0[j]);
-    atomicAdd(&sh[g.c + ch0 + j], (double)s1[j]);
-  }
-  __syncthreads();
-  for (int i = threadIdx.x; i < 2 * g.c; i += 256) atomicAdd(&sums[i], sh[i]);
-}
-
-template <bool GATE_FROM_X>
-__global__ void __launch_bounds__(256) bn_bwd_apply_nhwc8_kernel(BwdArgs a, Nhwc8 g) {
-  ChanParams p;
-  const int ch0 = (threadIdx.x % g.cv) * 8;
-  load_params(p, ch0, a.mean, a.invstd, a.gamma, a.beta);
-  const float slope_neg = a.act == EADGAN_ACT_RELU ? 0.f : a.slope;
-  const double inv_count = 1.0 / a.count;
-  derive_params(p);
-  float c2[8], c3[8];   // dx = sc*dz - sc*mean(dz) - xhat*sc*mean(dz*xhat)
-#pragma unroll
-  for (int j = 0; j < 8; ++j) {
-    c2[j] = p.sc[j] * (float)(a.sums[ch0 + j] * inv_count);
-    c3[j] = p.sc[j] * (float)(a.sums[g.c + ch0 + j] * inv_count);
-  }
-  const int rows = g.n * g.h;
-  for (int row0 = blockIdx.x * NHWC8_U; row0 < rows; row0 += gridDim.x * NHWC8_U) {
-    const uint4 *dyr[NHWC8_U], *xr[NHWC8_U], *yr[NHWC8_U];
-    uint4* dxr[NHWC8_U];
-#pragma unroll
-    for (int u = 0; u < NHWC8_U; ++u) {
-      const int row = min(row0 + u, rows - 1);
-      const int b = row / g.h, y = row - b * g.h;
-      dyr[u] = row_ptr(a.dy, b, y);
-      xr[u] = row_ptr(a.x, b, y);
-      yr[u] = GATE_FROM_X ? nullptr : row_ptr(a.y, b, y);
-      dxr[u] = const_cast<uint4*>(row_ptr(a.dx, b, y));
-    }
-    for (int v = threadIdx.x; v < g.row_vecs; v += 256) {
-      uint4 rdz[NHWC8_U], rx[NHWC8_U], ry[NHWC8_U];
-#pragma unroll
-      for (int u = 0; u < NHWC8_U; ++u) {
-        rdz[u] = __ldg(dyr[u] + v);
-        rx[u] = __ldg(xr[u] + v);
-        if (!GATE_FROM_X) ry[u] = __ldg(yr[u] + v);
-      }
-#pragma unroll
-      for (int u = 0; u < NHWC8_U; ++u) {
-        if (row0 + u < rows) {
-          float dz[8], xv[8];
-          bf8_to_f32(rdz[u], dz);
-          bf8_to_f32(rx[u], xv);
-          if (GATE_FROM_X) {
-            if (a.act != EADGAN_ACT_NONE) {
-#pragma unroll
-              for (int j = 0; j < 8; ++j) dz[j] *= bn_gate(xv[j], p, j, slope_neg);
-            }
-          } else {
-            float yv[8];
-            bf8_to_f32(ry[u], yv);
-#pragma unroll
-            for (int j = 0; j < 8; ++j) dz[j] *= eg_act_grad(yv[j], a.act, a.slope);
-          }
-#pragma unroll
-          for (int j = 0; j < 8; ++j) {
-            const float xhat = fmaf(xv[j], p.is[j], p.nm[j]);
-            dz[j] = fmaf(-xhat, c3[j], fmaf(dz[j], p.sc[j], -c2[j]));
-          }
-          dxr[u][v] = f32_to_bf8(dz);
-        }
-      }
-    }
-  }
-}
-
-// eval-mode backward on the padded bf16 buffers: bn_bwd_reduce_nhwc8 and the dx store in one pass (dx = dz * sc).
-// The parameters are the running statistics, converted exactly as bn_apply_nhwc8_kernel converts them, so the
-// recomputed ReLU / LeakyReLU gate equals the stored output's gate bit for bit.  dx may alias dy: every 16-byte
-// vector is loaded before the same thread stores it.  Bytes per element: 4R+2W (6R+2W with the gate read from y).
-template <bool GATE_FROM_X>
-__global__ void __launch_bounds__(256) bn_eval_bwd_nhwc8_kernel(BwdArgs a, Nhwc8 g, float eps, double* sums) {
-  __shared__ double sh[2 * 1024];
-  for (int i = threadIdx.x; i < 2 * g.c; i += 256) sh[i] = 0.0;
-  __syncthreads();
-  ChanParams p;
-  const int ch0 = (threadIdx.x % g.cv) * 8;
-  load_params(p, ch0, a.mean, a.invstd, a.gamma, a.beta);
-#pragma unroll
-  for (int j = 0; j < 8; ++j) p.is[j] = rsqrtf(p.is[j] + eps);
-  derive_params(p);
-  const float slope_neg = a.act == EADGAN_ACT_RELU ? 0.f : a.slope;
-  float s0[8], s1[8];
-#pragma unroll
-  for (int j = 0; j < 8; ++j) s0[j] = s1[j] = 0.f;
-  const int rows = g.n * g.h;
-  for (int row0 = blockIdx.x * NHWC8_U; row0 < rows; row0 += gridDim.x * NHWC8_U) {
-    const uint4 *dyr[NHWC8_U], *xr[NHWC8_U], *yr[NHWC8_U];
-    uint4* dxr[NHWC8_U];
-#pragma unroll
-    for (int u = 0; u < NHWC8_U; ++u) {
-      const int row = min(row0 + u, rows - 1);
-      const int b = row / g.h, y = row - b * g.h;
-      dyr[u] = row_ptr(a.dy, b, y);
-      xr[u] = row_ptr(a.x, b, y);
-      yr[u] = GATE_FROM_X ? nullptr : row_ptr(a.y, b, y);
-      dxr[u] = const_cast<uint4*>(row_ptr(a.dx, b, y));
-    }
-    for (int v = threadIdx.x; v < g.row_vecs; v += 256) {
-      uint4 rdz[NHWC8_U], rx[NHWC8_U], ry[NHWC8_U];
-#pragma unroll
-      for (int u = 0; u < NHWC8_U; ++u) {
-        rdz[u] = dyr[u][v];     // plain loads: dy may be the buffer this kernel writes
-        rx[u] = __ldg(xr[u] + v);
-        if (!GATE_FROM_X) ry[u] = __ldg(yr[u] + v);
-      }
-#pragma unroll
-      for (int u = 0; u < NHWC8_U; ++u) {
-        if (row0 + u < rows) {
-          float dz[8], xv[8];
-          bf8_to_f32(rdz[u], dz);
-          bf8_to_f32(rx[u], xv);
-          if (GATE_FROM_X) {
-            if (a.act != EADGAN_ACT_NONE) {
-#pragma unroll
-              for (int j = 0; j < 8; ++j) dz[j] *= bn_gate(xv[j], p, j, slope_neg);
-            }
-          } else {
-            float yv[8];
-            bf8_to_f32(ry[u], yv);
-#pragma unroll
-            for (int j = 0; j < 8; ++j) dz[j] *= eg_act_grad(yv[j], a.act, a.slope);
-          }
-#pragma unroll
-          for (int j = 0; j < 8; ++j) {
-            s0[j] += dz[j];
-            s1[j] = fmaf(dz[j], fmaf(xv[j], p.is[j], p.nm[j]), s1[j]);
-            dz[j] *= p.sc[j];
-          }
-          dxr[u][v] = f32_to_bf8(dz);
-        }
-      }
-    }
-  }
-#pragma unroll
-  for (int j = 0; j < 8; ++j) {
-    atomicAdd(&sh[ch0 + j], (double)s0[j]);
-    atomicAdd(&sh[g.c + ch0 + j], (double)s1[j]);
-  }
-  __syncthreads();
-  for (int i = threadIdx.x; i < 2 * g.c; i += 256) atomicAdd(&sums[i], sh[i]);
+    if (MODE != BWD_REDUCE) *dst = f32_to_bf8(dz);
+  });
+  if (MODE != BWD_APPLY) block_sums(g.c, ch0, s0, s1, a.sums);
 }
 
 // all tensors channel-fastest bf16 rows with 16-byte aligned runs, and c/8 divides 256
@@ -685,6 +529,53 @@ int elem_grid(const Geo& g) {
   return (int)(jobs > cap ? cap : jobs);
 }
 
+// the apply pass of eadgan_bn_apply (batch statistics) and eadgan_bn_eval (running statistics, a.eval)
+int bn_apply(const eadgan_tensor4* x, const eadgan_tensor4* y, int n, int c, int h, int w, const ApplyArgs& a,
+             void* stream, const char* who) {
+  Geo g;
+  const eadgan_tensor4* ts[] = {x, y};
+  if (int e = make_geo(&g, n, c, h, w, ts, 2, who)) return e;
+  if (nhwc8_ok(g, ts, 2)) {
+    bn_apply_nhwc8_kernel<<<nhwc8_grid(g), 256, 0, (cudaStream_t)stream>>>(a, make_nhwc8(g));
+    EG_LAUNCH_CHECK("bn_apply_nhwc8_kernel");
+    return 0;
+  }
+  bn_apply_kernel<<<elem_grid(g), 256, 0, (cudaStream_t)stream>>>(a, g);
+  EG_LAUNCH_CHECK("bn_apply_kernel");
+  return 0;
+}
+
+// one backward pass (BwdMode) of eadgan_bn_bwd_reduce (dx NULL), eadgan_bn_bwd_apply or eadgan_bn_eval_bwd
+template <int MODE>
+int bn_bwd(const eadgan_tensor4* dy, const eadgan_tensor4* x, const eadgan_tensor4* y, const eadgan_tensor4* dx,
+           int n, int c, int h, int w, const float* mean, const float* invstd, float eps, const float* gamma,
+           const float* beta, int act, float slope, double* sums, double count, void* stream, const char* who) {
+  EG_REQUIRE(act == EADGAN_ACT_NONE || y, EADGAN_ERR_INVALID, "%s: fused activation needs y", who);
+  Geo g;
+  const eadgan_tensor4* ts[] = {dy, x, dx, act != EADGAN_ACT_NONE ? y : nullptr};
+  if (int e = make_geo(&g, n, c, h, w, ts, 4, who)) return e;
+  BwdArgs a{};
+  a.dy = *dy; a.x = *x; if (y) a.y = *y; if (dx) a.dx = *dx;
+  a.mean = mean; a.invstd = invstd; a.gamma = gamma; a.beta = beta; a.act = act; a.slope = slope; a.eps = eps;
+  a.sums = sums; a.count = count;
+  cudaStream_t s = (cudaStream_t)stream;
+  // the nhwc8 kernels recompute a ReLU / LeakyReLU gate from x and then do not read y
+  const bool gate_x = act == EADGAN_ACT_NONE || act == EADGAN_ACT_RELU || act == EADGAN_ACT_LRELU;
+  const eadgan_tensor4* fs[] = {dy, x, dx, gate_x ? nullptr : y};
+  if (nhwc8_ok(g, fs, 4)) {
+    (gate_x ? bn_bwd_nhwc8_kernel<MODE, true> : bn_bwd_nhwc8_kernel<MODE, false>)<<<nhwc8_grid(g), 256, 0, s>>>(
+        a, make_nhwc8(g));
+    EG_LAUNCH_CHECK("bn_bwd_nhwc8_kernel");
+  } else if constexpr (MODE == BWD_APPLY) {
+    bn_bwd_apply_kernel<<<elem_grid(g), 256, 0, s>>>(a, g);
+    EG_LAUNCH_CHECK("bn_bwd_apply_kernel");
+  } else {
+    bn_bwd_reduce_kernel<MODE><<<reduce_grid(g), 256, 0, s>>>(a, g);
+    EG_LAUNCH_CHECK("bn_bwd_reduce_kernel");
+  }
+  return 0;
+}
+
 }  // namespace
 
 extern "C" int eadgan_bn_stats(const eadgan_tensor4* x, int n, int c, int h, int w, double* sums,
@@ -717,38 +608,18 @@ extern "C" int eadgan_bn_finalize(const double* sums, double count, int c, float
 extern "C" int eadgan_bn_apply(const eadgan_tensor4* x, int n, int c, int h, int w, const float* mean,
                                const float* invstd, const float* gamma, const float* beta, int act,
                                float slope, const eadgan_tensor4* y, void* stream) {
-  Geo g;
-  const eadgan_tensor4* ts[] = {x, y};
   EG_REQUIRE(x && y && mean && invstd, EADGAN_ERR_INVALID, "bn_apply: NULL argument");
-  if (int e = make_geo(&g, n, c, h, w, ts, 2, "bn_apply")) return e;
-  ApplyArgs a{*x, *y, mean, invstd, gamma, beta, act, slope, 0.f, 0};
-  if (nhwc8_ok(g, ts, 2)) {
-    bn_apply_nhwc8_kernel<<<nhwc8_grid(g), 256, 0, (cudaStream_t)stream>>>(a, make_nhwc8(g));
-    EG_LAUNCH_CHECK("bn_apply_nhwc8_kernel");
-    return 0;
-  }
-  bn_apply_kernel<<<elem_grid(g), 256, 0, (cudaStream_t)stream>>>(a, g);
-  EG_LAUNCH_CHECK("bn_apply_kernel");
-  return 0;
+  return bn_apply(x, y, n, c, h, w, ApplyArgs{*x, *y, mean, invstd, gamma, beta, act, slope, 0.f, 0}, stream,
+                  "bn_apply");
 }
 
 extern "C" int eadgan_bn_eval(const eadgan_tensor4* x, int n, int c, int h, int w,
                               const float* running_mean, const float* running_var, float eps,
                               const float* gamma, const float* beta, int act, float slope,
                               const eadgan_tensor4* y, void* stream) {
-  Geo g;
-  const eadgan_tensor4* ts[] = {x, y};
   EG_REQUIRE(x && y && running_mean && running_var, EADGAN_ERR_INVALID, "bn_eval: NULL argument");
-  if (int e = make_geo(&g, n, c, h, w, ts, 2, "bn_eval")) return e;
-  ApplyArgs a{*x, *y, running_mean, running_var, gamma, beta, act, slope, eps, 1};
-  if (nhwc8_ok(g, ts, 2)) {
-    bn_apply_nhwc8_kernel<<<nhwc8_grid(g), 256, 0, (cudaStream_t)stream>>>(a, make_nhwc8(g));
-    EG_LAUNCH_CHECK("bn_apply_nhwc8_kernel(eval)");
-    return 0;
-  }
-  bn_apply_kernel<<<elem_grid(g), 256, 0, (cudaStream_t)stream>>>(a, g);
-  EG_LAUNCH_CHECK("bn_apply_kernel(eval)");
-  return 0;
+  return bn_apply(x, y, n, c, h, w, ApplyArgs{*x, *y, running_mean, running_var, gamma, beta, act, slope, eps, 1},
+                  stream, "bn_eval");
 }
 
 extern "C" int eadgan_bn_eval_bwd(const eadgan_tensor4* dy, const eadgan_tensor4* x, const eadgan_tensor4* y,
@@ -756,29 +627,14 @@ extern "C" int eadgan_bn_eval_bwd(const eadgan_tensor4* dy, const eadgan_tensor4
                                   float eps, const float* gamma, const float* beta, int act, float slope,
                                   double* sums, const eadgan_tensor4* dx, float* dgamma, float* dbeta, float* dbias,
                                   void* stream) {
-  Geo g;
   EG_REQUIRE(dy && x && dx && running_mean && running_var && sums, EADGAN_ERR_INVALID,
              "bn_eval_bwd: NULL argument");
-  EG_REQUIRE(act == EADGAN_ACT_NONE || y, EADGAN_ERR_INVALID, "bn_eval_bwd: fused activation needs y");
-  const eadgan_tensor4* ts[] = {dy, x, dx, act != EADGAN_ACT_NONE ? y : nullptr};
-  if (int e = make_geo(&g, n, c, h, w, ts, 4, "bn_eval_bwd")) return e;
-  BwdArgs a{};
-  a.dy = *dy; a.x = *x; if (y) a.y = *y; a.dx = *dx;
-  a.mean = running_mean; a.invstd = running_var; a.gamma = gamma; a.beta = beta; a.act = act; a.slope = slope;
-  cudaStream_t s = (cudaStream_t)stream;
-  const bool gate_x = act == EADGAN_ACT_NONE || act == EADGAN_ACT_RELU || act == EADGAN_ACT_LRELU;
-  const eadgan_tensor4* fs[] = {dy, x, dx, gate_x ? nullptr : y};
-  if (nhwc8_ok(g, fs, 4)) {
-    if (gate_x) bn_eval_bwd_nhwc8_kernel<true><<<nhwc8_grid(g), 256, 0, s>>>(a, make_nhwc8(g), eps, sums);
-    else bn_eval_bwd_nhwc8_kernel<false><<<nhwc8_grid(g), 256, 0, s>>>(a, make_nhwc8(g), eps, sums);
-    EG_LAUNCH_CHECK("bn_eval_bwd_nhwc8_kernel");
-  } else {
-    bn_eval_bwd_kernel<<<reduce_grid(g), 256, 0, s>>>(a, g, eps, sums);
-    EG_LAUNCH_CHECK("bn_eval_bwd_kernel");
-  }
+  if (int e = bn_bwd<BWD_EVAL>(dy, x, y, dx, n, c, h, w, running_mean, running_var, eps, gamma, beta, act, slope,
+                               sums, 0.0, stream, "bn_eval_bwd"))
+    return e;
   if (dgamma || dbeta || dbias) {
-    bn_eval_bwd_finalize_kernel<<<(c + 127) / 128, 128, 0, s>>>(sums, running_var, eps, gamma, c, dgamma, dbeta,
-                                                                dbias);
+    bn_eval_bwd_finalize_kernel<<<(c + 127) / 128, 128, 0, (cudaStream_t)stream>>>(sums, running_var, eps, gamma, c,
+                                                                                  dgamma, dbeta, dbias);
     EG_LAUNCH_CHECK("bn_eval_bwd_finalize_kernel");
   }
   return 0;
@@ -789,25 +645,9 @@ extern "C" int eadgan_bn_bwd_reduce(const eadgan_tensor4* dy, const eadgan_tenso
                                     const float* mean, const float* invstd, const float* gamma,
                                     const float* beta, int act, float slope, double* sums,
                                     void* stream) {
-  Geo g;
   EG_REQUIRE(dy && x && mean && invstd && sums, EADGAN_ERR_INVALID, "bn_bwd_reduce: NULL argument");
-  EG_REQUIRE(act == EADGAN_ACT_NONE || y, EADGAN_ERR_INVALID, "bn_bwd_reduce: fused activation needs y");
-  const eadgan_tensor4* ts[] = {dy, x, act != EADGAN_ACT_NONE ? y : nullptr};
-  if (int e = make_geo(&g, n, c, h, w, ts, 3, "bn_bwd_reduce")) return e;
-  BwdArgs a{};
-  a.dy = *dy; a.x = *x; if (y) a.y = *y;
-  a.mean = mean; a.invstd = invstd; a.gamma = gamma; a.beta = beta; a.act = act; a.slope = slope;
-  const bool gate_x = act == EADGAN_ACT_NONE || act == EADGAN_ACT_RELU || act == EADGAN_ACT_LRELU;
-  const eadgan_tensor4* fs[] = {dy, x, gate_x ? nullptr : y};
-  if (nhwc8_ok(g, fs, 3)) {
-    if (gate_x) bn_bwd_reduce_nhwc8_kernel<true><<<nhwc8_grid(g), 256, 0, (cudaStream_t)stream>>>(a, make_nhwc8(g), sums);
-    else bn_bwd_reduce_nhwc8_kernel<false><<<nhwc8_grid(g), 256, 0, (cudaStream_t)stream>>>(a, make_nhwc8(g), sums);
-    EG_LAUNCH_CHECK("bn_bwd_reduce_nhwc8_kernel");
-    return 0;
-  }
-  bn_bwd_reduce_kernel<<<reduce_grid(g), 256, 0, (cudaStream_t)stream>>>(a, g, sums);
-  EG_LAUNCH_CHECK("bn_bwd_reduce_kernel");
-  return 0;
+  return bn_bwd<BWD_REDUCE>(dy, x, y, nullptr, n, c, h, w, mean, invstd, 0.f, gamma, beta, act, slope, sums, 0.0,
+                            stream, "bn_bwd_reduce");
 }
 
 extern "C" int eadgan_bn_bwd_apply(const eadgan_tensor4* dy, const eadgan_tensor4* x,
@@ -815,27 +655,10 @@ extern "C" int eadgan_bn_bwd_apply(const eadgan_tensor4* dy, const eadgan_tensor
                                    const float* mean, const float* invstd, const float* gamma,
                                    const float* beta, int act, float slope, const double* sums,
                                    double count, const eadgan_tensor4* dx, void* stream) {
-  Geo g;
   EG_REQUIRE(dy && x && dx && mean && invstd && sums && count > 0, EADGAN_ERR_INVALID,
              "bn_bwd_apply: NULL argument");
-  EG_REQUIRE(act == EADGAN_ACT_NONE || y, EADGAN_ERR_INVALID, "bn_bwd_apply: fused activation needs y");
-  const eadgan_tensor4* ts[] = {dy, x, dx, act != EADGAN_ACT_NONE ? y : nullptr};
-  if (int e = make_geo(&g, n, c, h, w, ts, 4, "bn_bwd_apply")) return e;
-  BwdArgs a{};
-  a.dy = *dy; a.x = *x; if (y) a.y = *y; a.dx = *dx;
-  a.mean = mean; a.invstd = invstd; a.gamma = gamma; a.beta = beta; a.act = act; a.slope = slope;
-  a.sums = sums; a.count = count;
-  const bool gate_x = act == EADGAN_ACT_NONE || act == EADGAN_ACT_RELU || act == EADGAN_ACT_LRELU;
-  const eadgan_tensor4* fs[] = {dy, x, dx, gate_x ? nullptr : y};
-  if (nhwc8_ok(g, fs, 4)) {
-    if (gate_x) bn_bwd_apply_nhwc8_kernel<true><<<nhwc8_grid(g), 256, 0, (cudaStream_t)stream>>>(a, make_nhwc8(g));
-    else bn_bwd_apply_nhwc8_kernel<false><<<nhwc8_grid(g), 256, 0, (cudaStream_t)stream>>>(a, make_nhwc8(g));
-    EG_LAUNCH_CHECK("bn_bwd_apply_nhwc8_kernel");
-    return 0;
-  }
-  bn_bwd_apply_kernel<<<elem_grid(g), 256, 0, (cudaStream_t)stream>>>(a, g);
-  EG_LAUNCH_CHECK("bn_bwd_apply_kernel");
-  return 0;
+  return bn_bwd<BWD_APPLY>(dy, x, y, dx, n, c, h, w, mean, invstd, 0.f, gamma, beta, act, slope,
+                           const_cast<double*>(sums), count, stream, "bn_bwd_apply");   // BWD_APPLY only reads sums
 }
 
 extern "C" int eadgan_bn_bwd_finalize(const double* local_sums, const double* global_sums,

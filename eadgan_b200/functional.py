@@ -192,6 +192,71 @@ def linear(x, w, b=None, act=ACT_NONE, slope=0.0):
 # ----------------------------------------------------------------------------------
 # batch norm (+ fused activation), SyncBN across ranks when data-parallel
 # ----------------------------------------------------------------------------------
+# The host sequence of both callers, _BatchNormFn and the bf16 chain (eadgan_b200.chain).  Tensors are [N, C, H, W]
+# views in any layout bn.cu takes (fp32 NCHW, or the chain's padded bf16 NHWC interiors); the fp64 [2C] sum buffers
+# belong to the caller, zero-filled.
+def _ref(t):
+    return None if t is None else C.byref(t4(t))
+
+
+def bn_train_forward(x, sums, gamma, beta, rmean, rvar, momentum, eps, act, slope, y, keep_sum_x=False):
+    """y = act(BatchNorm(x)) with the batch's statistics, from sums = [S x | S x^2] of this rank's x.  When data-parallel
+    the sums are all-reduced in place first.  Updates rmean / rvar.  Returns (mean, invstd, count, sum_x): count is the
+    element count per channel over all ranks; with keep_sum_x, sum_x is this rank's S x, which bn_train_backward needs
+    for the gradient of a conv bias in front of the BatchNorm."""
+    n, c, h, w = x.shape
+    count = float(n * h * w)
+    sum_x = sums[:c] if keep_sum_x else None
+    if _allreduce_sum is not None:
+        if keep_sum_x:
+            sum_x = sum_x.clone()
+        _allreduce_sum(sums)
+        count *= _world_size
+    mean = torch.empty(c, device=x.device, dtype=torch.float32)
+    invstd = torch.empty(c, device=x.device, dtype=torch.float32)
+    st = stream()
+    call("eadgan_bn_finalize", ptr(sums), count, c, float(eps), float(momentum), ptr(mean), ptr(invstd), ptr(rmean),
+         ptr(rvar), st)
+    call("eadgan_bn_apply", _ref(x), n, c, h, w, ptr(mean), ptr(invstd), ptr(gamma), ptr(beta), act, float(slope),
+         _ref(y), st)
+    return mean, invstd, count, sum_x
+
+
+def bn_train_backward(dy, x, y, mean, invstd, gamma, beta, act, slope, count, sums, dx, sum_x=None):
+    """Backward of bn_train_forward: writes dx (which may be dy) and returns (dgamma, dbeta, dbias).  y is the forward's
+    output (None without an activation); sums is scratch.  The fp64 sums [S dz | S dz*xhat] are all-reduced between the
+    two passes; dgamma and dbeta are this rank's, as every other parameter gradient.  dbias, the gradient of a conv bias
+    in front of the BatchNorm, is computed when sum_x (bn_train_forward's) is given, else None."""
+    n, c, h, w = x.shape
+    st = stream()
+    call("eadgan_bn_bwd_reduce", _ref(dy), _ref(x), _ref(y), n, c, h, w, ptr(mean), ptr(invstd), ptr(gamma), ptr(beta),
+         act, float(slope), ptr(sums), st)
+    local = sums
+    if _allreduce_sum is not None:
+        local = sums.clone()
+        _allreduce_sum(sums)
+    call("eadgan_bn_bwd_apply", _ref(dy), _ref(x), _ref(y), n, c, h, w, ptr(mean), ptr(invstd), ptr(gamma), ptr(beta),
+         act, float(slope), ptr(sums), float(count), _ref(dx), st)
+    small = torch.empty((2 if sum_x is None else 3) * c, device=x.device, dtype=torch.float32)
+    dgamma, dbeta, dbias = small[:c], small[c:2 * c], small[2 * c:] if sum_x is not None else None
+    # in closed form from the fp64 sums: no extra pass over dx
+    call("eadgan_bn_bwd_finalize", ptr(local), ptr(sums), ptr(sum_x), float(n * h * w), float(count), ptr(mean),
+         ptr(invstd), ptr(gamma), c, ptr(dgamma), ptr(dbeta), ptr(dbias), st)
+    return dgamma, dbeta, dbias
+
+
+def bn_eval_backward(dy, x, y, rmean, rvar, eps, gamma, beta, act, slope, sums, dx, want_dbias=False):
+    """Backward of y = act(BatchNorm(x)) with the running statistics, one pass: writes dx (which may be dy) and returns
+    (dgamma, dbeta, dbias), dbias (the gradient of a conv bias in front of the BatchNorm) only with want_dbias.  No
+    all-reduce: the normalisation does not depend on other ranks' data."""
+    n, c, h, w = x.shape
+    small = torch.empty((3 if want_dbias else 2) * c, device=x.device, dtype=torch.float32)
+    dgamma, dbeta, dbias = small[:c], small[c:2 * c], small[2 * c:] if want_dbias else None
+    call("eadgan_bn_eval_bwd", _ref(dy), _ref(x), _ref(y), n, c, h, w, ptr(rmean), ptr(rvar), float(eps), ptr(gamma),
+         ptr(beta), act, float(slope), ptr(sums), _ref(dx), ptr(dgamma), ptr(dbeta), ptr(dbias), stream())
+    return dgamma, dbeta, dbias
+
+
 class _BatchNormFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, gamma, beta, rmean, rvar, training, momentum, eps, act, slope):
@@ -199,28 +264,16 @@ class _BatchNormFn(torch.autograd.Function):
         x = x if x.is_contiguous() else x.contiguous()
         n, c, h, w = x.shape
         y = torch.empty_like(x)
-        xd, yd = t4(x), t4(y)
-        st = stream()
+        ctx.training = training
         if not training:
-            call("eadgan_bn_eval", C.byref(xd), n, c, h, w, ptr(rmean), ptr(rvar), float(eps), ptr(gamma),
-                 ptr(beta), act, float(slope), C.byref(yd), st)
-            ctx.training = False
+            call("eadgan_bn_eval", _ref(x), n, c, h, w, ptr(rmean), ptr(rvar), float(eps), ptr(gamma), ptr(beta), act,
+                 float(slope), _ref(y), stream())
             ctx.save_for_backward(x, gamma, beta, rmean, rvar, y if act != ACT_NONE else None)
             ctx.cfg = (eps, act, slope)
             return y
         sums = torch.zeros(2 * c, device=x.device, dtype=torch.float64)
-        call("eadgan_bn_stats", C.byref(xd), n, c, h, w, ptr(sums), st)
-        count = float(n * h * w)
-        if _allreduce_sum is not None:
-            _allreduce_sum(sums)
-            count *= _world_size
-        mean = torch.empty(c, device=x.device, dtype=torch.float32)
-        invstd = torch.empty(c, device=x.device, dtype=torch.float32)
-        call("eadgan_bn_finalize", ptr(sums), count, c, float(eps), float(momentum), ptr(mean), ptr(invstd),
-             ptr(rmean), ptr(rvar), st)
-        call("eadgan_bn_apply", C.byref(xd), n, c, h, w, ptr(mean), ptr(invstd), ptr(gamma), ptr(beta), act,
-             float(slope), C.byref(yd), st)
-        ctx.training = True
+        call("eadgan_bn_stats", _ref(x), n, c, h, w, ptr(sums), stream())
+        mean, invstd, count, _ = bn_train_forward(x, sums, gamma, beta, rmean, rvar, momentum, eps, act, slope, y)
         ctx.save_for_backward(x, gamma, beta, mean, invstd, y if act != ACT_NONE else None)
         ctx.cfg = (count, act, slope)
         return y
@@ -228,42 +281,16 @@ class _BatchNormFn(torch.autograd.Function):
     @staticmethod
     def backward(ctx, dy):
         dy = dy.contiguous()
-        st = stream()
-        if not ctx.training:
-            # running statistics: no batch-wide term, one pass for dx and the per-channel sums (no all-reduce: the
-            # normalisation does not depend on other ranks' data)
-            x, gamma, beta, rmean, rvar, y = ctx.saved_tensors
-            eps, act, slope = ctx.cfg
-            n, c, h, w = x.shape
-            sums = torch.zeros(2 * c, device=x.device, dtype=torch.float64)
-            small = torch.empty(2 * c, device=x.device, dtype=torch.float32)
-            dgamma, dbeta = small[:c], small[c:]
-            dx = torch.empty_like(x)
-            dyd, xd, dxd = t4(dy), t4(x), t4(dx)
-            yd = t4(y) if y is not None else None
-            call("eadgan_bn_eval_bwd", C.byref(dyd), C.byref(xd), C.byref(yd) if yd is not None else None, n, c, h, w,
-                 ptr(rmean), ptr(rvar), float(eps), ptr(gamma), ptr(beta), act, float(slope), ptr(sums),
-                 C.byref(dxd), ptr(dgamma), ptr(dbeta), None, st)
-            return dx, dgamma, dbeta, None, None, None, None, None, None, None
-        x, gamma, beta, mean, invstd, y = ctx.saved_tensors
-        count, act, slope = ctx.cfg
-        n, c, h, w = x.shape
+        x, gamma, beta, a, b, y = ctx.saved_tensors     # a, b: mean, invstd (training) / running_mean, running_var
+        c = x.shape[1]
         sums = torch.zeros(2 * c, device=x.device, dtype=torch.float64)
-        dyd, xd = t4(dy), t4(x)
-        yd = t4(y) if y is not None else None
-        yref = C.byref(yd) if yd is not None else None
-        call("eadgan_bn_bwd_reduce", C.byref(dyd), C.byref(xd), yref, n, c, h, w, ptr(mean), ptr(invstd),
-             ptr(gamma), ptr(beta), act, float(slope), ptr(sums), st)
-        local = sums.clone() if _allreduce_sum is not None else sums
-        if _allreduce_sum is not None:
-            _allreduce_sum(sums)
         dx = torch.empty_like(x)
-        dxd = t4(dx)
-        call("eadgan_bn_bwd_apply", C.byref(dyd), C.byref(xd), yref, n, c, h, w, ptr(mean), ptr(invstd),
-             ptr(gamma), ptr(beta), act, float(slope), ptr(sums), count, C.byref(dxd), st)
-        # dgamma / dbeta are LOCAL sums (they get all-reduced with the other gradients)
-        dbeta = local[:c].float()
-        dgamma = local[c:].float()
+        if ctx.training:
+            count, act, slope = ctx.cfg
+            dgamma, dbeta, _ = bn_train_backward(dy, x, y, a, b, gamma, beta, act, slope, count, sums, dx)
+        else:
+            eps, act, slope = ctx.cfg
+            dgamma, dbeta, _ = bn_eval_backward(dy, x, y, a, b, eps, gamma, beta, act, slope, sums, dx)
         return dx, dgamma, dbeta, None, None, None, None, None, None, None
 
 

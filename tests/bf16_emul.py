@@ -10,6 +10,9 @@ By default rounding is straight-through in backward (gradients are not rounded; 
 bf16 when it stores them, a smooth <=0.4 % perturbation).  The options of ``emulate`` turn it into an
 fp64 referee that also matches the backward: forced gates, gradients rounded where the chain stores them,
 and spectral-normalised tensor-core layers evaluated the way their kernels evaluate them.
+
+BatchNorm follows the mode the chain planned for it (``_StagePlan.bn``): the batch's statistics in training mode, the
+running statistics in eval mode, with the same bf16 rounding points in both.
 """
 import torch
 import torch.nn.functional as TF
@@ -116,7 +119,9 @@ def emulate(ours_seq, ref_seq, x, update_running=False, gates=None, round_grads=
     ref_seq: torch.nn.Sequential with the same layout holding the parameters to differentiate.
 
     The computation runs in the dtype of ``x`` and ``ref_seq`` (float64 for a referee); rounding is to bf16 either way.
-      update_running: BatchNorm layers of ref_seq update running_mean / running_var as torch's do;
+    A BatchNorm that is in eval mode in ``ours_seq`` (the chain's plan says so) normalises with the running statistics
+    of its ref_seq twin and updates nothing.
+      update_running: training-mode BatchNorm layers of ref_seq update running_mean / running_var as torch's do;
       gates:        the gate masks of this forward from ``chain.gate_log`` (one per ReLU / LeakyReLU stage, in order),
                     applied as where(mask, h, slope * h), so that both runs differentiate the same branch;
       round_grads:  gradients are rounded to bf16 where the chain stores them (every inter-stage buffer, the
@@ -179,16 +184,21 @@ def emulate(ours_seq, ref_seq, x, update_running=False, gates=None, round_grads=
             h = TF.conv2d(hin, w, conv.bias, stride=st.stride, padding=st.pad)
         else:
             h = TF.conv_transpose2d(hin, w, conv.bias, stride=st.stride, padding=st.pad)
-        if st.bn is not None:
+        if p.bn is not None:
+            # both modes round the conv output to bf16 before normalising it (the chain stores it so), and the
+            # BatchNorm dz the chain stores in bf16 is the _RoundGrad above
             bn = ref_mods[idx[id(st.bn)]]
-            mean = h.mean((0, 2, 3))
-            var = h.var((0, 2, 3), unbiased=False)
-            if update_running:
-                with torch.no_grad():
-                    cnt = h.numel() // h.shape[1]
-                    bn.running_mean.mul_(1 - bn.momentum).add_(bn.momentum * mean.detach())
-                    bn.running_var.mul_(1 - bn.momentum).add_(bn.momentum * var.detach() * cnt / (cnt - 1))
-                    bn.num_batches_tracked.add_(1)
+            if p.bn == "eval":
+                mean, var = bn.running_mean.to(h.dtype), bn.running_var.to(h.dtype)
+            else:
+                mean = h.mean((0, 2, 3))
+                var = h.var((0, 2, 3), unbiased=False)
+                if update_running:
+                    with torch.no_grad():
+                        cnt = h.numel() // h.shape[1]
+                        bn.running_mean.mul_(1 - bn.momentum).add_(bn.momentum * mean.detach())
+                        bn.running_var.mul_(1 - bn.momentum).add_(bn.momentum * var.detach() * cnt / (cnt - 1))
+                        bn.num_batches_tracked.add_(1)
             hb = rb(h)
             h = (hb - mean[None, :, None, None]) * torch.rsqrt(var + bn.eps)[None, :, None, None]
             h = h * bn.weight[None, :, None, None] + bn.bias[None, :, None, None]

@@ -65,30 +65,3 @@ def test_eval_catalogue_covers_every_family_in_front_of_a_batchnorm():
     assert layouts == {"nhwc8", "generic"}, layouts
     assert acts == {ACT_NONE, ACT_RELU, ACT_LRELU, ACT_TANH, ACT_SIGMOID}, acts
 
-
-def test_eval_referee_equals_the_training_referee_on_training_stacks():
-    """tests/bf16_emul_eval.py differs from tests/bf16_emul.py only for eval-mode BatchNorm: on every stack of the stage
-    catalogue in training mode both give the same output, gradients and running statistics, bit for bit (float64, CPU)"""
-    import copy
-    import bf16_emul
-    import bf16_emul_eval
-    import eadgan_b200.nn as enn
-    from test_chain_stages_gpu import STAGES, build
-
-    for name, spec, shape in STAGES:
-        torch.manual_seed(1)
-        ours = build(enn, spec)
-        ref = build(torch.nn, spec).double()
-        ref.load_state_dict(ours.state_dict())
-        x = torch.randn(*shape, dtype=torch.float64)
-        runs = []
-        for emul in (bf16_emul, bf16_emul_eval):
-            r = copy.deepcopy(ref)
-            xe = x.clone().requires_grad_()
-            y = emul.emulate(ours, r, xe, update_running=True, round_grads=True, sn_epilogue=True)
-            params = [p for _, p in r.named_parameters()]
-            grads = torch.autograd.grad(y, [xe] + params, torch.ones_like(y))
-            runs.append([y.detach()] + list(grads) + [t for k, t in r.state_dict().items() if "running" in k])
-        assert len(runs[0]) == len(runs[1])
-        for a, b in zip(*runs):
-            assert torch.equal(a, b), name

@@ -2,9 +2,8 @@
 
 ``EVAL_STAGES`` are the BatchNorm-bearing entries of tests/test_chain_stages_gpu.py plus a tensor-core Conv2d and a thin
 Conv2d in front of a BatchNorm.  Each runs with every BatchNorm in eval mode (random running statistics, gamma and beta)
-through the chain with its gates logged, and through the fp64 referee of tests/bf16_emul_eval.py (tests/bf16_emul.py's
-referee with eval-mode BatchNorm) with the same gates forced: output, input gradient and every parameter gradient within
-STAGE_MAX.  The conv bias in front of an eval BatchNorm has a
+through the chain with its gates logged, and through the fp64 referee of tests/bf16_emul.py with the same gates forced:
+output, input gradient and every parameter gradient within STAGE_MAX.  The conv bias in front of an eval BatchNorm has a
 real gradient (gamma * rsqrt(running_var + eps) * sum dz) and is compared like any other tensor.  The running statistics
 and num_batches_tracked must not move."""
 import copy
@@ -65,7 +64,7 @@ def run_eval_entry(spec, shape, dev, seed=0, train_idx=()):
     """-> ({tensor: error against the fp64 referee}, {tensor: error of the frozen / no-input-gradient runs against the
     full run}, {buffer: bit-identical before and after})"""
     import eadgan_b200.nn as enn
-    import bf16_emul_eval
+    import bf16_emul
     os.environ["EADGAN_PRECISION"] = "bf16"
     torch.manual_seed(seed)
     gen = torch.Generator().manual_seed(seed + 100)
@@ -92,7 +91,7 @@ def run_eval_entry(spec, shape, dev, seed=0, train_idx=()):
                 unchanged[f"{i}.{b}"] = torch.equal(after[f"{i}.{b}"], sd0[f"{i}.{b}"])
 
     xe = x.double().requires_grad_()
-    ye = bf16_emul_eval.emulate(ours, ref, xe, update_running=True, gates=gates, round_grads=True, sn_epilogue=True)
+    ye = bf16_emul.emulate(ours, ref, xe, update_running=True, gates=gates, round_grads=True, sn_epilogue=True)
     gse = torch.autograd.grad(ye, [xe] + [p for _, p in ref.named_parameters()], go.double())
     errs = {"y": rel_err(yo, ye)}
     ref_g = dict(zip(names, gse))
