@@ -433,8 +433,9 @@ def sample_dsprites(rs: np.random.RandomState, batch, code_dim=4, n_classes=3):
     return d
 
 
-def step_dsprites(st, img_u8, draws, record=True):
-    """One iteration of dSprites/rp.py:362-482 on ``img_u8`` uint8 [B,64,64]."""
+def step_dsprites(st, img_u8, draws, record=True, after_phase=None):
+    """One iteration of dSprites/rp.py:362-482 on ``img_u8`` uint8 [B,64,64].  ``after_phase(0)`` runs after the
+    optimiser step of phase D, as in step_celeba."""
     Epxy, E, D, G = st["Epxy"], st["E"], st["D"], st["G"]
     dt = next(G.parameters()).dtype
     dev = next(G.parameters()).device
@@ -468,6 +469,8 @@ def step_dsprites(st, img_u8, draws, record=True):
         rec["phases"][-1]["params_after"] = _params(st["opt_D"])
         rec["phases"][-1]["state_after"] = {k: {n: v.detach().clone() for n, v in st[k].state_dict().items()}
                                             for k in ("G", "D", "E")}
+    if after_phase is not None:
+        after_phase(0)
 
     # ---- phase info  (:424-482)
     code = draws["code_info"].to(dev, dt)
@@ -518,8 +521,9 @@ def sample_colored(rs: np.random.RandomState, batch, code_dim=7, n_classes=3):
     return d
 
 
-def step_colored(st, img_u8, draws, record=True):
-    """One iteration of colored_dSprites/rp_color.py:362-516 on ``img_u8`` uint8 [B,64,64]."""
+def step_colored(st, img_u8, draws, record=True, after_phase=None):
+    """One iteration of colored_dSprites/rp_color.py:362-516 on ``img_u8`` uint8 [B,64,64].  ``after_phase(0)`` runs
+    after the optimiser step of phase D, as in step_celeba."""
     Epxy, E, D, G = st["Epxy"], st["E"], st["D"], st["G"]
     dt = next(G.parameters()).dtype
     dev = next(G.parameters()).device
@@ -559,6 +563,8 @@ def step_colored(st, img_u8, draws, record=True):
         rec["phases"][-1]["params_after"] = _params(st["opt_D"])
         rec["phases"][-1]["state_after"] = {k: {n: v.detach().clone() for n, v in st[k].state_dict().items()}
                                             for k in ("G", "D", "E")}
+    if after_phase is not None:
+        after_phase(0)
 
     # ---- phase info  (:444-516)
     code = draws["code_info"].to(dev, dt)
@@ -746,8 +752,9 @@ def sample_mnist(rs: np.random.RandomState, batch, latent_dim=62, code_dim=7, n_
             "labels": torch.tensor(labels, dtype=torch.long)}
 
 
-def step_mnist(st, imgs, draws, record=True):
-    """One iteration of MNIST/EAD-GAN_rpqmnxy.py:337-446 on ``imgs`` [B,1,32,32] in [-1,1]."""
+def step_mnist(st, imgs, draws, record=True, after_phase=None):
+    """One iteration of MNIST/EAD-GAN_rpqmnxy.py:337-446 on ``imgs`` [B,1,32,32] in [-1,1].  ``after_phase(i)`` runs
+    after the optimiser step of phase i = 0 (G), 1 (D), as in step_celeba."""
     A, G, D, E = st["A"], st["G"], st["D"], st["E"]
     dt = next(G.parameters()).dtype
     dev = next(G.parameters()).device
@@ -763,7 +770,7 @@ def step_mnist(st, imgs, draws, record=True):
     scaled = stn(real, mnist_get_matrix(code)[:, 0:2])                         # :363-365
     rec = {"phases": []}
 
-    def snap(name, opt, nets):
+    def snap(name, opt, phase):
         if record:
             rec["phases"].append({"name": name, "grads": _snap(opt)})
         opt.step()
@@ -771,18 +778,20 @@ def step_mnist(st, imgs, draws, record=True):
             rec["phases"][-1]["params_after"] = _params(opt)
             rec["phases"][-1]["state_after"] = {k: {n: v.detach().clone() for n, v in st[k].state_dict().items()}
                                                 for k in ("G", "D", "E")}
+        if after_phase is not None and phase is not None:
+            after_phase(phase)
 
     # ---- phase G  (:373-386)
     st["opt_G"].zero_grad()
     gen = G(z, lab, code)
     g_loss = mse(D(gen), valid)
     g_loss.backward()
-    snap("G", st["opt_G"], None)
+    snap("G", st["opt_G"], 0)
     # ---- phase D  (:393-407)
     st["opt_D"].zero_grad()
     d_loss = (mse(D(scaled), valid) + mse(D(gen.detach()), fake)) / 2
     d_loss.backward()
-    snap("D", st["opt_D"], None)
+    snap("D", st["opt_D"], 1)
     # ---- phase info  (:413-446)
     st["opt_info"].zero_grad()
     gen = G(z, lab, code)

@@ -2,20 +2,32 @@
 
 A ReLU / LeakyReLU network is piecewise linear in its parameters' gradients: a single gate that differs between
 two evaluations (a pre-activation within rounding of 0) moves EVERY upstream gradient by a finite amount, whatever
-the quality of the kernels.  To hold every gradient tensor of the bf16 tensor-core step to north_star's 2e-2, the
+the quality of the kernels.  To hold every gradient tensor of a bf16 tensor-core step to north_star's 2e-2, the
 oracle is therefore evaluated on the SAME piecewise-linear branch as our run:
 
-  1. our step runs with ``eadgan_b200.chain.gate_log`` switched on: every conv stack records, per ReLU / LeakyReLU
-     stage, the mask ``saved output > 0`` -- the very bits its fused backward kernels read;
-  2. the oracle's ``nn.ReLU`` / ``nn.LeakyReLU`` modules are replaced by ``ForcedGate`` modules that consume those
-     masks in call order: y = where(mask, x, slope * x).  Where the oracle's own gate agrees (all but ~0.1 % of the
+  1. our step runs with ``eadgan_b200.chain.gate_log`` switched on: every Sequential records, per ReLU / LeakyReLU
+     stage and per call, the mask ``output > 0`` -- for a chain stack the very bits its fused backward kernels read;
+  2. the oracle's ``nn.ReLU`` / ``nn.LeakyReLU`` modules are replaced by ``ForcedGate`` modules that consume the
+     masks logged by the Sequential of the same qualified name (``G.conv_block``, ``D.fc1``, ``A.fc_block``, ...),
+     in call order: y = where(mask, x, slope * x).  Where the oracle's own gate agrees (all but ~0.1 % of the
      elements) this IS ReLU / LeakyReLU; where it does not, |x| is within bf16 rounding of 0, so the forward value
      moves by less than one bf16 ulp of the activation scale.
 
-What is left between the two runs is rounding of smooth arithmetic, which the 2e-2 bound is about."""
+The frozen Encoder_pxy of the dSprites steps sets the alignment grid of every real image; its code is forced too
+(the oracle's own code is kept for comparison), so that a rounding-level difference of that code does not move the
+sampled sprite edges under D and E.  What is left between the two runs is rounding of smooth arithmetic, which the
+2e-2 bound is about."""
+import os
+
 import numpy as np
 import torch
 import torch.nn as tnn
+
+GATED = (tnn.ReLU, tnn.LeakyReLU)
+
+# the networks of each configuration's step, by attribute name (ours) == state key (oracle)
+NETS = {"celeba": ("G", "D"), "dsprites": ("Epxy", "E", "D", "G"), "colored": ("Epxy", "E", "D", "G"),
+        "mnist": ("A", "G", "D", "E"), "pxy": ("E",), "pxy_color": ("E",)}
 
 
 class ForcedGate(tnn.Module):
@@ -46,60 +58,160 @@ def install(seq, queue):
     return gates
 
 
-def celeba_forced(dev, B, precision="bf16", seed=0, oracle_dtypes=(torch.float64,)):
+def sequentials(nets):
+    """{qualified name: Sequential} over ``nets`` = {key: module}, e.g. 'G.conv_block', 'D.fc1'"""
+    return {f"{key}.{name}": m for key, net in nets.items() for name, m in net.named_modules()
+            if isinstance(m, tnn.Sequential)}
+
+
+def oracle_gates(nets):
+    """{qualified name: number of ReLU / LeakyReLU children} of the oracle's Sequentials"""
+    return {qn: sum(isinstance(m, GATED) for m in seq.children()) for qn, seq in sequentials(nets).items()}
+
+
+def our_gates(nets):
+    """{qualified name: number of gated stages} of our Sequentials: one logged mask per ReLU / LeakyReLU per call"""
+    from eadgan_b200 import nn as enn
+    from eadgan_b200._lib import ACT_LRELU, ACT_RELU
+    return {qn: sum(isinstance(m, enn._Act) and m.act()[0] in (ACT_RELU, ACT_LRELU) for m in seq.children())
+            for qn, seq in sequentials(nets).items()}
+
+
+def _setup(config, dev, B, seed):
+    """-> (build(dtype) -> oracle state, run_oracle(st, dtype, after_phase) -> record, our step,
+    run_ours(record, after_phase) -> losses, the phases after which both runs restart from the free oracle)"""
+    from oracle import torch_oracle as O
+    rs = np.random.RandomState(seed)
+    if config == "celeba":
+        from eadgan_b200.steps.celeba import CelebAStep
+        imgs, d = O.synth_celeba_images(B, seed).to(dev), O.sample_celeba(rs, B)
+        ours = CelebAStep(seed=seed, device=dev)
+        return (lambda dt: O.build_celeba(seed=seed, device=dev, dtype=dt),
+                lambda st, dt, after: O.step_celeba(st, imgs.to(dt), d, after_phase=after), ours,
+                lambda rec, after: ours(imgs, d["z"].to(dev), d["code"].to(dev), d["labels"].to(dev), record=rec,
+                                        after_phase=after), (0, 1))
+    if config in ("dsprites", "colored"):
+        colored = config == "colored"
+        imgs = O.synth_dsprites_images(B, seed).to(dev)
+        if colored:
+            from eadgan_b200.steps.colored import ColoredDSpritesStep as Step
+            d = O.sample_colored(rs, B)
+            extra, step_fn = (d["color"].to(dev),), O.step_colored
+        else:
+            from eadgan_b200.steps.dsprites import DSpritesStep as Step
+            d = O.sample_dsprites(rs, B)
+            extra, step_fn = (), O.step_dsprites
+        ours = Step(seed=seed, device=dev, pxy_state=O.dsprites_pxy_state(seed, colored=colored))
+        return (lambda dt: O.build_dsprites(seed=seed, device=dev, dtype=dt, colored=colored),
+                lambda st, dt, after: step_fn(st, imgs, d, after_phase=after), ours,
+                lambda rec, after: ours(imgs, *extra, d["code_d"].to(dev), d["labels_d"].to(dev),
+                                        d["code_info"].to(dev), d["labels_info"].to(dev), record=rec,
+                                        after_phase=after), (0,))
+    if config == "mnist":
+        from eadgan_b200.steps.mnist import MnistStep
+        imgs, d = O.synth_mnist_images(B, seed).to(dev), O.sample_mnist(rs, B)
+        ours = MnistStep(seed=seed, device=dev, approximator_state=O.mnist_approximator_state(seed))
+        return (lambda dt: O.build_mnist(seed=seed, device=dev, dtype=dt),
+                lambda st, dt, after: O.step_mnist(st, imgs, d, after_phase=after), ours,
+                lambda rec, after: ours(imgs, d["z"].to(dev), d["code"].to(dev), d["labels"].to(dev), record=rec,
+                                        after_phase=after), (0, 1))
+    if config in ("pxy", "pxy_color"):
+        from eadgan_b200.steps.pxy import PxyStep
+        colored = config == "pxy_color"
+        imgs, d = O.synth_dsprites_images(B, seed).to(dev), O.sample_pxy(rs, B, colored)
+        ours = PxyStep(seed=seed, device=dev, colored=colored)
+        return (lambda dt: O.build_pxy(seed=seed, device=dev, dtype=dt, colored=colored),
+                lambda st, dt, after: O.step_pxy(st, imgs, d), ours,
+                lambda rec, after: ours(imgs, d["code"].to(dev), d["color"].to(dev) if colored else None,
+                                        record=rec), ())
+    raise ValueError(config)
+
+
+def _cast(sd, dt):
+    return {k: v.to(dt) if v.is_floating_point() else v for k, v in sd.items()}
+
+
+def _state(nets):
+    return {key: {k: v.detach().clone() for k, v in net.state_dict().items()} for key, net in nets.items()}
+
+
+def net_states(step, config):
+    """{net: state_dict} of our step's networks, keyed as the forced records' ``state``"""
+    return _state({k: getattr(step, k) for k in NETS[config]})
+
+
+def forced_step(config, dev, B, precision="bf16", seed=0, oracle_dtypes=(torch.float64,)):
     """-> dict(forced=[oracle record per dtype in ``oracle_dtypes``], ours=our per-phase record, losses=our losses,
-    free=free oracle record (first dtype), flips=..., gates=..., step=our step object).
+    free=free oracle record (first dtype), flips=..., gates=..., step=our step object, codes=[our Encoder_pxy
+    outputs]).  Each forced record also carries ``state`` (its nets' state after the step) and, for the dSprites
+    configurations, ``codes`` (the oracle's own Encoder_pxy outputs on the forced gates).
 
     Runs on identical seeded inputs / weights: the free oracle (its post-phase states are the common starting point
-    of every later phase of every run), OUR step (gates logged), then the oracle with OUR gates forced, once per
-    requested dtype (fp64 = the referee; fp32 = stock torch's own rounding error on the same branch)."""
-    import os
+    of every later phase of every run), OUR step (gates logged), then the oracle with OUR gates -- and our
+    Encoder_pxy code -- forced, once per requested dtype (fp64 = the referee; fp32 = stock torch's own rounding
+    error on the same branch)."""
     from eadgan_b200 import chain
-    from eadgan_b200.steps.celeba import CelebAStep
-    from oracle import torch_oracle as O
     os.environ["EADGAN_PRECISION"] = precision
-    imgs = O.synth_celeba_images(B, seed).to(dev)
-    draws = O.sample_celeba(np.random.RandomState(seed), B)
+    build, run_oracle, ours, run_ours, restarts = _setup(config, dev, B, seed)
+    keys = NETS[config]
     dt0 = oracle_dtypes[0]
 
-    free = O.step_celeba(O.build_celeba(seed=seed, device=dev, dtype=dt0), imgs.to(dt0), draws)
-    states = [free["phases"][i]["state_after"] for i in range(2)]
+    free = run_oracle(build(dt0), dt0, None)
+    states = {i: free["phases"][i]["state_after"] for i in restarts}
 
-    def cast(sd, dt):
-        return {k: v.to(dt) if v.is_floating_point() else v for k, v in sd.items()}
+    def restart(nets, dt):
+        def after_phase(i):
+            if i in states:
+                for key, sd in states[i].items():
+                    nets[key].load_state_dict(_cast(sd, dt))
+        return after_phase
 
-    ours = CelebAStep(seed=seed, device=dev)
-
-    def load_ours(i):
-        ours.G.load_state_dict(cast(states[i]["G"], torch.float32))
-        ours.D.load_state_dict(cast(states[i]["D"], torch.float32))
-
+    our_nets = {k: getattr(ours, k) for k in keys}
+    codes = []
+    hooks = [ours.Epxy.register_forward_hook(lambda m, a, out: codes.append(out.detach().clone()))] \
+        if "Epxy" in keys else []
     rec = []
     chain.gate_log = []
     try:
-        losses = ours(imgs, draws["z"].to(dev), draws["code"].to(dev), draws["labels"].to(dev), record=rec,
-                      after_phase=load_ours)
+        losses = run_ours(rec, restart(our_nets, torch.float32))
         log = chain.gate_log
     finally:
         chain.gate_log = None
-    qG = [m for seq, masks in log if seq is ours.G.conv_blocks for m in masks]
-    qD = [m for seq, masks in log if seq is ours.D.main for m in masks]
-    assert len(qG) == 2 * 3 and len(qD) == 6 * 4, (len(qG), len(qD))
+        for h in hooks:
+            h.remove()
+    names = {id(seq): qn for qn, seq in sequentials(our_nets).items()}
+    masks = {}
+    for seq, ms in log:
+        masks.setdefault(names[id(seq)], []).extend(ms)
 
     forced, flips, total = [], 0, 0
     for dt in oracle_dtypes:
-        st = O.build_celeba(seed=seed, device=dev, dtype=dt)
-        g_q, d_q = list(qG), list(qD)
-        gates = install(st["G"].conv_blocks, g_q) + install(st["D"].main, d_q)
-
-        def load_ref(i, _st=st, _dt=dt):
-            _st["G"].load_state_dict(cast(states[i]["G"], _dt))
-            _st["D"].load_state_dict(cast(states[i]["D"], _dt))
-
-        forced.append(O.step_celeba(st, imgs.to(dt), draws, after_phase=load_ref))
-        assert not g_q and not d_q
+        st = build(dt)
+        nets = {k: st[k] for k in keys}
+        queues = {qn: list(ms) for qn, ms in masks.items()}
+        gates = []
+        for qn, seq in sequentials(nets).items():
+            gates += install(seq, queues.setdefault(qn, []))
+        assert not [m for net in nets.values() for m in net.modules() if isinstance(m, GATED)], "unforced gate"
+        own, code_q = [], list(codes)
+        if "Epxy" in keys:
+            def force_code(m, a, out, _dt=dt):
+                own.append(out.detach().clone())
+                return code_q.pop(0).to(_dt)
+            st["Epxy"].register_forward_hook(force_code)
+        r = run_oracle(st, dt, restart(nets, dt))
+        assert not any(queues.values()), {qn: len(q) for qn, q in queues.items() if q}
+        assert not code_q
+        r["state"], r["codes"] = _state(nets), own
+        r["flips"], r["gates"] = sum(g.flips for g in gates), sum(g.total for g in gates)
         if dt == dt0:
-            flips, total = sum(g.flips for g in gates), sum(g.total for g in gates)
-        del st
+            flips, total = r["flips"], r["gates"]
+        forced.append(r)
+        del st, nets
     return {"forced": forced, "ours": rec, "losses": {k: float(v) for k, v in losses.items()}, "free": free,
-            "flips": flips, "gates": total, "step": ours}
+            "flips": flips, "gates": total, "step": ours, "codes": codes}
+
+
+def celeba_forced(dev, B, precision="bf16", seed=0, oracle_dtypes=(torch.float64,)):
+    """the CelebA step of ``forced_step`` (bench.py's parity block calls it by this name)"""
+    return forced_step("celeba", dev, B, precision, seed, oracle_dtypes)

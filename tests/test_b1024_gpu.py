@@ -193,7 +193,7 @@ def test_celeba_step_b1024_forced_gates(cuda):
     losses and every gradient tensor of every phase to north_star's 2e-2."""
     import gates
     import step_util as U
-    out = gates.celeba_forced(cuda, N, "bf16", oracle_dtypes=(torch.float32,))
+    out = gates.forced_step("celeba", cuda, N, "bf16", oracle_dtypes=(torch.float32,))
     ref = out["forced"][0]
     assert out["flips"] <= 0.01 * out["gates"]
     names = U.grad_names(out["step"])

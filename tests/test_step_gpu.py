@@ -122,7 +122,7 @@ def test_celeba_step_bf16_forced_gates(cuda, B):
     """north_star's bf16 bound on EVERY gradient tensor of EVERY phase: max|ours - oracle| / max|oracle| <= 2e-2
     with the fp64 oracle evaluated on the activation gates of our run (tests/gates.py)."""
     import gates
-    out = gates.celeba_forced(cuda, B, "bf16")
+    out = gates.forced_step("celeba", cuda, B, "bf16")
     assert out["flips"] <= 0.01 * out["gates"]          # the forced branch is the oracle's own up to ~0.1-0.3 %
     worst = _assert_forced(out, 2e-2, f"bf16 B={B}")
     print(f"bf16 B={B}: gate flips {out['flips']} of {out['gates']}, worst tensor-normalised gradient error {worst:.2e}")
@@ -132,7 +132,7 @@ def test_celeba_step_fp32_relative_to_stock_fp32(cuda):
     """SURVEY.md section 7.3-1 (ii): with fp64 as referee, OUR fp32 error may not exceed 3x stock torch fp32's own
     error (cuDNN / cuBLAS, TF32 off) on the same inputs, tensor by tensor -- all three runs on the same gates."""
     import gates
-    out = gates.celeba_forced(cuda, 8, "fp32", oracle_dtypes=(torch.float64, torch.float32))
+    out = gates.forced_step("celeba", cuda, 8, "fp32", oracle_dtypes=(torch.float64, torch.float32))
     ref64, ref32 = out["forced"]
     for k in ("g_loss", "d_loss", "info_loss"):
         assert abs(out["losses"][k] - ref64["losses"][k]) <= 2e-5 * max(1.0, abs(ref64["losses"][k])), k
