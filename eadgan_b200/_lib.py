@@ -87,6 +87,7 @@ _PROTOS = {
     "eadgan_spectral_norm_fwd": [_P, _I, _I, _P, _P, _I, _F, _P, _P, _P, _P],
     "eadgan_spectral_norm_scale": [_P, _P, _P, C.c_longlong, _P],
     "eadgan_spectral_norm_bwd": [_P, _P, _P, _P, _P, _I, _I, _P, _P, _P],
+    "eadgan_fold_bn_sn": [_P, C.c_longlong, _I, C.c_longlong, _P, _P, _P, _P, _P, _D, _P, _P, _P, _P],
     "eadgan_bce_fwd": [_P, _P, _L, _P, _P],
     "eadgan_bce_bwd": [_P, _P, _P, _L, _P, _P],
     "eadgan_mse_fwd": [_P, _P, _L, _P, _P],

@@ -1,5 +1,5 @@
-// Pointwise activations, row softmax, nearest 2x upsample, fill, and the error /
-// version plumbing of the C ABI.  All kernels are HBM-bound streaming passes:
+// Pointwise activations, row softmax, nearest 2x upsample, fill, the BatchNorm / spectral-norm
+// weight fold of freeze(), and the error / version plumbing of the C ABI.  All kernels are HBM-bound streaming passes:
 // 128-bit vectorised loads/stores, grid sized to a multiple of the SM count.
 // Reference call sites: nn.LeakyReLU / nn.ReLU / nn.Tanh / F.sigmoid / F.softmax /
 // nn.Softmax / nn.Upsample in celebA/EAD-GAN_celebA.py:80-92,111-134,
@@ -235,6 +235,49 @@ __global__ void zero_halo_kernel(uint4* __restrict__ xp, int n, int h, int w, in
   }
 }
 }  // namespace
+
+namespace {
+// W viewed as [outer, c, inner] (c = output channels).  One thread per weight element; the first c threads also
+// write the bias.  The scale s[j] is recomputed per element in fp64 (this runs once per layer, at freeze time).
+__global__ void __launch_bounds__(256) fold_bn_sn_kernel(const float* __restrict__ w, int64_t outer, int c,
+                                                         int64_t inner, const float* __restrict__ sigma,
+                                                         const float* __restrict__ gamma, const float* __restrict__ beta,
+                                                         const float* __restrict__ rmean, const float* __restrict__ rvar,
+                                                         double eps, const float* __restrict__ bias,
+                                                         float* __restrict__ w_out, float* __restrict__ b_out) {
+  const double inv_sigma = sigma != nullptr ? 1.0 / (double)__ldg(sigma) : 1.0;
+  const int64_t n = outer * c * inner;
+  const int64_t tid = blockIdx.x * (int64_t)blockDim.x + threadIdx.x, nth = (int64_t)gridDim.x * blockDim.x;
+  for (int64_t i = tid; i < n; i += nth) {
+    const int j = (int)((i / inner) % c);
+    const double s = gamma != nullptr ? (double)gamma[j] / sqrt((double)rvar[j] + eps) : 1.0;
+    w_out[i] = (float)((double)w[i] * (s * inv_sigma));
+  }
+  if (b_out != nullptr) {
+    for (int64_t j = tid; j < c; j += nth) {
+      const double b = bias != nullptr ? (double)bias[j] : 0.0;
+      b_out[j] = gamma != nullptr
+                     ? (float)((b - (double)rmean[j]) * ((double)gamma[j] / sqrt((double)rvar[j] + eps)) + (double)beta[j])
+                     : (float)b;
+    }
+  }
+}
+}  // namespace
+
+extern "C" int eadgan_fold_bn_sn(const float* w, long long outer, int c, long long inner, const float* sigma,
+                                 const float* gamma, const float* beta, const float* running_mean,
+                                 const float* running_var, double eps, const float* bias, float* w_out, float* b_out,
+                                 void* stream) {
+  const bool bn = gamma != nullptr;
+  EG_REQUIRE(w && w_out && outer > 0 && c > 0 && inner > 0 && w != w_out && (sigma || bn) &&
+                 bn == (beta && running_mean && running_var) && (b_out == nullptr || bn),
+             EADGAN_ERR_INVALID, "fold_bn_sn: bad arguments");
+  const int64_t n = (int64_t)outer * c * inner;
+  fold_bn_sn_kernel<<<stream_grid(n, 1024), 256, 0, (cudaStream_t)stream>>>(
+      w, outer, c, inner, sigma, gamma, beta, running_mean, running_var, eps, bias, w_out, b_out);
+  EG_LAUNCH_CHECK("fold_bn_sn_kernel");
+  return 0;
+}
 
 extern "C" int eadgan_f64_to_f32(const double* src, float* dst, int64_t numel, void* stream) {
   EG_REQUIRE(src && dst && numel > 0, EADGAN_ERR_INVALID, "f64_to_f32: bad arguments");

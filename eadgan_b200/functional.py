@@ -426,6 +426,35 @@ def spectral_norm_materialize(w_orig, sigma, w_sn):
     call("eadgan_spectral_norm_scale", ptr(w_orig.detach().contiguous()), ptr(sigma), ptr(w_sn), w_sn.numel(), stream())
 
 
+def spectral_norm_sigma(w_orig, u, v, eps):
+    """sigma = u^T W v from the stored u, v: the eval-mode spectral norm (no power iteration; u, v are only read)
+    -> fp32 [1] device tensor."""
+    w = _f32(w_orig, "spectral_norm").detach().contiguous()
+    rows = w.shape[0]
+    cols = w.numel() // rows
+    sigma = torch.empty(1, device=w.device, dtype=torch.float32)
+    scratch = torch.empty(L.lib().eadgan_spectral_norm_scratch_floats(rows, cols, 0), device=w.device,
+                          dtype=torch.float32)
+    call("eadgan_spectral_norm_fwd", ptr(w), rows, cols, ptr(u), ptr(v), 0, float(eps), ptr(sigma), None,
+         ptr(scratch), stream())
+    return sigma
+
+
+def fold_bn_sn(w, channel_dim, sigma=None, bn=None, bias=None):
+    """(W', b') of a layer with its legacy spectral norm (sigma: the fp32 [1] device scalar) and / or the eval-mode
+    BatchNorm2d after it folded in, along the output-channel axis ``channel_dim`` of W (0: Conv2d / Linear, 1:
+    ConvTranspose2d).  b' is None without a BatchNorm (the bias is unchanged then)."""
+    w = _f32(w, "fold_bn_sn").detach().contiguous()
+    c = w.shape[channel_dim]
+    outer = w.shape[0] if channel_dim == 1 else 1
+    w_out = torch.empty_like(w)
+    b_out = torch.empty(c, device=w.device, dtype=torch.float32) if bn is not None else None
+    g = (bn.weight, bn.bias, bn.running_mean, bn.running_var) if bn is not None else (None,) * 4
+    call("eadgan_fold_bn_sn", ptr(w), outer, c, w.numel() // (outer * c), ptr(sigma), *(ptr(t) for t in g),
+         float(bn.eps) if bn is not None else 0.0, ptr(bias), ptr(w_out), ptr(b_out), stream())
+    return w_out, b_out
+
+
 def spectral_norm_weight(w_orig, u, v, do_power_iter, eps):
     return _SpectralNormFn.apply(w_orig, u, v, bool(do_power_iter), float(eps))
 

@@ -303,6 +303,24 @@ int eadgan_spectral_norm_bwd(const float* dw_sn, const float* w_orig, const floa
                              float* dw_orig, float* scratch, void* stream);
 
 /* ------------------------------------------------------------------------- */
+/* eadgan_b200.freeze(): fold an eval-mode BatchNorm2d and / or a legacy spectral norm into the   */
+/* weight and bias of the Conv2d / ConvTranspose2d / Linear in front of it.  Replaces              */
+/* torch.nn.utils.fusion.fuse_conv_bn_weights (transpose=True for ConvTranspose2d) /               */
+/* fuse_linear_bn_weights, and SpectralNorm.compute_weight(do_power_iteration=False) = W / sigma   */
+/* with sigma from eadgan_spectral_norm_fwd(do_power_iter = 0).                                     */
+/* ------------------------------------------------------------------------- */
+/* W is viewed as [outer, c, inner] with c the OUTPUT channels: outer = 1 for Conv2d and Linear (channel dim 0),
+ * outer = input channels for ConvTranspose2d (channel dim 1).  With s[j] = gamma[j] / sqrt(running_var[j] + eps):
+ *   w_out = W * s / sigma            (sigma NULL: no spectral norm; gamma NULL: no BatchNorm, s = 1)
+ *   b_out = (bias - running_mean) * s + beta   (bias NULL: 0; b_out NULL: not written; needs the BatchNorm)
+ * gamma, beta, running_mean and running_var are all given or all NULL; sigma or gamma must be given.
+ * Arithmetic in fp64, one rounding to fp32.  w_out must not alias w. */
+int eadgan_fold_bn_sn(const float* w, long long outer, int c, long long inner, const float* sigma,
+                      const float* gamma, const float* beta, const float* running_mean,
+                      const float* running_var, double eps, const float* bias, float* w_out, float* b_out,
+                      void* stream);
+
+/* ------------------------------------------------------------------------- */
 /* losses, forward + backward (celebA/EAD-GAN_celebA.py:161-164;               */
 /* dSprites/rp.py:225-232,249-251; MNIST/EAD-GAN_rpqmnxy.py:195-198)           */
 /* loss outputs are single device floats; *_bwd multiply by the upstream       */

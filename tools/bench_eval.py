@@ -5,12 +5,15 @@
 Paths, all on the same seeded inputs and generator state (random running statistics, .eval()):
   ours_bf16       eadgan_b200 with EADGAN_PRECISION=bf16 (tcgen05 chain, eval-mode BatchNorm on the chain)
   ours_fp32       eadgan_b200 with EADGAN_PRECISION=fp32 (the fp32 SIMT per-operator path)
+  ours_bf16_frozen  eadgan_b200.freeze() of the same generator, bf16 (BatchNorm folded into the ConvTranspose weights
+                  and biases; forward only: a frozen copy does not differentiate)
   torch_tf32      the stock oracle module through cuDNN with TF32 allowed
   torch_bf16_amp  the stock oracle module under torch.autocast(dtype=torch.bfloat16)
 
 Each case is warmed up, then timed with CUDA events over a window of at least --window seconds.  One JSON line per case
 goes to stdout (and to --out); the first line names the device and its power limit.  --profile writes a
-torch.profiler kernel list of ONE bf16 eval forward at the largest batch (a separate run, after the timing)."""
+torch.profiler kernel list of ONE bf16 eval forward at the largest batch (a separate run, after the timing),
+--profile-frozen the same for the frozen copy."""
 import argparse
 import json
 import os
@@ -61,8 +64,9 @@ def inputs(B, dev):
     return z, lab, code, go
 
 
-def make_fn(path, mode, ours, ref, z, lab, code, go):
-    net = ours if path.startswith("ours") else ref
+def make_fn(path, mode, nets, z, lab, code, go):
+    ours, frozen, ref = nets
+    net = frozen if path == "ours_bf16_frozen" else ours if path.startswith("ours") else ref
 
     def run():
         ctx = (torch.autocast("cuda", dtype=torch.bfloat16) if path == "torch_bf16_amp"
@@ -113,25 +117,29 @@ def main():
     ap.add_argument("--window", type=float, default=1.0)
     ap.add_argument("--out", default=None)
     ap.add_argument("--profile", default=None)
+    ap.add_argument("--profile-frozen", default=None)
     args = ap.parse_args()
     if not torch.cuda.is_available():
         sys.exit("bench_eval.py needs a CUDA device")
     dev = torch.device("cuda:0")
+    import eadgan_b200
     ours, ref = make_nets(dev)
+    nets = (ours, eadgan_b200.freeze(ours), ref)
     lines = [dict(device_info(), what="CelebA generator, eval mode, random running statistics")]
     print(json.dumps(lines[0]), flush=True)
-    paths = ("ours_bf16", "ours_fp32", "torch_tf32", "torch_bf16_amp")
+    all_paths = ("ours_bf16", "ours_bf16_frozen", "ours_fp32", "torch_tf32", "torch_bf16_amp")
     for B in [int(b) for b in args.batches.split(",")]:
         z, lab, code, go = inputs(B, dev)
         outs = {}
         for mode in ("forward", "forward_backward_z"):
+            paths = all_paths if mode == "forward" else tuple(p for p in all_paths if p != "ours_bf16_frozen")
             for path in paths:     # results first: every path is compared with the fp32 one
                 set_path(path)
-                outs[(mode, path)] = make_fn(path, mode, ours, ref, z, lab, code, go)().float()
+                outs[(mode, path)] = make_fn(path, mode, nets, z, lab, code, go)().float()
             base = outs[(mode, "ours_fp32")]
             for path in paths:
                 set_path(path)
-                sec, iters, total = time_case(make_fn(path, mode, ours, ref, z, lab, code, go), args.window)
+                sec, iters, total = time_case(make_fn(path, mode, nets, z, lab, code, go), args.window)
                 rec = {"batch": B, "mode": mode, "path": path, "ms": round(sec * 1e3, 4),
                        "samples_per_s": round(B / sec, 1), "iters": iters, "window_s": round(total, 3)}
                 if path != "ours_fp32":
@@ -143,18 +151,21 @@ def main():
         with open(args.out, "w") as f:
             for rec in lines:
                 f.write(json.dumps(rec) + "\n")
-    if args.profile:
+    for out, net, what in ((args.profile, ours, "one bf16 eval forward"),
+                           (args.profile_frozen, nets[1], "one bf16 forward of the frozen copy (freeze())")):
+        if not out:
+            continue
         from torch.profiler import ProfilerActivity, profile
         z, lab, code, _ = inputs(max(int(b) for b in args.batches.split(",")), dev)
         with torch.no_grad():
-            ours(z, lab, code)
+            net(z, lab, code)
             torch.cuda.synchronize()
             with profile(activities=[ProfilerActivity.CUDA]) as prof:
-                ours(z, lab, code)
+                net(z, lab, code)
                 torch.cuda.synchronize()
         evs = [e for e in prof.events() if e.device_type.name == "CUDA"]
-        with open(args.profile, "w") as f:
-            f.write(f"# {json.dumps(lines[0])}\n# one bf16 eval forward of the CelebA generator, batch {z.shape[0]}, "
+        with open(out, "w") as f:
+            f.write(f"# {json.dumps(lines[0])}\n# {what} of the CelebA generator, batch {z.shape[0]}, "
                     f"warm pack cache; {len(evs)} device activities in launch order (us, name)\n")
             for e in evs:
                 f.write(f"{e.device_time:10.1f}  {e.name}\n")
