@@ -331,8 +331,8 @@ def _thin_ok(d, direction):
         return False
     if direction == "fprop":
         return d.k % 32 == 0 and d.q <= 128
-    if direction == "dgrad":      # GEMM + col2im epilogue: 32-wide small map, <= 3 image channels
-        return (d.k % 64 == 0 or d.k == 32) and d.q == 32 and d.c <= 3
+    if direction == "dgrad":      # GEMM + col2im epilogue: 32-wide small map of 2-row tiles, <= 3 image channels
+        return (d.k % 64 == 0 or d.k == 32) and d.q == 32 and d.p >= 2 and d.c <= 3
     return d.k % 32 == 0 and d.q <= 64  # wgrad
 
 

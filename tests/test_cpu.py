@@ -424,6 +424,23 @@ def test_chain_plans_of_small_and_channel_padded_stacks():
     assert _kernel_plan(seq, (8, 64, 8, 8))[0][0] == "tc/tc/tc c64:64 k2048 pad>pad"
 
 
+def test_chain_plans_of_single_row_maps():
+    """a 32-wide small map of ONE row: the thin input-gradient kernel works on 2-row tiles and rejects it, so the plan
+    must send that direction elsewhere (tests/test_tc_geometry_gpu.py runs both stacks forward and backward)"""
+    import eadgan_b200.nn as enn
+    from test_tc_geometry_gpu import P1_CONVT_LAST, P1_THIN_FIRST
+    from test_chain_stages_gpu import build
+
+    # ConvTranspose onto a 3-channel 2x64 image: the tensor-core dgrad with the image channel-padded to 32
+    name, spec, shape = P1_CONVT_LAST
+    assert _kernel_plan(build(enn, spec), shape) == (["simt/simt/simt c64:64 k64 ext>pad",
+                                                      "tc/tc/tc c3:32 k64 pad>ext fuse"], (4, 3, 2, 64)), name
+    # a 3-channel 2x64 image into a thin conv: its image gradient runs on SIMT
+    name, spec, shape = P1_THIN_FIRST
+    assert _kernel_plan(build(enn, spec), shape) == (["thin/thin/simt c3:3 k64 ext>pad",
+                                                      "simt/simt/simt c64:64 k64 pad>ext fuse"], (4, 64, 1, 32)), name
+
+
 # Every (forward, weight gradient, input gradient, input format, output format, fused mask, channel-padded) row and every
 # (BatchNorm, activation) pair that tests/test_chain_stages_gpu.py runs against its fp64 referee.  A planner rule that
 # adds a row makes this test fail until a catalogue entry reaches it.
