@@ -77,53 +77,74 @@ def our_gates(nets):
             for qn, seq in sequentials(nets).items()}
 
 
-def _setup(config, dev, B, seed):
-    """-> (build(dtype) -> oracle state, run_oracle(st, dtype, after_phase) -> record, our step,
-    run_ours(record, after_phase) -> losses, the phases after which both runs restart from the free oracle)"""
+def make_step(config, dev, seed=0):
+    """-> our step object of ``config``, with seeded weights (and the seeded frozen Encoder_pxy / approximator)"""
+    from oracle import torch_oracle as O
+    if config == "celeba":
+        from eadgan_b200.steps.celeba import CelebAStep
+        return CelebAStep(seed=seed, device=dev)
+    if config in ("dsprites", "colored"):
+        from eadgan_b200.steps.colored import ColoredDSpritesStep
+        from eadgan_b200.steps.dsprites import DSpritesStep
+        colored = config == "colored"
+        return (ColoredDSpritesStep if colored else DSpritesStep)(
+            seed=seed, device=dev, pxy_state=O.dsprites_pxy_state(seed, colored=colored))
+    if config == "mnist":
+        from eadgan_b200.steps.mnist import MnistStep
+        return MnistStep(seed=seed, device=dev, approximator_state=O.mnist_approximator_state(seed))
+    if config in ("pxy", "pxy_color"):
+        from eadgan_b200.steps.pxy import PxyStep
+        return PxyStep(seed=seed, device=dev, colored=config == "pxy_color")
+    raise ValueError(config)
+
+
+def batch(config, dev, B, seed):
+    """-> (our step's positional inputs, the oracle's (images, draws)) of one seeded batch of ``config``"""
     from oracle import torch_oracle as O
     rs = np.random.RandomState(seed)
     if config == "celeba":
-        from eadgan_b200.steps.celeba import CelebAStep
         imgs, d = O.synth_celeba_images(B, seed).to(dev), O.sample_celeba(rs, B)
-        ours = CelebAStep(seed=seed, device=dev)
+        return (imgs, d["z"].to(dev), d["code"].to(dev), d["labels"].to(dev)), (imgs, d)
+    if config in ("dsprites", "colored"):
+        imgs = O.synth_dsprites_images(B, seed).to(dev)
+        d = O.sample_colored(rs, B) if config == "colored" else O.sample_dsprites(rs, B)
+        extra = (d["color"].to(dev),) if config == "colored" else ()
+        return (imgs, *extra, d["code_d"].to(dev), d["labels_d"].to(dev), d["code_info"].to(dev),
+                d["labels_info"].to(dev)), (imgs, d)
+    if config == "mnist":
+        imgs, d = O.synth_mnist_images(B, seed).to(dev), O.sample_mnist(rs, B)
+        return (imgs, d["z"].to(dev), d["code"].to(dev), d["labels"].to(dev)), (imgs, d)
+    if config in ("pxy", "pxy_color"):
+        imgs, d = O.synth_dsprites_images(B, seed).to(dev), O.sample_pxy(rs, B, config == "pxy_color")
+        extra = (d["color"].to(dev),) if config == "pxy_color" else ()
+        return (imgs, d["code"].to(dev), *extra), (imgs, d)
+    raise ValueError(config)
+
+
+def _setup(config, dev, B, seed, data_seed):
+    """-> (build(dtype) -> oracle state, run_oracle(st, dtype, after_phase) -> record, our step,
+    run_ours(step, record, after_phase) -> losses, the phases after which both runs restart from the free oracle)"""
+    from oracle import torch_oracle as O
+    args, (imgs, d) = batch(config, dev, B, data_seed)
+    if config == "celeba":
         return (lambda dt: O.build_celeba(seed=seed, device=dev, dtype=dt),
-                lambda st, dt, after: O.step_celeba(st, imgs.to(dt), d, after_phase=after), ours,
-                lambda rec, after: ours(imgs, d["z"].to(dev), d["code"].to(dev), d["labels"].to(dev), record=rec,
-                                        after_phase=after), (0, 1))
+                lambda st, dt, after: O.step_celeba(st, imgs.to(dt), d, after_phase=after),
+                lambda ours, rec, after: ours(*args, record=rec, after_phase=after), (0, 1))
     if config in ("dsprites", "colored"):
         colored = config == "colored"
-        imgs = O.synth_dsprites_images(B, seed).to(dev)
-        if colored:
-            from eadgan_b200.steps.colored import ColoredDSpritesStep as Step
-            d = O.sample_colored(rs, B)
-            extra, step_fn = (d["color"].to(dev),), O.step_colored
-        else:
-            from eadgan_b200.steps.dsprites import DSpritesStep as Step
-            d = O.sample_dsprites(rs, B)
-            extra, step_fn = (), O.step_dsprites
-        ours = Step(seed=seed, device=dev, pxy_state=O.dsprites_pxy_state(seed, colored=colored))
+        step_fn = O.step_colored if colored else O.step_dsprites
         return (lambda dt: O.build_dsprites(seed=seed, device=dev, dtype=dt, colored=colored),
-                lambda st, dt, after: step_fn(st, imgs, d, after_phase=after), ours,
-                lambda rec, after: ours(imgs, *extra, d["code_d"].to(dev), d["labels_d"].to(dev),
-                                        d["code_info"].to(dev), d["labels_info"].to(dev), record=rec,
-                                        after_phase=after), (0,))
+                lambda st, dt, after: step_fn(st, imgs, d, after_phase=after),
+                lambda ours, rec, after: ours(*args, record=rec, after_phase=after), (0,))
     if config == "mnist":
-        from eadgan_b200.steps.mnist import MnistStep
-        imgs, d = O.synth_mnist_images(B, seed).to(dev), O.sample_mnist(rs, B)
-        ours = MnistStep(seed=seed, device=dev, approximator_state=O.mnist_approximator_state(seed))
         return (lambda dt: O.build_mnist(seed=seed, device=dev, dtype=dt),
-                lambda st, dt, after: O.step_mnist(st, imgs, d, after_phase=after), ours,
-                lambda rec, after: ours(imgs, d["z"].to(dev), d["code"].to(dev), d["labels"].to(dev), record=rec,
-                                        after_phase=after), (0, 1))
+                lambda st, dt, after: O.step_mnist(st, imgs, d, after_phase=after),
+                lambda ours, rec, after: ours(*args, record=rec, after_phase=after), (0, 1))
     if config in ("pxy", "pxy_color"):
-        from eadgan_b200.steps.pxy import PxyStep
         colored = config == "pxy_color"
-        imgs, d = O.synth_dsprites_images(B, seed).to(dev), O.sample_pxy(rs, B, colored)
-        ours = PxyStep(seed=seed, device=dev, colored=colored)
         return (lambda dt: O.build_pxy(seed=seed, device=dev, dtype=dt, colored=colored),
-                lambda st, dt, after: O.step_pxy(st, imgs, d), ours,
-                lambda rec, after: ours(imgs, d["code"].to(dev), d["color"].to(dev) if colored else None,
-                                        record=rec), ())
+                lambda st, dt, after: O.step_pxy(st, imgs, d),
+                lambda ours, rec, after: ours(*args, record=rec), ())
     raise ValueError(config)
 
 
@@ -140,24 +161,96 @@ def net_states(step, config):
     return _state({k: getattr(step, k) for k in NETS[config]})
 
 
-def forced_step(config, dev, B, precision="bf16", seed=0, oracle_dtypes=(torch.float64,)):
-    """-> dict(forced=[oracle record per dtype in ``oracle_dtypes``], ours=our per-phase record, losses=our losses,
-    free=free oracle record (first dtype), flips=..., gates=..., step=our step object, codes=[our Encoder_pxy
-    outputs]).  Each forced record also carries ``state`` (its nets' state after the step) and, for the dSprites
-    configurations, ``codes`` (the oracle's own Encoder_pxy outputs on the forced gates).
+# the optimisers of each configuration's step, by attribute name (ours) == state key (oracle)
+OPTS = {"celeba": ("opt_G", "opt_D", "opt_info"), "dsprites": ("opt_D", "opt_info"), "colored": ("opt_D", "opt_info"),
+        "mnist": ("opt_G", "opt_D", "opt_info"), "pxy": ("opt_E",), "pxy_color": ("opt_E",)}
 
-    Runs on identical seeded inputs / weights: the free oracle (its post-phase states are the common starting point
-    of every later phase of every run), OUR step (gates logged), then the oracle with OUR gates -- and our
-    Encoder_pxy code -- forced, once per requested dtype (fp64 = the referee; fp32 = stock torch's own rounding
-    error on the same branch)."""
+
+def _member(holder, key):
+    """a network / optimiser of our step object (attribute) or of an oracle state (build_*: dict entry)"""
+    return holder[key] if isinstance(holder, dict) else getattr(holder, key)
+
+
+def opt_params(opt):
+    return [p for g in opt.param_groups for p in g["params"]]
+
+
+def training_state(step, config):
+    """-> {"nets": {net: state_dict}, "opts": {optimiser: [per parameter in param_groups order: None (no state yet)
+    or {"step": int, "exp_avg", "exp_avg_sq"}]}}: a copy of everything one training step hands to the next, taken from
+    our step object or from an oracle state (build_*)"""
+    opts = {}
+    for name in OPTS[config]:
+        opt = _member(step, name)
+        per = []
+        for p in opt_params(opt):
+            s = opt.state.get(p)
+            per.append({"step": int(s["step"]), "exp_avg": s["exp_avg"].detach().clone(),
+                        "exp_avg_sq": s["exp_avg_sq"].detach().clone()} if s else None)
+        opts[name] = per
+    return {"nets": _state({k: _member(step, k) for k in NETS[config]}), "opts": opts}
+
+
+def load_training_state(step, config, state):
+    """put ``state`` (training_state) into our step object or an oracle state (build_*), floating-point tensors cast to
+    the receiving parameters' dtype.  torch.optim.Adam keeps ``step`` as a tensor, our Adam as an int; a parameter
+    without state is left without state (it has not had a gradient yet: MNIST's E.noise_layer never gets one)."""
+    for key, sd in state["nets"].items():
+        net = _member(step, key)
+        net.load_state_dict(_cast(sd, next(net.parameters()).dtype))
+    for name, per in state["opts"].items():
+        opt = _member(step, name)
+        ps = opt_params(opt)
+        assert len(ps) == len(per), (name, len(ps), len(per))
+        for p, s in zip(ps, per):
+            opt.state.pop(p, None)
+            if s is None:
+                continue
+            assert s["exp_avg"].shape == s["exp_avg_sq"].shape == p.shape, (name, tuple(p.shape))
+            opt.state[p] = {"step": torch.tensor(float(s["step"])) if isinstance(opt, torch.optim.Adam) else s["step"],
+                            "exp_avg": s["exp_avg"].to(p.device, p.dtype).clone(memory_format=torch.contiguous_format),
+                            "exp_avg_sq": s["exp_avg_sq"].to(p.device, p.dtype).clone(
+                                memory_format=torch.contiguous_format)}
+
+
+def forced_step(config, dev, B, precision="bf16", seed=0, oracle_dtypes=(torch.float64,), start=None, ours=None,
+                data_seed=None):
+    """-> dict(forced=[oracle record per dtype in ``oracle_dtypes``], ours=our per-phase record, losses=our losses,
+    free=free oracle record (first dtype; None with ``start``), flips=..., gates=..., step=our step object,
+    codes=[our Encoder_pxy outputs]).  Each forced record also carries ``state`` (its nets' state after the step) and,
+    for the dSprites configurations, ``codes`` (the oracle's own Encoder_pxy outputs on the forced gates).
+
+    Runs on identical seeded inputs (batch ``data_seed``, default ``seed``) and weights: the free oracle (its
+    post-phase states are the common starting point of every later phase of every run), OUR step (gates logged), then
+    the oracle with OUR gates -- and our Encoder_pxy code -- forced, once per requested dtype (fp64 = the referee;
+    fp32 = stock torch's own rounding error on the same branch).
+
+    ``start`` (training_state): both runs begin from that training state instead of the seeded initial one, and no
+    phase is restarted.  Restarts exist because Adam's first update, at t = 1 with zero moments, is lr * sign(g):
+    a gradient element at rounding level of 0 moves its weight by a full step either way.  From t = 2 on the update
+    m^/(sqrt(v^)+eps) is a smooth function of the gradient, so the phases may run on as the step runs them.  (The
+    zero-gradient biases of the ZERO_GRAD maps are still noise-driven, but the train-mode BatchNorm right after each
+    removes their update exactly.)  ``ours``: a step object to run instead of a freshly seeded one -- with ``start``
+    it is NOT reloaded (``start`` must be its own training_state), so the bf16 packs, prefetched spectral-norm results
+    and frozen / trainable flags it carries over from its earlier steps are what this step runs on."""
     from eadgan_b200 import chain
     os.environ["EADGAN_PRECISION"] = precision
-    build, run_oracle, ours, run_ours, restarts = _setup(config, dev, B, seed)
+    build, run_oracle, run_ours, restarts = _setup(config, dev, B, seed, seed if data_seed is None else data_seed)
+    if ours is None:
+        ours = make_step(config, dev, seed)
+        if start is not None:
+            load_training_state(ours, config, start)
     keys = NETS[config]
     dt0 = oracle_dtypes[0]
 
-    free = run_oracle(build(dt0), dt0, None)
-    states = {i: free["phases"][i]["state_after"] for i in restarts}
+    def build_from(dt):
+        st = build(dt)
+        if start is not None:
+            load_training_state(st, config, start)
+        return st
+
+    free = None if start is not None else run_oracle(build(dt0), dt0, None)
+    states = {i: free["phases"][i]["state_after"] for i in restarts} if free is not None else {}
 
     def restart(nets, dt):
         def after_phase(i):
@@ -173,7 +266,7 @@ def forced_step(config, dev, B, precision="bf16", seed=0, oracle_dtypes=(torch.f
     rec = []
     chain.gate_log = []
     try:
-        losses = run_ours(rec, restart(our_nets, torch.float32))
+        losses = run_ours(ours, rec, restart(our_nets, torch.float32))
         log = chain.gate_log
     finally:
         chain.gate_log = None
@@ -186,7 +279,7 @@ def forced_step(config, dev, B, precision="bf16", seed=0, oracle_dtypes=(torch.f
 
     forced, flips, total = [], 0, 0
     for dt in oracle_dtypes:
-        st = build(dt)
+        st = build_from(dt)
         nets = {k: st[k] for k in keys}
         queues = {qn: list(ms) for qn, ms in masks.items()}
         gates = []

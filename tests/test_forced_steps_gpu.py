@@ -19,6 +19,8 @@ pytestmark = pytest.mark.gpu
 
 def _names(config, step):
     """-> (per-phase parameter names, zero-gradient sibling map) of a configuration's optimisers"""
+    if config == "celeba":
+        return U.grad_names(step), U.ZERO_GRAD
     if config in ("dsprites", "colored"):
         return U.dsprites_grad_names(step), U.DSPRITES_ZERO_GRAD
     if config == "mnist":
@@ -64,8 +66,9 @@ def _running(k):
     return "running" in k
 
 
-def _check(config, out, tol, stock=None):
-    """every bound of a forced-gate step; ``stock`` = stock torch fp32's forced record (fp32 mode) -> worst values"""
+def _check(config, out, tol, stock=None, sn_nets=("D", "E")):
+    """every bound of a forced-gate step; ``stock`` = stock torch fp32's forced record (fp32 mode); ``sn_nets``: the
+    networks whose spectral-norm u / v are compared with the oracle's -> worst values"""
     step, ref = out["step"], out["forced"][0]
     assert out["gates"] > 0 and out["flips"] <= 0.01 * out["gates"], (out["flips"], out["gates"])
     code_err = 0.0
@@ -90,7 +93,7 @@ def _check(config, out, tol, stock=None):
     assert not bad, bad
     # spectral-norm u / v depend on fp32 weights only (never on activations): 1e-5 in both precisions
     ours = gates.net_states(step, config)
-    sn = _buffers(ours, ref["state"], ("D", "E"), _sn)
+    sn = _buffers(ours, ref["state"], sn_nets, _sn)
     assert all(v <= 1e-5 for v in sn.values()), sn
     bn = _buffers(ours, ref["state"], ("G", "E"), _running)
     bn_bound = bounds(bn, stock and _buffers(stock["state"], ref["state"], ("G", "E"), _running))
