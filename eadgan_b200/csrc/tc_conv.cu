@@ -1452,32 +1452,211 @@ int map_matrix(CUtensorMap* m, const void* base, uint64_t rows, uint64_t cols, u
   return encode_map(m, base, 2, dims, st, box);
 }
 
+// ------------------------------------------------------------------------------------
+// host: launch plans, one per kernel family, of the descriptor, the SM count and the test hooks (no CUDA call)
+// ------------------------------------------------------------------------------------
+// Test hooks, read at every launch: EADGAN_TC_CG = 1 / 2 forces CTA pairs off / on where the family allows pairs;
+// EADGAN_TC_DGRADT = 0 (or empty) / 2: never / always the channel-major kernel where it applies (unset: -1, size rule).
+struct TestHooks { int cg, dgradt; };
+TestHooks read_hooks() {
+  const char* cg = getenv("EADGAN_TC_CG");
+  const char* dgradt = getenv("EADGAN_TC_DGRADT");
+  return {cg ? atoi(cg) : 0, dgradt ? atoi(dgradt) : -1};
+}
 
-// cudaFuncSetAttribute(MaxDynamicSharedMemorySize) applies PER DEVICE: remember which devices have been opted in
-// (bit d of an atomic mask; devices >= 64 simply set the attribute on every launch).  Safe from any thread
-// (backward runs on autograd's per-device worker threads).
-template <typename K>
-int opt_in_smem(K kernel, int bytes, std::atomic<uint64_t>& done) {
+bool pow2(int v) { return v > 0 && (v & (v - 1)) == 0; }
+
+// tile of `pixels` positions of a p x q grid: Tw = q, Th rows, Tb images; m_tiles tiles cover n images
+struct Tile { int Tw, Th, Tb, tiles_y, m_tiles; };
+bool pick_tile(int n, int p, int q, int pixels, Tile* t) {
+  if (!pow2(q) || !pow2(p) || q > pixels) return false;
+  t->Tw = q;
+  t->Th = pixels / q < p ? pixels / q : p;
+  t->Tb = pixels / (q * t->Th);
+  t->tiles_y = p / t->Th;
+  t->m_tiles = ((n + t->Tb - 1) / t->Tb) * t->tiles_y;
+  return true;
+}
+
+// tile configuration of one tc_conv_kernel launch: BLOCK_N, M tiles per CTA, cta_group (bn <= 0: no BLOCK_N fits)
+struct TileCfg { int bn, mt, cg; };
+
+// m_tiles x parities 128-row tiles of nch output channels.  `wide` launches may take BLOCK_N = 256, which halves the A
+// re-reads and the smem traffic per MAC (kept at 128 while the tile count is too small to fill the machine twice), and
+// cg = 2 (CTA pairs, see Cfg) when there are enough tiles to keep every pair busy for several tiles; the small / ragged
+// launches (dSprites 32..64-channel layers, dense and thin GEMMs) stay on the single-CTA path.
+TileCfg pick_cfg(int nch, int m_tiles, int parities, bool wide, int sms, int cg_hook) {
+  TileCfg t{-1, 1, 1};
+  if (wide && nch % 256 == 0 && (int64_t)m_tiles * parities * (nch / 256) >= 2 * sms) t.bn = 256;
+  else if (nch % 128 == 0) t.bn = 128;
+  else if (nch % 64 == 0) t.bn = 64;
+  else if (nch % 32 == 0) t.bn = 32;
+  if (t.bn <= 0) return t;
+  const int64_t tiles = (int64_t)m_tiles * parities * (nch / t.bn);
+  t.cg = (wide && t.bn >= 128 && m_tiles >= 2 && tiles >= 2 * sms) ? 2 : 1;
+  if (wide && t.bn >= 128 && (cg_hook == 1 || cg_hook == 2)) t.cg = cg_hook;
+  // two 128-row tiles per CTA tile (sharing every B load) when BLOCK_N <= 128 and there is enough work
+  t.mt = (t.bn <= 128 && tiles >= 4 * sms * t.cg) ? 2 : 1;
+  return t;
+}
+
+// the channel-major kernel (tc_dgradT_kernel, 128 channels x 256 pixels per tile) where it applies and the launch has
+// at least 8 tiles of 128 x 128 per SM
+bool use_channel_major(bool applies, int64_t tiles, int sms, int dgradt_hook) {
+  return applies && dgradt_hook != 0 && (dgradt_hook == 2 || tiles >= 8 * sms);
+}
+
+// plan of a tc fprop / tc dgrad / thin fprop launch: the 128-pixel tile, and the channel-major kernel or tc_conv_kernel
+// with cfg
+struct ConvPlan { Tile t; TileCfg cfg; bool channel_major; };
+
+int fprop_plan(const eadgan_tc_desc* d, int sms, TestHooks h, ConvPlan* pl) {
+  const int p = d->h / 2, q = d->w / 2;
+  EG_REQUIRE((2 * d->c) % 64 == 0, EADGAN_ERR_UNSUPPORTED, "tc_fprop: c=%d must be a multiple of 32", d->c);
+  EG_REQUIRE(pick_tile(d->n, p, q, 128, &pl->t), EADGAN_ERR_UNSUPPORTED,
+             "tc_fprop: output map %dx%d must be a power of two <= 128 wide", p, q);
+  pl->cfg = pick_cfg(d->k, pl->t.m_tiles, 1, true, sms, h.cg);
+  EG_REQUIRE(pl->cfg.bn > 0, EADGAN_ERR_UNSUPPORTED, "tc_fprop: k=%d must be a multiple of 32", d->k);
+  pl->channel_major = false;
+  return 0;
+}
+
+int dgrad_plan(const eadgan_tc_desc* d, int sms, TestHooks h, ConvPlan* pl) {
+  const int p = d->h / 2, q = d->w / 2;
+  // k = 32: the 64-channel TMA boxes run past the tensor and are zero-filled (half of each k block is idle)
+  EG_REQUIRE(d->k % 64 == 0 || d->k == 32, EADGAN_ERR_UNSUPPORTED, "tc_dgrad: k=%d must be 32 or a multiple of 64", d->k);
+  EG_REQUIRE(pick_tile(d->n, p, q, 128, &pl->t), EADGAN_ERR_UNSUPPORTED,
+             "tc_dgrad: small map %dx%d must be a power of two <= 128 wide", p, q);
+  pl->cfg = pick_cfg(d->c, pl->t.m_tiles, 4, true, sms, h.cg);
+  EG_REQUIRE(pl->cfg.bn > 0, EADGAN_ERR_UNSUPPORTED, "tc_dgrad: c=%d must be a multiple of 32", d->c);
+  // 128-channel outputs with a long pixel dimension.  The channel-major kernel shares TcParams: its conditions
+  // k % 64 == 0, c_real == c and no out_f32_nchw are what make eadgan_tc_dgrad's qblocks, n_store and out_f32_nchw right
+  // for it too.
+  const bool applies = d->c == 128 && d->k % 64 == 0 && !d->out_f32_nchw && (d->c_real <= 0 || d->c_real == d->c);
+  pl->channel_major = use_channel_major(applies, (int64_t)pl->t.m_tiles * 4, sms, h.dgradt);
+  return 0;
+}
+
+int thin_fprop_plan(const eadgan_tc_desc* d, int sms, TestHooks h, ConvPlan* pl) {
+  const int p = d->h / 2, q = d->w / 2;
+  EG_REQUIRE(pick_tile(d->n, p, q, 128, &pl->t), EADGAN_ERR_UNSUPPORTED,
+             "tc_thin_fprop: output map %dx%d must be a power of two <= 128 wide", p, q);
+  pl->cfg = pick_cfg(d->k, pl->t.m_tiles, 1, false, sms, h.cg);
+  EG_REQUIRE(pl->cfg.bn > 0, EADGAN_ERR_UNSUPPORTED, "tc_thin_fprop: k=%d must be a multiple of 32", d->k);
+  const bool applies = d->k % 128 == 0 && !d->out_f32_nchw;
+  pl->channel_major = use_channel_major(applies, (int64_t)pl->t.m_tiles * (d->k / 128), sms, h.dgradt);
+  return 0;
+}
+
+// plan of a tc wgrad / thin wgrad launch
+struct WgPlan {
+  WgParams P;        // all but P.partial; P.k = k padded to 128: partial rows have stride P.k, rows past k stay in bounds
+  int bn, cg;
+  size_t ws_bytes;   // fp32 partial sums [splits][P.k][Ktot]
+};
+
+// 64-pixel steps over the p x q small map of d
+int wgrad_tile(const eadgan_tc_desc* d, const char* who, WgParams* P) {
+  const int p = d->h / 2, q = d->w / 2;
+  Tile t;
+  EG_REQUIRE(pick_tile(d->n, p, q, 64, &t), EADGAN_ERR_UNSUPPORTED, "%s: small map %dx%d must be a power of two <= 64 wide",
+             who, p, q);
+  *P = WgParams{};
+  P->n = d->n; P->p = p; P->q = q; P->Tw = t.Tw; P->Th = t.Th; P->Tb = t.Tb; P->tiles_y = t.tiles_y;
+  P->steps_total = t.m_tiles;
+  P->k = ((d->k + 127) / 128) * 128;
+  return 0;
+}
+
+// the pixel reduction in splits of whole steps (s at most), the persistent item space and the workspace
+void wgrad_split(WgPlan* pl, int s, int bn, int cg) {
+  WgParams& P = pl->P;
+  P.steps_per_split = (P.steps_total + s - 1) / s;
+  P.splits = (P.steps_total + P.steps_per_split - 1) / P.steps_per_split;
+  P.kk_tiles = P.Ktot / bn; P.ko_tiles = P.k / (128 * cg);
+  pl->bn = bn; pl->cg = cg;
+  pl->ws_bytes = (size_t)P.splits * P.k * (size_t)P.Ktot * sizeof(float);
+}
+
+int wgrad_plan(const eadgan_tc_desc* d, int sms, TestHooks h, WgPlan* pl) {
+  // dy channel boxes past k are zero-filled by TMA and the matching partial rows are never read
+  EG_REQUIRE(d->k % 32 == 0, EADGAN_ERR_UNSUPPORTED, "tc_wgrad: k=%d must be a multiple of 32", d->k);
+  EG_REQUIRE((2 * d->c) % 64 == 0, EADGAN_ERR_UNSUPPORTED, "tc_wgrad: c=%d must be a multiple of 32", d->c);
+  WgParams& P = pl->P;
+  if (int e = wgrad_tile(d, "tc_wgrad", &P)) return e;
+  P.c = d->c; P.qblocks = 2 * d->c / 64; P.Ktot = 16 * d->c;
+  const int bn = (P.Ktot % 256 == 0) ? 256 : (P.Ktot % 128 == 0 ? 128 : 64);
+  // CTA pairs (256 ko rows per tile, see WgCfg) when there are whole 256-row tiles and a long reduction
+  const bool pairs = bn == 256 && d->k % 256 == 0;
+  int cg = (pairs && P.steps_total >= 256) ? 2 : 1;
+  if (pairs && (h.cg == 1 || h.cg == 2)) cg = h.cg;
+  const int tiles = (P.Ktot / bn) * (P.k / 128) / cg;
+  // split of the pixel reduction: one CTA per (tile, split) and one CTA per SM at a time, so the kernel runs in
+  // waves of sm_count CTAs.  Pick the split count minimising  waves * steps_per_split  (tensor time, a 64-pixel
+  // step of a 128 x bn tile is bn*2 clocks) plus the fp32 partial-sum traffic (written once, read once).
+  const int units = sms / cg;   // concurrently running CTAs (CTA pairs)
+  const int max_s = (P.steps_total + 7) / 8;
+  double best = 1e300;
+  int best_s = 1;
+  for (int s = 1; s <= max_s && s <= 4 * units; ++s) {
+    const int sps = (P.steps_total + s - 1) / s;
+    const int s_eff = (P.steps_total + sps - 1) / sps;
+    const int64_t ctas = (int64_t)tiles * s_eff;
+    const int64_t waves = (ctas + units - 1) / units;
+    const double t_mma = (double)waves * (sps * bn * 2.0 + 1500.0) / 1.9e9 / 0.9;  // + pipeline refill per item
+    const double t_part = (double)s_eff * P.k * (double)P.Ktot * 8.0 / 6.0e12;
+    if (t_mma + t_part < best) { best = t_mma + t_part; best_s = s_eff; }
+  }
+  wgrad_split(pl, best_s, bn, cg);
+  return 0;
+}
+
+int thin_wgrad_plan(const eadgan_tc_desc* d, int sms, WgPlan* pl) {
+  EG_REQUIRE(d->k % 32 == 0, EADGAN_ERR_UNSUPPORTED, "tc_thin_wgrad: k=%d must be a multiple of 32", d->k);
+  WgParams& P = pl->P;
+  if (int e = wgrad_tile(d, "tc_thin_wgrad", &P)) return e;
+  P.c = 4; P.thin = 1; P.qblocks = 1; P.Ktot = 64;
+  // the only parallelism is the split of the pixel reduction: one CTA per SM (per 128-row ko tile)
+  int s = sms / (P.k / 128);
+  const int max_s = (P.steps_total + 7) / 8;
+  if (s > max_s) s = max_s;
+  if (s < 1) s = 1;
+  wgrad_split(pl, s, 64, 1);
+  return 0;
+}
+
+// Persistent launch of `total` work items: every CTA (CTA pair when CG = 2) runs the same number of items (+-1), at
+// most one CTA per SM.  cudaFuncSetAttribute(MaxDynamicSharedMemorySize) applies PER DEVICE: each kernel instance
+// remembers which devices it has opted in (bit d of an atomic mask; devices >= 64 simply set the attribute on every
+// launch).  Safe from any thread (backward runs on autograd's per-device worker threads).
+template <auto Kernel, int CG, typename... Args>
+int launch_persistent(const char* name, int total, int threads, int smem, cudaStream_t st, const Args&... args) {
+  static std::atomic<uint64_t> opted{0};
   int dev = 0;
   EG_CUDA(cudaGetDevice(&dev));
   const uint64_t bit = dev < 64 ? (1ull << dev) : 0ull;
-  if (bit && (done.load(std::memory_order_acquire) & bit)) return 0;
-  EG_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
-  if (bit) done.fetch_or(bit, std::memory_order_release);
+  if (!(opted.load(std::memory_order_acquire) & bit)) {
+    EG_CUDA(cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    opted.fetch_or(bit, std::memory_order_release);
+  }
+  const int units = eg_sm_count() / CG;
+  const int waves = (total + units - 1) / units;
+  cudaLaunchConfig_t cfg{};
+  cfg.gridDim = dim3(((total + waves - 1) / waves) * CG); cfg.blockDim = dim3(threads); cfg.dynamicSmemBytes = smem;
+  cfg.stream = st;
+  cudaLaunchAttribute attr[1];
+  attr[0].id = cudaLaunchAttributeClusterDimension;
+  attr[0].val.clusterDim.x = CG; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
+  cfg.attrs = attr; cfg.numAttrs = CG == 2 ? 1 : 0;
+  EG_CUDA(cudaLaunchKernelEx(&cfg, Kernel, args...));
+  EG_LAUNCH_CHECK(name);
   return 0;
 }
 
 template <int SPEC>
 int launch_channel_major_t(const CUtensorMap& mx, const CUtensorMap& mw, const TcParams& P, cudaStream_t st) {
-  static std::atomic<uint64_t> opted{0};
-  if (int e = opt_in_smem(tc_dgradT_kernel<SPEC>, DgTCfg::SMEM, opted)) return e;
-  const int total = P.parities * P.m_tiles * P.n_tiles;
-  const int units = eg_sm_count();
-  const int waves = (total + units - 1) / units;
-  const int grid = (total + waves - 1) / waves;
-  tc_dgradT_kernel<SPEC><<<grid, 64 + DgTCfg::EW * 32, DgTCfg::SMEM, st>>>(mx, mw, P);
-  EG_LAUNCH_CHECK("tc_dgradT_kernel");
-  return 0;
+  return launch_persistent<tc_dgradT_kernel<SPEC>, 1>("tc_dgradT_kernel", P.parities * P.m_tiles * P.n_tiles,
+                                                       64 + DgTCfg::EW * 32, DgTCfg::SMEM, st, mx, mw, P);
 }
 
 int launch_channel_major(const CUtensorMap& mx, const CUtensorMap& mw, TcParams P, cudaStream_t st) {
@@ -1502,58 +1681,10 @@ int launch_channel_major(const CUtensorMap& mx, const CUtensorMap& mw, TcParams 
   return launch_channel_major_t<0>(mx, mw, P, st);
 }
 
-bool pow2(int v) { return v > 0 && (v & (v - 1)) == 0; }
-
-// tile of `pixels` positions of a p x q grid: Tw = q, Th rows, Tb images
-int pick_tile(int p, int q, int pixels, int* Tw, int* Th, int* Tb) {
-  if (!pow2(q) || !pow2(p) || q > pixels) return -1;
-  *Tw = q;
-  int th = pixels / q;
-  if (th > p) th = p;
-  *Th = th;
-  *Tb = pixels / (q * th);
-  return 0;
-}
-
 template <int BN, int MT, int CG>
 int launch_conv(const CUtensorMap& ma, const CUtensorMap& mb, const TcParams& P, cudaStream_t st) {
-  static std::atomic<uint64_t> opted{0};
-  if (int e = opt_in_smem(tc_conv_kernel<BN, MT, CG>, Cfg<BN, MT, CG>::SMEM, opted)) return e;
-  // persistent grid: every CTA (CTA pair) runs the same number of tiles (+-1), at most one CTA per SM
-  const int total = P.parities * P.m_tiles * P.n_tiles;
-  const int units = eg_sm_count() / CG;
-  const int waves = (total + units - 1) / units;
-  const int grid = ((total + waves - 1) / waves) * CG;
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3(grid); cfg.blockDim = dim3(320); cfg.dynamicSmemBytes = Cfg<BN, MT, CG>::SMEM; cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = CG; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr; cfg.numAttrs = CG == 2 ? 1 : 0;
-  EG_CUDA(cudaLaunchKernelEx(&cfg, tc_conv_kernel<BN, MT, CG>, ma, mb, P));
-  EG_LAUNCH_CHECK("tc_conv_kernel");
-  return 0;
-}
-
-// tile configuration of one launch: BLOCK_N, M tiles per CTA, cta_group
-struct TileCfg { int bn, mt, cg; };
-
-int pick_bn_tiles(int nch, int m_tiles_x_par);
-
-// cg = 2 (CTA pairs, see Cfg) for the layers with enough tiles to keep every pair busy for several tiles; the small /
-// ragged launches (dSprites 32..64-channel layers, dense and thin GEMMs) stay on the single-CTA path.
-TileCfg pick_cfg(int nch, int m_tiles, int parities, bool allow_pair, int force_bn = 0) {
-  TileCfg t;
-  t.bn = force_bn ? force_bn : pick_bn_tiles(nch, m_tiles * parities);
-  if (t.bn <= 0) return t;
-  const int sms = eg_sm_count();
-  const int64_t tiles = (int64_t)m_tiles * parities * (nch / t.bn);
-  t.cg = (allow_pair && t.bn >= 128 && m_tiles >= 2 && tiles >= 2 * sms) ? 2 : 1;
-  // test hook: force CTA pairs on (2) / off (1), so that small, ragged shapes exercise the pair protocol
-  if (const char* e = getenv("EADGAN_TC_CG")) { if (allow_pair && t.bn >= 128 && (atoi(e) == 1 || atoi(e) == 2)) t.cg = atoi(e); }
-  // two 128-row tiles per CTA tile (sharing every B load) when BLOCK_N <= 128 and there is enough work
-  t.mt = (t.bn <= 128 && tiles >= 4 * sms * t.cg) ? 2 : 1;
-  return t;
+  return launch_persistent<tc_conv_kernel<BN, MT, CG>, CG>("tc_conv_kernel", P.parities * P.m_tiles * P.n_tiles, 320,
+                                                            Cfg<BN, MT, CG>::SMEM, st, ma, mb, P);
 }
 
 int dispatch_conv(const TileCfg& t, const CUtensorMap& ma, const CUtensorMap& mb, TcParams& P, int m_tiles, int n_total,
@@ -1582,21 +1713,48 @@ int dispatch_conv(const TileCfg& t, const CUtensorMap& ma, const CUtensorMap& mb
                           bn, mt, t.cg);
 }
 
-// BLOCK_N: 256 halves the A re-reads and the smem traffic per MAC; keep 128 while the tile count is too
-// small to fill the machine twice
-int pick_bn_tiles(int nch, int m_tiles_x_par) {
-  if (nch % 256 == 0 && (int64_t)m_tiles_x_par * (nch / 256) >= 2 * eg_sm_count()) return 256;
-  if (nch % 128 == 0) return 128;
-  if (nch % 64 == 0) return 64;
-  if (nch % 32 == 0) return 32;
-  return -1;
+// TcParams of a tc fprop / tc dgrad / thin fprop launch: the plan's tile of d's map, and d's epilogue (activation,
+// output format, fused mask and statistics) with its bias, output, mask, statistics and sigma pointers
+int conv_params(TcParams* P, int mode, const eadgan_tc_desc* d, const Tile& t, const float* bias, void* out,
+                const void* mask, double* stats, const float* sigma, const char* who) {
+  P->mode = mode; P->n = d->n; P->p = d->h / 2; P->q = d->w / 2;
+  P->Tw = t.Tw; P->Th = t.Th; P->Tb = t.Tb; P->tiles_y = t.tiles_y;
+  P->act = d->act; P->slope = d->slope; P->out_f32_nchw = d->out_f32_nchw; P->want_stats = d->want_stats;
+  P->mask_mode = d->mask_mode; P->bias = bias; P->out = out; P->mask = (const __nv_bfloat16*)mask; P->stats = stats;
+  P->sigma = sigma;
+  EG_REQUIRE(!P->mask_mode || mask, EADGAN_ERR_INVALID, "%s: mask_mode without mask", who);
+  EG_REQUIRE(!P->want_stats || stats, EADGAN_ERR_INVALID, "%s: want_stats without stats", who);
+  return 0;
 }
 
-int pick_bn(int nch) {
-  if (nch % 128 == 0) return 128;
-  if (nch % 64 == 0) return 64;
-  if (nch % 32 == 0) return 32;
-  return -1;
+// the planned kernel over n_total output channels x parities, with the packed weight [w_rows][w_cols] as B operand
+int launch_conv_plan(const ConvPlan& pl, const CUtensorMap& ma, const void* w, uint64_t w_rows, uint64_t w_cols,
+                     TcParams& P, int n_total, int parities, cudaStream_t st) {
+  CUtensorMap mb;
+  if (pl.channel_major) {   // two 128-pixel M tiles per tile
+    if (int e = map_matrix(&mb, w, w_rows, w_cols, 128)) return e;
+    P.m_tiles = (pl.t.m_tiles + 1) / 2; P.n_tiles = n_total / 128; P.parities = parities;
+    return launch_channel_major(ma, mb, P, st);
+  }
+  if (int e = map_matrix(&mb, w, w_rows, w_cols, pl.cfg.bn / pl.cfg.cg)) return e;
+  return dispatch_conv(pl.cfg, ma, mb, P, pl.t.m_tiles, n_total, parities, st);
+}
+
+template <int BN, int CG>
+int launch_wgrad(const CUtensorMap& mdy, const CUtensorMap& mx, const WgParams& P, cudaStream_t st) {
+  return launch_persistent<tc_wgrad_kernel<BN, CG>, CG>("tc_wgrad_kernel", P.kk_tiles * P.ko_tiles * P.splits, 192,
+                                                         WgCfg<BN, CG>::SMEM, st, mdy, mx, P);
+}
+
+int dispatch_wgrad(const WgPlan& pl, const CUtensorMap& mdy, const CUtensorMap& mx, cudaStream_t st) {
+  switch (pl.bn * 10 + pl.cg) {
+    case 641: return launch_wgrad<64, 1>(mdy, mx, pl.P, st);
+    case 1281: return launch_wgrad<128, 1>(mdy, mx, pl.P, st);
+    case 2562: return launch_wgrad<256, 2>(mdy, mx, pl.P, st);
+    case 2561: return launch_wgrad<256, 1>(mdy, mx, pl.P, st);
+  }
+  return eadgan_set_error(EADGAN_ERR_UNSUPPORTED, "tc wgrad: unsupported tile configuration BLOCK_N %d, cta_group %d",
+                          pl.bn, pl.cg);
 }
 
 int check_tc(const eadgan_tc_desc* d, const char* who) {
@@ -1632,173 +1790,58 @@ extern "C" int eadgan_tc_fprop(const eadgan_tc_desc* d, const void* x_pad, const
                                void* y, const void* mask, double* stats, const float* sigma, void* stream) {
   if (int e = check_tc(d, "tc_fprop")) return e;
   EG_REQUIRE(x_pad && w_packed && y, EADGAN_ERR_INVALID, "tc_fprop: NULL pointer");
-  const int p = d->h / 2, q = d->w / 2;
-  EG_REQUIRE((2 * d->c) % 64 == 0, EADGAN_ERR_UNSUPPORTED, "tc_fprop: c=%d must be a multiple of 32", d->c);
+  ConvPlan pl;
+  if (int e = fprop_plan(d, eg_sm_count(), read_hooks(), &pl)) return e;
   TcParams P{};
-  P.mode = MODE_FPROP; P.n = d->n; P.p = p; P.q = q;
-  EG_REQUIRE(pick_tile(p, q, 128, &P.Tw, &P.Th, &P.Tb) == 0, EADGAN_ERR_UNSUPPORTED,
-             "tc_fprop: output map %dx%d must be a power of two <= 128 wide", p, q);
-  const int m_tiles = ((d->n + P.Tb - 1) / P.Tb) * (p / P.Th);
-  const TileCfg tcfg = pick_cfg(d->k, m_tiles, 1, true);
-  const int bn = tcfg.bn;
-  EG_REQUIRE(bn > 0, EADGAN_ERR_UNSUPPORTED, "tc_fprop: k=%d must be a multiple of 32", d->k);
-  P.tiles_y = p / P.Th; P.N_total = d->k; P.K_ch = d->c; P.qblocks = 2 * d->c / 64; P.nkb = 8 * P.qblocks;
-  P.act = d->act; P.slope = d->slope; P.out_f32_nchw = d->out_f32_nchw; P.want_stats = d->want_stats;
-  P.mask_mode = d->mask_mode; P.OH = p; P.OW = q; P.bias = bias; P.out = y;
-  P.mask = (const __nv_bfloat16*)mask; P.stats = stats; P.n_store = d->k; P.stat_channels = d->k; P.sigma = sigma;
-  EG_REQUIRE(!P.mask_mode || mask, EADGAN_ERR_INVALID, "tc_fprop: mask_mode without mask");
-  EG_REQUIRE(!P.want_stats || stats, EADGAN_ERR_INVALID, "tc_fprop: want_stats without stats");
-  CUtensorMap ma, mb;
+  P.N_total = d->k; P.K_ch = d->c; P.qblocks = 2 * d->c / 64; P.nkb = 8 * P.qblocks;
+  P.OH = d->h / 2; P.OW = d->w / 2; P.n_store = d->k; P.stat_channels = d->k;
+  if (int e = conv_params(&P, MODE_FPROP, d, pl.t, bias, y, mask, stats, sigma, "tc_fprop")) return e;
+  CUtensorMap ma;
   if (int e = map_big_s2d(&ma, x_pad, d->n, d->c, d->h, d->w, P.Tw, P.Th, P.Tb)) return e;
-  if (int e = map_matrix(&mb, w_packed, d->k, (uint64_t)16 * d->c, bn / tcfg.cg)) return e;
-  return dispatch_conv(tcfg, ma, mb, P, m_tiles, d->k, 1, (cudaStream_t)stream);
+  return launch_conv_plan(pl, ma, w_packed, d->k, (uint64_t)16 * d->c, P, d->k, 1, (cudaStream_t)stream);
 }
 
 extern "C" int eadgan_tc_dgrad(const eadgan_tc_desc* d, const void* dy_pad, const void* w_packed, const float* bias,
                                void* dx, const void* mask, double* stats, const float* sigma, void* stream) {
   if (int e = check_tc(d, "tc_dgrad")) return e;
   EG_REQUIRE(dy_pad && w_packed && dx, EADGAN_ERR_INVALID, "tc_dgrad: NULL pointer");
-  const int p = d->h / 2, q = d->w / 2;
-  // k = 32: the 64-channel TMA boxes run past the tensor and are zero-filled (half of each k block is idle)
-  EG_REQUIRE(d->k % 64 == 0 || d->k == 32, EADGAN_ERR_UNSUPPORTED, "tc_dgrad: k=%d must be 32 or a multiple of 64", d->k);
+  ConvPlan pl;
+  if (int e = dgrad_plan(d, eg_sm_count(), read_hooks(), &pl)) return e;
   TcParams P{};
-  P.mode = MODE_DGRAD; P.n = d->n; P.p = p; P.q = q;
-  EG_REQUIRE(pick_tile(p, q, 128, &P.Tw, &P.Th, &P.Tb) == 0, EADGAN_ERR_UNSUPPORTED,
-             "tc_dgrad: small map %dx%d must be a power of two <= 128 wide", p, q);
-  const int m_tiles = ((d->n + P.Tb - 1) / P.Tb) * (p / P.Th);
-  const TileCfg tcfg = pick_cfg(d->c, m_tiles, 4, true);
-  const int bn = tcfg.bn;
-  EG_REQUIRE(bn > 0, EADGAN_ERR_UNSUPPORTED, "tc_dgrad: c=%d must be a multiple of 32", d->c);
-  P.tiles_y = p / P.Th; P.N_total = d->c; P.K_ch = d->k; P.qblocks = (d->k + 63) / 64; P.nkb = 4 * P.qblocks;
-  P.act = d->act; P.slope = d->slope; P.out_f32_nchw = d->out_f32_nchw; P.want_stats = d->want_stats;
-  P.mask_mode = d->mask_mode; P.OH = d->h; P.OW = d->w; P.bias = bias; P.out = dx;
-  P.mask = (const __nv_bfloat16*)mask; P.stats = stats; P.sigma = sigma;
+  P.N_total = d->c; P.K_ch = d->k; P.qblocks = (d->k + 63) / 64; P.nkb = 4 * P.qblocks;
+  P.OH = d->h; P.OW = d->w;
   P.n_store = (d->c_real > 0 && d->c_real < d->c) ? d->c_real : d->c;
   P.stat_channels = P.n_store;
   EG_REQUIRE(P.n_store == d->c || d->out_f32_nchw, EADGAN_ERR_UNSUPPORTED,
              "tc_dgrad: zero-padded output channels (c_real < c) need out_f32_nchw");
-  EG_REQUIRE(!P.mask_mode || mask, EADGAN_ERR_INVALID, "tc_dgrad: mask_mode without mask");
-  EG_REQUIRE(!P.want_stats || stats, EADGAN_ERR_INVALID, "tc_dgrad: want_stats without stats");
-  CUtensorMap ma, mb;
-  if (int e = map_small(&ma, dy_pad, d->n, d->k, p, q, P.Tw, P.Th, P.Tb)) return e;
-  // 128-channel outputs with a long pixel dimension: the transposed kernel (see tc_dgradT_kernel), 128 channels x 256
-  // pixels per tile.  It shares P: its conditions k % 64 == 0, c_real == c and no out_f32_nchw are what make
-  // qblocks, n_store and out_f32_nchw above right for it too.
-  bool transposed = d->c == 128 && d->k % 64 == 0 && !d->out_f32_nchw && (d->c_real <= 0 || d->c_real == d->c);
-  bool enough = (int64_t)m_tiles * 4 >= 8 * eg_sm_count();
-  // test hook: 0 / 2 = never / always use the transposed kernel where it applies
-  if (const char* e = getenv("EADGAN_TC_DGRADT")) { if (atoi(e) == 0) transposed = false; else if (atoi(e) == 2) enough = true; }
-  if (transposed && enough) {
-    P.m_tiles = (m_tiles + 1) / 2; P.n_tiles = d->c / 128; P.parities = 4;
-    if (int e = map_matrix(&mb, w_packed, (uint64_t)4 * d->c, (uint64_t)4 * d->k, 128)) return e;
-    return launch_channel_major(ma, mb, P, (cudaStream_t)stream);
-  }
-  if (int e = map_matrix(&mb, w_packed, (uint64_t)4 * d->c, (uint64_t)4 * d->k, bn / tcfg.cg)) return e;
-  return dispatch_conv(tcfg, ma, mb, P, m_tiles, d->c, 4, (cudaStream_t)stream);
+  if (int e = conv_params(&P, MODE_DGRAD, d, pl.t, bias, dx, mask, stats, sigma, "tc_dgrad")) return e;
+  CUtensorMap ma;
+  if (int e = map_small(&ma, dy_pad, d->n, d->k, P.p, P.q, P.Tw, P.Th, P.Tb)) return e;
+  return launch_conv_plan(pl, ma, w_packed, (uint64_t)4 * d->c, (uint64_t)4 * d->k, P, d->c, 4, (cudaStream_t)stream);
 }
-
-namespace {
-int wgrad_plan(const eadgan_tc_desc* d, WgParams* P, int* bn, int* splits, int* cg) {
-  const int p = d->h / 2, q = d->w / 2;
-  // dy channel boxes past k are zero-filled by TMA and the matching partial rows are never read
-  EG_REQUIRE(d->k % 32 == 0, EADGAN_ERR_UNSUPPORTED, "tc_wgrad: k=%d must be a multiple of 32", d->k);
-  EG_REQUIRE((2 * d->c) % 64 == 0, EADGAN_ERR_UNSUPPORTED, "tc_wgrad: c=%d must be a multiple of 32", d->c);
-  P->n = d->n; P->p = p; P->q = q; P->k = d->k; P->c = d->c;
-  EG_REQUIRE(pick_tile(p, q, 64, &P->Tw, &P->Th, &P->Tb) == 0, EADGAN_ERR_UNSUPPORTED,
-             "tc_wgrad: small map %dx%d must be a power of two <= 64 wide", p, q);
-  P->tiles_y = p / P->Th;
-  P->qblocks = 2 * d->c / 64;
-  P->Ktot = 16 * d->c;
-  P->steps_total = ((d->n + P->Tb - 1) / P->Tb) * P->tiles_y;
-  *bn = (P->Ktot % 256 == 0) ? 256 : (P->Ktot % 128 == 0 ? 128 : 64);
-  // CTA pairs (256 ko rows per tile, see WgCfg) when there are whole 256-row tiles and a long reduction
-  *cg = (*bn == 256 && d->k % 256 == 0 && P->steps_total >= 256) ? 2 : 1;
-  // test hook: force CTA pairs on (2) / off (1), as in pick_cfg
-  if (const char* e = getenv("EADGAN_TC_CG")) { if (*bn == 256 && d->k % 256 == 0 && (atoi(e) == 1 || atoi(e) == 2)) *cg = atoi(e); }
-  const int tiles = (P->Ktot / *bn) * ((d->k + 127) / 128) / *cg;
-  // split of the pixel reduction: one CTA per (tile, split) and one CTA per SM at a time, so the kernel runs in
-  // waves of sm_count CTAs.  Pick the split count minimising  waves * steps_per_split  (tensor time, a 64-pixel
-  // step of a 128 x bn tile is bn*2 clocks) plus the fp32 partial-sum traffic (written once, read once).
-  const int sms = eg_sm_count() / *cg;   // concurrently running CTAs (CTA pairs)
-  const int max_s = (P->steps_total + 7) / 8;
-  const int k_pad = ((d->k + 127) / 128) * 128;
-  double best = 1e300;
-  int best_s = 1;
-  for (int s = 1; s <= max_s && s <= 4 * sms; ++s) {
-    const int sps = (P->steps_total + s - 1) / s;
-    const int s_eff = (P->steps_total + sps - 1) / sps;
-    const int64_t ctas = (int64_t)tiles * s_eff;
-    const int64_t waves = (ctas + sms - 1) / sms;
-    const double t_mma = (double)waves * (sps * (*bn) * 2.0 + 1500.0) / 1.9e9 / 0.9;  // + pipeline refill per item
-    const double t_part = (double)s_eff * k_pad * (double)P->Ktot * 8.0 / 6.0e12;
-    if (t_mma + t_part < best) { best = t_mma + t_part; best_s = s_eff; }
-  }
-  P->steps_per_split = (P->steps_total + best_s - 1) / best_s;
-  *splits = (P->steps_total + P->steps_per_split - 1) / P->steps_per_split;
-  return 0;
-}
-
-template <int BN, int CG = 1>
-int launch_wgrad(const CUtensorMap& mdy, const CUtensorMap& mx, const WgParams& P, dim3 grid, cudaStream_t st) {
-  static std::atomic<uint64_t> opted{0};
-  if (int e = opt_in_smem(tc_wgrad_kernel<BN, CG>, WgCfg<BN, CG>::SMEM, opted)) return e;
-  // `grid` is the logical item space (kk tiles, ko tiles, splits); the launch is one CTA per SM at most, every
-  // CTA running the same number of items (+-1)
-  WgParams Q = P;
-  Q.kk_tiles = (int)grid.x; Q.ko_tiles = (int)grid.y; Q.splits = (int)grid.z;
-  const int total = Q.kk_tiles * Q.ko_tiles * Q.splits;
-  const int units = eg_sm_count() / CG;
-  const int waves = (total + units - 1) / units;
-  const int ctas = ((total + waves - 1) / waves) * CG;
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3(ctas); cfg.blockDim = dim3(192); cfg.dynamicSmemBytes = WgCfg<BN, CG>::SMEM; cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = CG; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr; cfg.numAttrs = CG == 2 ? 1 : 0;
-  EG_CUDA(cudaLaunchKernelEx(&cfg, tc_wgrad_kernel<BN, CG>, mdy, mx, Q));
-  EG_LAUNCH_CHECK("tc_wgrad_kernel");
-  return 0;
-}
-}  // namespace
 
 extern "C" size_t eadgan_tc_workspace_bytes(const eadgan_tc_desc* d, int direction) {
-  if (direction != 2 || !d) return 0;
-  WgParams P{};
-  int bn = 0, splits = 0, cg = 1;
-  if (wgrad_plan(d, &P, &bn, &splits, &cg) != 0) return 0;
-  const int k_pad = ((d->k + 127) / 128) * 128;
-  return (size_t)splits * k_pad * (size_t)P.Ktot * sizeof(float);
+  WgPlan pl;
+  if (direction != 2 || !d || wgrad_plan(d, eg_sm_count(), read_hooks(), &pl) != 0) return 0;
+  return pl.ws_bytes;
 }
 
 extern "C" int eadgan_tc_wgrad(const eadgan_tc_desc* d, const void* x_pad, const void* dy_pad, float* dw,
                                void* workspace, size_t ws_bytes, void* stream) {
   if (int e = check_tc(d, "tc_wgrad")) return e;
   EG_REQUIRE(x_pad && dy_pad && dw && workspace, EADGAN_ERR_INVALID, "tc_wgrad: NULL pointer");
-  WgParams P{};
-  int bn = 0, splits = 0, cg = 1;
-  if (int e = wgrad_plan(d, &P, &bn, &splits, &cg)) return e;
-  const int k_pad = ((d->k + 127) / 128) * 128;
-  const size_t need = (size_t)splits * k_pad * (size_t)P.Ktot * sizeof(float);
-  EG_REQUIRE(ws_bytes >= need, EADGAN_ERR_WORKSPACE, "tc_wgrad: workspace %zu < %zu bytes", ws_bytes, need);
+  WgPlan pl;
+  if (int e = wgrad_plan(d, eg_sm_count(), read_hooks(), &pl)) return e;
+  EG_REQUIRE(ws_bytes >= pl.ws_bytes, EADGAN_ERR_WORKSPACE, "tc_wgrad: workspace %zu < %zu bytes", ws_bytes, pl.ws_bytes);
+  WgParams& P = pl.P;
   P.partial = (float*)workspace;
-  // partial rows are indexed with stride P.k: use the padded k so out-of-range rows stay in bounds
-  WgParams PK = P;
-  PK.k = k_pad;
   CUtensorMap mdy, mx;
   if (int e = map_small(&mdy, dy_pad, d->n, d->k, P.p, P.q, P.Tw, P.Th, P.Tb)) return e;
   if (int e = map_big_s2d(&mx, x_pad, d->n, d->c, d->h, d->w, P.Tw, P.Th, P.Tb)) return e;
-  dim3 grid(P.Ktot / bn, k_pad / (128 * cg), splits);
   cudaStream_t st = (cudaStream_t)stream;
-  int rc;
-  switch (bn) {
-    case 64: rc = launch_wgrad<64>(mdy, mx, PK, grid, st); break;
-    case 128: rc = launch_wgrad<128>(mdy, mx, PK, grid, st); break;
-    default: rc = cg == 2 ? launch_wgrad<256, 2>(mdy, mx, PK, grid, st) : launch_wgrad<256>(mdy, mx, PK, grid, st); break;
-  }
-  if (rc) return rc;
+  if (int e = dispatch_wgrad(pl, mdy, mx, st)) return e;
   const int c_real = (d->c_real > 0 && d->c_real < d->c) ? d->c_real : d->c;
-  wgrad_reduce_kernel<<<dim3((d->c + 63) / 64, d->k), 256, 0, st>>>(P.partial, splits, k_pad, d->c, c_real, dw);
+  wgrad_reduce_kernel<<<dim3((d->c + 63) / 64, d->k), 256, 0, st>>>(P.partial, P.splits, P.k, d->c, c_real, dw);
   EG_LAUNCH_CHECK("wgrad_reduce_kernel");
   return 0;
 }
@@ -1807,7 +1850,7 @@ extern "C" int eadgan_tc_gemm(const void* a_bf16, const void* b_bf16, float* c_f
                               void* stream) {
   EG_REQUIRE(a_bf16 && b_bf16 && c_f32 && m > 0 && n > 0 && kk > 0, EADGAN_ERR_INVALID, "tc_gemm: bad arguments");
   EG_REQUIRE(kk % 64 == 0, EADGAN_ERR_UNSUPPORTED, "tc_gemm: K=%d must be a multiple of 64", kk);
-  const TileCfg tcfg = pick_cfg(n, (m + 127) / 128, 1, true);
+  const TileCfg tcfg = pick_cfg(n, (m + 127) / 128, 1, true, eg_sm_count(), read_hooks().cg);
   const int bn = tcfg.bn;
   EG_REQUIRE(bn > 0, EADGAN_ERR_UNSUPPORTED, "tc_gemm: N=%d must be a multiple of 32", n);
   TcParams P{};
@@ -1873,8 +1916,8 @@ extern "C" int eadgan_tc_dense_gather(const void* y_pad, const void* w_rows, con
   CUtensorMap ma, mb;
   if (int e = map_pad6(&ma, y_pad, n, C, 128)) return e;
   if (int e = map_matrix(&mb, w_rows, 32, (uint64_t)16 * C, 32)) return e;
-  if (int e = dispatch_conv(pick_cfg(32, (n + 127) / 128, GATHER_SPLITS, false, 32), ma, mb, P, (n + 127) / 128, 32,
-                            GATHER_SPLITS, (cudaStream_t)stream)) return e;
+  if (int e = dispatch_conv(pick_cfg(32, (n + 127) / 128, GATHER_SPLITS, false, eg_sm_count(), 0), ma, mb, P,
+                            (n + 127) / 128, 32, GATHER_SPLITS, (cudaStream_t)stream)) return e;
   dense_gather_sum_kernel<<<(n * m_real + 255) / 256, 256, 0, (cudaStream_t)stream>>>((const float*)workspace, bias, n,
                                                                                       m_real, out);
   EG_LAUNCH_CHECK("dense_gather_sum_kernel");
@@ -1895,8 +1938,8 @@ extern "C" int eadgan_tc_dense_scatter(const void* a_bf16, const void* w_cols, c
   CUtensorMap ma, mb;
   if (int e = map_matrix(&ma, a_bf16, n, m_pad, 128)) return e;
   if (int e = map_matrix(&mb, w_cols, (uint64_t)16 * C, m_pad, 128)) return e;
-  return dispatch_conv(pick_cfg(16 * C, (n + 127) / 128, 1, false, 128), ma, mb, P, (n + 127) / 128, 16 * C, 1,
-                       (cudaStream_t)stream);
+  return dispatch_conv(pick_cfg(16 * C, (n + 127) / 128, 1, false, eg_sm_count(), 0), ma, mb, P, (n + 127) / 128, 16 * C,
+                       1, (cudaStream_t)stream);
 }
 
 extern "C" size_t eadgan_tc_dense_wgrad_workspace(int C, int m_pad) {
@@ -1910,17 +1953,18 @@ extern "C" int eadgan_tc_dense_wgrad(const void* a_bf16, const void* y_pad, floa
   EG_REQUIRE(a_bf16 && y_pad && dw && workspace && n > 0, EADGAN_ERR_INVALID, "tc_dense_wgrad: bad arguments");
   EG_REQUIRE(C % 64 == 0 && m_pad % 64 == 0 && m_real <= m_pad, EADGAN_ERR_UNSUPPORTED,
              "tc_dense_wgrad: needs C%%64==0 and m_pad%%64==0");
+  EG_REQUIRE(ws_bytes >= eadgan_tc_dense_wgrad_workspace(C, m_pad), EADGAN_ERR_WORKSPACE,
+             "tc_dense_wgrad: workspace too small");
   const int mp = ((m_pad + 127) / 128) * 128;
-  EG_REQUIRE(ws_bytes >= (size_t)mp * 16 * C * sizeof(float), EADGAN_ERR_WORKSPACE, "tc_dense_wgrad: workspace too small");
   WgParams P{};
   P.dense = 1; P.n = n; P.k = mp; P.c = C; P.qblocks = C / 64; P.Ktot = 16 * C;
   P.steps_total = (n + 63) / 64; P.steps_per_split = P.steps_total; P.partial = (float*)workspace;
+  P.kk_tiles = P.Ktot / 256; P.ko_tiles = mp / 128; P.splits = 1;
   CUtensorMap ma, mx;
   if (int e = map_matrix(&ma, a_bf16, n, m_pad, 64)) return e;
   if (int e = map_pad6(&mx, y_pad, n, C, 64)) return e;
-  dim3 grid(P.Ktot / 256, mp / 128, 1);
   cudaStream_t st = (cudaStream_t)stream;
-  if (int rc = launch_wgrad<256>(ma, mx, P, grid, st)) return rc;
+  if (int rc = launch_wgrad<256, 1>(ma, mx, P, st)) return rc;
   dense_wgrad_reduce_kernel<<<dim3(C / 64, m_real), 256, 0, st>>>(P.partial, mp, C, dw);
   EG_LAUNCH_CHECK("dense_wgrad_reduce_kernel");
   return 0;
@@ -2238,64 +2282,21 @@ extern "C" int eadgan_tc_thin_fprop(const eadgan_tc_desc* d, const void* r_buf, 
                                     void* y, const void* mask, double* stats, const float* sigma, void* stream) {
   if (int e = check_thin(d, "tc_thin_fprop")) return e;
   EG_REQUIRE(r_buf && w_packed && y, EADGAN_ERR_INVALID, "tc_thin_fprop: NULL pointer");
-  const int p = d->h / 2, q = d->w / 2;
+  ConvPlan pl;
+  if (int e = thin_fprop_plan(d, eg_sm_count(), read_hooks(), &pl)) return e;
   TcParams P{};
-  P.mode = MODE_FPROP; P.thin = 1; P.n = d->n; P.p = p; P.q = q;
-  EG_REQUIRE(pick_tile(p, q, 128, &P.Tw, &P.Th, &P.Tb) == 0, EADGAN_ERR_UNSUPPORTED,
-             "tc_thin_fprop: output map %dx%d must be a power of two <= 128 wide", p, q);
-  const int m_tiles = ((d->n + P.Tb - 1) / P.Tb) * (p / P.Th);
-  const int bn = pick_bn(d->k);
-  EG_REQUIRE(bn > 0, EADGAN_ERR_UNSUPPORTED, "tc_thin_fprop: k=%d must be a multiple of 32", d->k);
-  const TileCfg tcfg = pick_cfg(d->k, m_tiles, 1, false, bn);
-  P.tiles_y = p / P.Th; P.N_total = d->k; P.K_ch = 4; P.qblocks = 1; P.nkb = 1;
-  bool channel_major = d->k % 128 == 0 && !d->out_f32_nchw && (int64_t)m_tiles * (d->k / 128) >= 8 * eg_sm_count();
-  if (const char* e = getenv("EADGAN_TC_DGRADT")) {   // test hook: 0 / 2 = never / always channel-major where it applies
-    if (atoi(e) == 0) channel_major = false;
-    else if (atoi(e) == 2) channel_major = d->k % 128 == 0 && !d->out_f32_nchw;
-  }
-  P.act = d->act; P.slope = d->slope; P.out_f32_nchw = d->out_f32_nchw; P.want_stats = d->want_stats;
-  P.mask_mode = d->mask_mode; P.OH = p; P.OW = q; P.bias = bias; P.out = y;
-  P.mask = (const __nv_bfloat16*)mask; P.stats = stats; P.n_store = d->k; P.stat_channels = d->k; P.sigma = sigma;
-  EG_REQUIRE(!P.mask_mode || mask, EADGAN_ERR_INVALID, "tc_thin_fprop: mask_mode without mask");
-  EG_REQUIRE(!P.want_stats || stats, EADGAN_ERR_INVALID, "tc_thin_fprop: want_stats without stats");
-  CUtensorMap ma, mb;
+  P.thin = 1; P.N_total = d->k; P.K_ch = 4; P.qblocks = 1; P.nkb = 1;
+  P.OH = d->h / 2; P.OW = d->w / 2; P.n_store = d->k; P.stat_channels = d->k;
+  if (int e = conv_params(&P, MODE_FPROP, d, pl.t, bias, y, mask, stats, sigma, "tc_thin_fprop")) return e;
+  CUtensorMap ma;
   if (int e = map_thin(&ma, r_buf, d->n, d->h, d->w, P.Tw, P.Th, P.Tb)) return e;
-  if (channel_major) {   // tc_dgradT_kernel: 128 channels x 256 pixels per tile
-    P.m_tiles = (m_tiles + 1) / 2; P.n_tiles = d->k / 128; P.parities = 1;
-    if (int e = map_matrix(&mb, w_packed, d->k, 64, 128)) return e;
-    return launch_channel_major(ma, mb, P, (cudaStream_t)stream);
-  }
-  if (int e = map_matrix(&mb, w_packed, d->k, 64, bn)) return e;
-  return dispatch_conv(tcfg, ma, mb, P, m_tiles, d->k, 1, (cudaStream_t)stream);
+  return launch_conv_plan(pl, ma, w_packed, d->k, 64, P, d->k, 1, (cudaStream_t)stream);
 }
-
-namespace {
-int thin_wgrad_plan(const eadgan_tc_desc* d, WgParams* P, int* splits) {
-  const int p = d->h / 2, q = d->w / 2;
-  EG_REQUIRE(d->k % 32 == 0, EADGAN_ERR_UNSUPPORTED, "tc_thin_wgrad: k=%d must be a multiple of 32", d->k);
-  P->n = d->n; P->p = p; P->q = q; P->k = d->k; P->c = 4; P->thin = 1;
-  EG_REQUIRE(pick_tile(p, q, 64, &P->Tw, &P->Th, &P->Tb) == 0, EADGAN_ERR_UNSUPPORTED,
-             "tc_thin_wgrad: small map %dx%d must be a power of two <= 64 wide", p, q);
-  P->tiles_y = p / P->Th; P->qblocks = 1; P->Ktot = 64;
-  P->steps_total = ((d->n + P->Tb - 1) / P->Tb) * P->tiles_y;
-  // the only parallelism is the split of the pixel reduction: one CTA per SM (per 128-row ko tile)
-  const int ko_tiles = (d->k + 127) / 128;
-  int s = eg_sm_count() / ko_tiles;
-  const int max_s = (P->steps_total + 7) / 8;
-  if (s > max_s) s = max_s;
-  if (s < 1) s = 1;
-  P->steps_per_split = (P->steps_total + s - 1) / s;
-  *splits = (P->steps_total + P->steps_per_split - 1) / P->steps_per_split;
-  return 0;
-}
-}  // namespace
 
 extern "C" size_t eadgan_tc_thin_wgrad_workspace(const eadgan_tc_desc* d) {
-  if (!d) return 0;
-  WgParams P{};
-  int splits = 0;
-  if (thin_wgrad_plan(d, &P, &splits) != 0) return 0;
-  return (size_t)splits * (((d->k + 127) / 128) * 128) * 64 * sizeof(float);
+  WgPlan pl;
+  if (!d || thin_wgrad_plan(d, eg_sm_count(), &pl) != 0) return 0;
+  return pl.ws_bytes;
 }
 
 // dw[k][c][4][4] fp32 = sum over pixels of dy (padded NHWC bf16 small map) x image patch (row-expanded buffer)
@@ -2303,21 +2304,18 @@ extern "C" int eadgan_tc_thin_wgrad(const eadgan_tc_desc* d, const void* r_buf, 
                                     void* workspace, size_t ws_bytes, void* stream) {
   if (int e = check_thin(d, "tc_thin_wgrad")) return e;
   EG_REQUIRE(r_buf && dy_pad && dw && workspace, EADGAN_ERR_INVALID, "tc_thin_wgrad: NULL pointer");
-  WgParams P{};
-  int splits = 0;
-  if (int e = thin_wgrad_plan(d, &P, &splits)) return e;
-  const int k_pad = ((d->k + 127) / 128) * 128;
-  const size_t need = (size_t)splits * k_pad * 64 * sizeof(float);
-  EG_REQUIRE(ws_bytes >= need, EADGAN_ERR_WORKSPACE, "tc_thin_wgrad: workspace %zu < %zu bytes", ws_bytes, need);
+  WgPlan pl;
+  if (int e = thin_wgrad_plan(d, eg_sm_count(), &pl)) return e;
+  EG_REQUIRE(ws_bytes >= pl.ws_bytes, EADGAN_ERR_WORKSPACE, "tc_thin_wgrad: workspace %zu < %zu bytes", ws_bytes,
+             pl.ws_bytes);
+  WgParams& P = pl.P;
   P.partial = (float*)workspace;
-  WgParams PK = P;
-  PK.k = k_pad;
   CUtensorMap mdy, mx;
   if (int e = map_small(&mdy, dy_pad, d->n, d->k, P.p, P.q, P.Tw, P.Th, P.Tb)) return e;
   if (int e = map_thin(&mx, r_buf, d->n, d->h, d->w, P.Tw, P.Th, P.Tb)) return e;
   cudaStream_t st = (cudaStream_t)stream;
-  if (int rc = launch_wgrad<64>(mdy, mx, PK, dim3(1, k_pad / 128, splits), st)) return rc;
-  thin_wgrad_reduce_kernel<<<(d->k * 64 + 255) / 256, 256, 0, st>>>(P.partial, splits, k_pad, d->k, d->c, dw);
+  if (int e = dispatch_wgrad(pl, mdy, mx, st)) return e;
+  thin_wgrad_reduce_kernel<<<(d->k * 64 + 255) / 256, 256, 0, st>>>(P.partial, P.splits, P.k, d->k, d->c, dw);
   EG_LAUNCH_CHECK("thin_wgrad_reduce_kernel");
   return 0;
 }
@@ -2338,13 +2336,6 @@ extern "C" int eadgan_tc_thin_dgrad(const eadgan_tc_desc* d, const void* dy_pad,
   CUtensorMap ma, mb;
   if (int e = map_small(&ma, dy_pad, d->n, d->k, p, q, 32, 4, 1)) return e;
   if (int e = map_matrix(&mb, w_packed, 64, (uint64_t)d->k, 64)) return e;
-  static std::atomic<uint64_t> opted{0};
-  if (int e = opt_in_smem(tc_thin_dgrad_kernel, THIN_SMEM, opted)) return e;
-  const int total = d->n * (p / 2);
-  const int sms = eg_sm_count();
-  const int waves = (total + sms - 1) / sms;
-  const int grid = (total + waves - 1) / waves;
-  tc_thin_dgrad_kernel<<<grid, 320, THIN_SMEM, (cudaStream_t)stream>>>(ma, mb, P);
-  EG_LAUNCH_CHECK("tc_thin_dgrad_kernel");
-  return 0;
+  return launch_persistent<tc_thin_dgrad_kernel, 1>("tc_thin_dgrad_kernel", d->n * P.tiles_per_img, 320, THIN_SMEM,
+                                                    (cudaStream_t)stream, ma, mb, P);
 }

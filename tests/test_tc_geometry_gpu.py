@@ -11,9 +11,8 @@ goes unnoticed; this file uses non-square maps throughout.
 
 GEOMETRY names, for each kernel entry point, the shapes (n, c, p, q, k) -- c channels of the big map (2p x 2q), k of
 the small map -- with the test hook each runs under and the regime it must take.  The *_regime helpers restate the C
-size arithmetic (pick_tile, pick_bn_tiles / pick_cfg with the EADGAN_TC_CG hook, the channel-major predicates of
-eadgan_tc_dgrad and eadgan_tc_thin_fprop with the EADGAN_TC_DGRADT hook, wgrad_plan, thin_wgrad_plan) with the SM count
-as an argument.  test_geometry_table (no GPU) checks every entry at the B200's 148 SMs, and every GPU test asserts that
+launch plans (pick_tile, pick_cfg with the EADGAN_TC_CG hook, fprop_plan, dgrad_plan and thin_fprop_plan with the
+EADGAN_TC_DGRADT hook, wgrad_plan, thin_wgrad_plan), which also take the SM count as an argument.  test_geometry_table (no GPU) checks every entry at the B200's 148 SMs, and every GPU test asserts that
 its shape still takes its regime on the device it runs on.
 
 What each shape checks, against fp64 on the same bf16 operands (tolerances of tests/test_tc_gpu.py: 2e-3 for fp32
